@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DUSty-GAN generate-and-evaluate hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline (BASELINE.json): Chamfer pairs/sec. Default workload = configs[2]: 1000 vs 1000 clouds of 2048
 FPS-sampled points, full MMD/COV/1-NNA. One "step" is one complete evaluation through the public
@@ -497,6 +497,14 @@ def nccl_comm_evidence(world, device):
     return ev
 
 
+def dump_outputs(directory, scores):
+    """What compute_cov_mmd_1nna returned to its caller in the last timed step: one 0-d float64 array per score.
+    The inputs are made from fixed seeds, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(directory, exist_ok=True)
+    for name, value in scores.items():
+        np.save(os.path.join(directory, f"{name}.npy"), np.array(value, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -508,7 +516,11 @@ def main():
     ap.add_argument("--skip-extras", action="store_true", help="headline only (no stages / cpu baseline)")
     ap.add_argument("--dusty", type=int, default=None, choices=[1, 2], help="head that makes the clouds (default: the workload's)")
     ap.add_argument("--full-resolution", action="store_true", help="un-sampled 64x512 clouds (32768 points each), as cfg4")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the scores the last timed step returned as DIR/<name>.npy (float64), to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -603,6 +615,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, scores)
 
     ms_per_step = dev_ms / args.steps
     value = entries / (ms_per_step * 1e-3)

@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from dusty_gan_b200 import pipeline
 dev = torch.device("cuda:0")

@@ -1,5 +1,5 @@
 import os, sys, statistics
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, bench
 from dusty_gan_b200.utils.metrics.distance import chamfer_distance
 dev = torch.device("cuda:0")

@@ -1,5 +1,5 @@
-import sys, time, torch, statistics, ctypes as C
-sys.path.insert(0, "/root/repo")
+import os, sys, time, torch, statistics, ctypes as C
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from dusty_gan_b200 import _lib
 from dusty_gan_b200.utils.metrics import cov_mmd_1nna as M

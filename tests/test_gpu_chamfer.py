@@ -1,5 +1,5 @@
-"""Chamfer kernels (through the Python mirror -> C ABI) against the oracle, the golden vectors and,
-when oracle/_ref is present, the reference's own CUDA kernel on the same GPU."""
+"""Chamfer kernels (through the Python mirror -> C ABI) against the oracle, the golden vectors and the
+reference's own CUDA kernel (its stored outputs, plus a live run on the same GPU when oracle/_ref is present)."""
 import numpy as np
 import pytest
 import torch
@@ -86,23 +86,31 @@ def test_forward_empty_sides():
     assert d1.shape == (2, 0) and np.all(d2 == 0) and np.all(i2 == 0)      # outputs left zero like the reference
 
 
-def test_forward_against_reference_cuda_kernel():
+def reference_forward_cases(golden):
+    """(xyz1, xyz2, (dist1, dist2, idx1, idx2) of the reference CUDA kernel): every case it ran on a B200 for
+    tests/golden/gpu_reference_kernels.npz (oracle/gen_golden_gpu.py) and, when oracle/_ref holds the compiled
+    reference, one more run live on this GPU."""
+    g = golden("gpu_reference_kernels.npz")
+    for i in range(3):
+        b, n, m, seed = [int(v) for v in g[f"cd{i}_case"]]
+        yield (sampled_clouds(b, n, seed), lidar_like_clouds(b, m, seed + 1),
+               tuple(g[f"cd{i}_{k}"] for k in ("dist1", "dist2", "idx1", "idx2")))
     cd = refload.load("dustyref_cd")
-    if cd is None:
-        pytest.skip("oracle/_ref/dustyref_cd not built")
-    a = sampled_clouds(4, 2048, 31); b = sampled_clouds(4, 2048, 32)
-    ta, tb = cuda(a), cuda(b)
-    r1 = torch.zeros(4, 2048, device="cuda"); r2 = torch.zeros(4, 2048, device="cuda")
-    k1 = torch.zeros(4, 2048, dtype=torch.int32, device="cuda"); k2 = torch.zeros(4, 2048, dtype=torch.int32, device="cuda")
-    cd.forward_cuda(ta, tb, r1, r2, k1, k2)
-    torch.cuda.synchronize()
-    d1, d2, i1, i2 = run_forward(a, b)
-    for d, r, i, k in ((d1, r1, i1, k1), (d2, r2, i2, k2)):
-        assert np.array_equal(d, r.cpu().numpy()) and np.array_equal(i, k.cpu().numpy())
-    # and the oracle's CUDA-rounding restatement IS the reference kernel, bit for bit
-    o1, o2, j1, j2 = native.chamfer_forward(a, b, rounding="cuda")
-    assert np.array_equal(o1, r1.cpu().numpy()) and np.array_equal(j1, k1.cpu().numpy())
-    assert np.array_equal(o2, r2.cpu().numpy()) and np.array_equal(j2, k2.cpu().numpy())
+    if cd is not None:
+        a = sampled_clouds(4, 2048, 31); b = sampled_clouds(4, 2048, 32)
+        r1 = torch.zeros(4, 2048, device="cuda"); r2 = torch.zeros(4, 2048, device="cuda")
+        k1 = torch.zeros(4, 2048, dtype=torch.int32, device="cuda"); k2 = torch.zeros(4, 2048, dtype=torch.int32, device="cuda")
+        cd.forward_cuda(cuda(a), cuda(b), r1, r2, k1, k2)
+        torch.cuda.synchronize()
+        yield a, b, tuple(t.cpu().numpy() for t in (r1, r2, k1, k2))
+
+
+def test_forward_against_reference_cuda_kernel(golden):
+    for a, b, want in reference_forward_cases(golden):
+        for got in (run_forward(a, b),
+                    native.chamfer_forward(a, b, rounding="cuda")):    # the oracle's CUDA-rounding restatement IS the reference kernel, bit for bit
+            for x, r in zip(got, want):
+                assert np.array_equal(x, r), (a.shape, b.shape)
 
 
 def test_autograd_wrapper_and_backward(golden):

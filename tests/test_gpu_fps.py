@@ -1,5 +1,6 @@
 """FPS kernel: indices bit-exact against the oracle's thread-by-thread replay of the reference
-kernel and, when oracle/_ref is present, against the reference's own CUDA kernel on this GPU."""
+kernel and against the reference's own CUDA kernel (its stored outputs, plus a live run on this GPU
+when oracle/_ref is present)."""
 import numpy as np
 import pytest
 import torch
@@ -79,17 +80,30 @@ def test_downsample_and_gather():
     assert torch.allclose(feats.grad, expect)
 
 
-def test_against_reference_cuda_kernel():
+def reference_kernel_cases(golden):
+    """(clouds, samples, the reference CUDA kernel's indices): every case it ran on a B200 for
+    tests/golden/gpu_reference_kernels.npz (oracle/gen_golden_gpu.py) and, when oracle/_ref holds the
+    compiled reference, three more run live on this GPU."""
+    g = golden("gpu_reference_kernels.npz")
+    i = 0
+    while f"fps{i}_case" in g:
+        b, n, m, seed, dropped, near = [int(v) for v in g[f"fps{i}_case"]]
+        yield lidar_like_clouds(b, n, seed, dropped=dropped / 1000, near=near / 1000), m, g[f"fps{i}_idx"]
+        i += 1
+    yield g["fps_deg_input"], 200, g["fps_deg_idx"]
     ref = refload.load("dustyref_fps")
-    if ref is None:
-        pytest.skip("oracle/_ref/dustyref_fps not built")
-    for n, m, seed in ((32768, 2048, 21), (5000, 512, 22), (700, 64, 23)):
-        x = lidar_like_clouds(3, n, seed)
-        t = cuda(x)
-        r = ref.furthest_point_sampling(t, m)
-        torch.cuda.synchronize()
-        assert np.array_equal(fps_gpu(x, m), r.cpu().numpy())
-        assert np.array_equal(native.fps(x, m), r.cpu().numpy())       # pins the oracle too
+    if ref is not None:
+        for n, m, seed in ((32768, 2048, 21), (5000, 512, 22), (700, 64, 23)):
+            x = lidar_like_clouds(3, n, seed)
+            r = ref.furthest_point_sampling(cuda(x), m)
+            torch.cuda.synchronize()
+            yield x, m, r.cpu().numpy()
+
+
+def test_against_reference_cuda_kernel(golden):
+    for x, m, want in reference_kernel_cases(golden):
+        assert np.array_equal(fps_gpu(x, m), want), (x.shape, m)
+        assert np.array_equal(native.fps(x, m), want), (x.shape, m)     # pins the oracle too
 
 
 def test_against_reference_cuda_golden(golden):
