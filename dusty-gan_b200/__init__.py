@@ -6,8 +6,8 @@ The package mirrors the reference's module paths for that path and nothing else:
     utils                        tanh_to_sigmoid, sigmoid_to_tanh, flatten (reference utils/__init__.py:70-79,213)
     utils.lidar                  Coordinate, LiDAR                      (reference utils/lidar.py)
     utils.sampling.fps           furthest_point_sampling, gather_operation, downsample_point_clouds
-    utils.metrics.distance       chamfer_distance, ChamferDistance
-    utils.metrics.cov_mmd_1nna   compute_cd, _pairwise_distance, compute_cov_mmd_1nna
+    utils.metrics.distance       chamfer_distance, ChamferDistance, earth_mover_distance
+    utils.metrics.cov_mmd_1nna   compute_cd, compute_emd, emd_matrix, _pairwise_distance, compute_cov_mmd_1nna
     utils.metrics.jsd            compute_jsd                              (reference utils/metrics/jsd.py)
     datasets                     define_dataset, KITTIOdometry, preprocess_scans (reference datasets/kitti.py)
     pipeline                     fused generate->points entry (project_2d_to_3d of evaluate_synthesis.py:59-64),

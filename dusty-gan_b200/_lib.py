@@ -70,7 +70,16 @@ SIGNATURES = {
                                               C.c_void_p, C.c_size_t, C.c_void_p]),
     "dusty_cov_mmd_knna_finalize": (C.c_int, [c_float_p, c_float_p, c_float_p, C.c_int, C.c_int, C.c_int, c_float_p,
                                               C.c_void_p, C.c_size_t, C.c_void_p]),
-    "dusty_jsd_vote": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_int, c_float_p, c_int_p, c_float_p, C.c_float,
+    "dusty_emd_forward_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "dusty_emd_forward": (C.c_int, [c_float_p, c_float_p, C.c_int, C.c_int, C.c_int, c_float_p, c_float_p, C.c_void_p,
+                                    C.c_size_t, C.c_void_p]),
+    "dusty_emd_backward": (C.c_int, [c_float_p, c_float_p, C.c_int, C.c_int, C.c_int, c_float_p, c_float_p, c_float_p,
+                                     c_float_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dusty_emd_matrix_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "dusty_emd_matrix": (C.c_int, [c_float_p, C.c_int, C.c_int, c_float_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                   c_float_p, C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                   C.c_size_t, C.c_void_p]),
+    "dusty_jsd_vote":(C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_int, c_float_p, c_int_p, c_float_p, C.c_float,
                                  C.c_void_p, C.c_void_p, C.c_void_p]),
     "dusty_jsd_from_counts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, c_float_p, C.c_void_p]),
     "dusty_fps_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),

@@ -16,7 +16,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libdustyb200.so")
-SOURCES = ["api.cu", "chamfer.cu", "fps.cu", "head_project.cu", "metrics.cu", "jsd.cu", "scan_preprocess.cu"]
+SOURCES = ["api.cu", "chamfer.cu", "fps.cu", "head_project.cu", "metrics.cu", "jsd.cu", "scan_preprocess.cu", "emd.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

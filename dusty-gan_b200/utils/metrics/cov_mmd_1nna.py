@@ -19,7 +19,7 @@ import numpy as np
 import torch
 
 from ... import _lib, sharding
-from .distance import chamfer_distance
+from .distance import chamfer_distance, earth_mover_distance
 
 
 # When bench.py sets this to a list, every matrix launch appends a (start, end) CUDA event pair.
@@ -29,6 +29,11 @@ KERNEL_EVENTS = None
 def compute_cd(pcs_1, pcs_2):
     dl, dr = chamfer_distance(pcs_1, pcs_2)
     return dl.mean(dim=1) + dr.mean(dim=1)
+
+
+def compute_emd(pcs_1, pcs_2):
+    """Approximate EMD per point (PointFlow's emd_approx): the match cost divided by the point count of pcs_1."""
+    return earth_mover_distance(pcs_1, pcs_2, transpose=False) / pcs_1.size(1)
 
 
 def _check_clouds(pcs, name):
@@ -115,9 +120,50 @@ def chamfer_matrix(pcs_1, pcs_2=None, rows=None, compact_rows=False, out=None, m
     return out if store else None
 
 
+def emd_matrix(pcs_1, pcs_2, rows=None, out=None, fused=None):
+    """M[i,j] = compute_emd(pcs_1[i:i+1], pcs_2[j:j+1]) bit for bit, in one launch. EMD is not symmetric, so every
+    entry is computed. ``rows=(begin,end,stride)`` restricts the computation to a row shard (other rows of ``out``
+    are left as they are). ``fused=(keys, stacked_offset_1, stacked_offset_2, n_ref, n_total)`` also reduces every
+    entry into the packed minima ``keys`` (int64, 3 n_total; see ``emd_scores``); with ``out=False`` the matrix is
+    then not stored at all."""
+    a = _check_clouds(pcs_1, "pcs_1")
+    b = _check_clouds(pcs_2, "pcs_2")
+    na, pa, _ = a.shape
+    nb, pb, _ = b.shape
+    begin, end, stride = rows if rows is not None else (0, na, 1)
+    store = out is not False
+    if not store and fused is None:
+        raise ValueError("out=False needs fused=...")
+    if out is None:
+        out = torch.zeros(na, nb, device=a.device, dtype=torch.float32)
+    if pa == 0 or pb == 0:
+        raise ValueError("clouds must hold at least one point")
+    if na == 0 or nb == 0 or len(range(begin, end, stride)) == 0:
+        return out if store else None
+    keys, off_1, off_2, n_ref, n_total = fused if fused is not None else (None, 0, 0, 0, 0)
+    if keys is not None:
+        assert keys.dtype == torch.int64 and keys.numel() == 3 * n_total and keys.is_contiguous()
+    lib = _lib.load()
+    nbytes = lib.dusty_emd_matrix_workspace_bytes(na, pa, nb, pb)
+    ws = _lib.workspace(nbytes, a.device)
+    with torch.cuda.device(a.device):
+        if KERNEL_EVENTS is not None:
+            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            ev[0].record()
+        m_ptr, ldm = (_lib.ptr(out), out.stride(0)) if store else (None, 0)
+        _lib.check(lib.dusty_emd_matrix(_lib.ptr(a), na, pa, _lib.ptr(b), nb, pb, begin, end, stride, m_ptr, ldm, off_1, off_2,
+                                        n_ref, n_total, _lib.ptr(keys), _lib.ptr(ws), nbytes, _lib.stream_of(a)),
+                   "dusty_emd_matrix")
+        if KERNEL_EVENTS is not None:
+            ev[1].record()
+            KERNEL_EVENTS.append(ev)
+    return out if store else None
+
+
 def _pairwise_distance(pcs_1, pcs_2, batch_size, metrics=("cd",), verbose=True):
     """{"cd": (B_1,B_2)} like the reference (cov_mmd_1nna.py:24-51). ``batch_size`` (the reference's
     column block) and ``verbose`` (its tqdm bar) are accepted and have no effect."""
+    # EMD matrices come from emd_matrix(pcs_1, pcs_2); this function keeps refusing "emd".
     if "emd" in metrics:
         raise NotImplementedError("EMD is not part of the path (the reference's extension does not build on "
                                   "torch>=2 and its callers pass metrics=('cd',))")
@@ -226,33 +272,67 @@ def fused_scores(pcs_gen, pcs_ref, group=None):
         chamfer_matrix(ref, None, rows=sharding.owned_rows(nr, rank, G), compact_rows=True, out=False, fused=(keys, 0, 0, nr, n))
         chamfer_matrix(ref, gen, rows=sharding.owned_rows(nr, rank, G), compact_rows=True, out=False, fused=(keys, 0, nr, nr, n))
         chamfer_matrix(gen, None, rows=sharding.owned_rows(ng, rank, G), compact_rows=True, out=False, fused=(keys, nr, nr, nr, n))
+    return _scores_from_keys(keys, nr, ng, group)
+
+
+def _scores_from_keys(keys, nr, ng, group):
+    """All-gather every rank's packed minima and reduce them to (cov/mmd dict, 1-NNA dict)."""
+    n = nr + ng
+    lib = _lib.load()
     gathered = sharding.all_gather_keys(keys, group)
     nbytes = lib.dusty_cov_mmd_1nna_workspace_bytes(nr, ng)
-    ws = _lib.workspace(nbytes, ref.device)
-    out = torch.empty(7, device=ref.device, dtype=torch.float32)
-    with torch.cuda.device(ref.device):
+    ws = _lib.workspace(nbytes, keys.device)
+    out = torch.empty(7, device=keys.device, dtype=torch.float32)
+    with torch.cuda.device(keys.device):
         _lib.check(lib.dusty_cov_mmd_1nna_from_keys(_lib.ptr(gathered), gathered.size(0), nr, ng, _lib.ptr(out), _lib.ptr(ws),
-                                                    nbytes, _lib.stream_of(ref)), "dusty_cov_mmd_1nna_from_keys")
+                                                    nbytes, _lib.stream_of(keys)), "dusty_cov_mmd_1nna_from_keys")
     o = [float(v) for v in out.tolist()]
     cov_mmd = {"mmd": o[0], "mmd-sample": o[1], "cov": float(o[2]) / float(nr)}
     return cov_mmd, _nna_scores(o[3], o[4], o[5], o[6], n)
 
 
+def emd_pairwise_matrices(pcs_gen, pcs_ref):
+    """(M_rr, M_rg, M_gg) of compute_emd, each computed in full (EMD is not symmetric; M_gr is never needed)."""
+    gen = _check_clouds(pcs_gen, "pcs_gen")
+    ref = _check_clouds(pcs_ref, "pcs_ref")
+    return emd_matrix(ref, ref), emd_matrix(ref, gen), emd_matrix(gen, gen)
+
+
+def emd_scores(pcs_gen, pcs_ref, group=None):
+    """fused_scores for EMD: three launches (M_rr, M_rg, M_gg), each row-sharded over ``group``, reduce every entry
+    into the packed minima of the column-wise 1-NN matrix [[M_rr, M_rg], [M_rg^T, M_gg]] and the cross-set minima;
+    one all-gather of those vectors, no matrix stored."""
+    gen = _check_clouds(pcs_gen, "pcs_gen")
+    ref = _check_clouds(pcs_ref, "pcs_ref")
+    nr, ng = ref.size(0), gen.size(0)
+    n = nr + ng
+    if nr == 0 or ng == 0:
+        raise ValueError("both sets must hold at least one cloud")
+    rank, G = sharding.world(group)
+    lib = _lib.load()
+    keys = torch.empty(3 * n, device=ref.device, dtype=torch.int64)
+    with torch.cuda.device(ref.device):
+        _lib.check(lib.dusty_nn_keys_reset(_lib.ptr(keys), n, _lib.stream_of(keys)), "dusty_nn_keys_reset")
+    emd_matrix(ref, ref, rows=sharding.owned_rows(nr, rank, G), out=False, fused=(keys, 0, 0, nr, n))
+    emd_matrix(ref, gen, rows=sharding.owned_rows(nr, rank, G), out=False, fused=(keys, 0, nr, nr, n))
+    emd_matrix(gen, gen, rows=sharding.owned_rows(ng, rank, G), out=False, fused=(keys, nr, nr, nr, n))
+    return _scores_from_keys(keys, nr, ng, group)
+
+
 @torch.no_grad()
 def compute_cov_mmd_1nna(pcs_gen, pcs_ref, batch_size, metrics=("cd",), verbose=True):
     assert isinstance(metrics, tuple)
-    if "emd" in metrics:
-        raise NotImplementedError("EMD is not part of the path; pass metrics=('cd',)")
     results = {}
-    if "cd" not in metrics:
-        return results
-    if FUSED_EPILOGUE:
-        cov_mmd, nna = fused_scores(pcs_gen, pcs_ref)
-    else:       # the three matrices, then three small kernels over them (kept for A/B tests)
-        M_rr, M_rg, M_gg = pairwise_matrices(pcs_gen, pcs_ref)
-        cov_mmd, nna = _finalize_device(M_rr, M_rg, M_gg)
-    for k, v in cov_mmd.items():
-        results.update({"{}-{}".format(k, "cd"): v})
-    for k, v in nna.items():
-        results.update({"1-nn-{}-{}".format(k, "cd"): v})
+    for metric in ("cd", "emd"):
+        if metric not in metrics:
+            continue
+        if FUSED_EPILOGUE:
+            cov_mmd, nna = (fused_scores if metric == "cd" else emd_scores)(pcs_gen, pcs_ref)
+        else:       # the three matrices, then three small kernels over them (kept for A/B tests)
+            M_rr, M_rg, M_gg = (pairwise_matrices if metric == "cd" else emd_pairwise_matrices)(pcs_gen, pcs_ref)
+            cov_mmd, nna = _finalize_device(M_rr, M_rg, M_gg)
+        for k, v in cov_mmd.items():
+            results.update({"{}-{}".format(k, metric): v})
+        for k, v in nna.items():
+            results.update({"1-nn-{}-{}".format(k, metric): v})
     return results

@@ -73,7 +73,11 @@ def main():
     ap.add_argument("--tol", type=float, default=0.0)
     ap.add_argument("--batch-size", type=int, default=32)       # cfg.solver.batch_size
     ap.add_argument("--dusty", type=int, default=1, choices=[1, 2])
+    ap.add_argument("--metrics", default="cd", help="comma-separated subset of cd,emd for MMD/COV/1-NNA")
     args = ap.parse_args()
+    metrics = tuple(m.strip() for m in args.metrics.split(",") if m.strip())
+    if not metrics or any(m not in ("cd", "emd") for m in metrics):
+        ap.error(f"--metrics: expected a subset of cd,emd, got {args.metrics!r}")
     torch.set_grad_enabled(False)
     device = torch.device("cuda")
     torch.manual_seed(0)
@@ -100,7 +104,7 @@ def main():
     torch.cuda.synchronize(); t2 = time.perf_counter()
 
     scores = {"jsd": compute_jsd(pcs_gen=fakes["3d"] / 2.0, pcs_ref=reals["3d"] / 2.0)}
-    scores.update(compute_cov_mmd_1nna(pcs_gen=fakes["3d"], pcs_ref=reals["3d"], batch_size=512, metrics=("cd",)))
+    scores.update(compute_cov_mmd_1nna(pcs_gen=fakes["3d"], pcs_ref=reals["3d"], batch_size=512, metrics=metrics))
     torch.cuda.synchronize(); t3 = time.perf_counter()
     scores["#test"] = args.num_test
     scores["#points"] = args.num_points

@@ -23,6 +23,11 @@
  *                                folded into the matrix kernel's epilogue -- no (Nr+Ng)^2 tensor is ever stored
  *   dusty_symmetric_from_shards  the multi-GPU assembly of a row-sharded symmetric matrix (no reference
  *                                counterpart: the reference is single-GPU on this path)
+ *   dusty_emd_forward            utils/metrics/distance/emd/ (approxmatch + matchcost, SURVEY.md S2a), the
+ *                                forward of earth_mover_distance; no (b,m,n) match matrix
+ *   dusty_emd_backward           the same extension's matchcostgrad1 / matchcostgrad2
+ *   dusty_emd_matrix             utils/metrics/cov_mmd_1nna.py compute_emd and the "emd" metric of
+ *                                compute_cov_mmd_1nna, with the fused minima of dusty_chamfer_matrix_fused
  *   dusty_jsd_vote, dusty_jsd_from_counts   utils/metrics/jsd.py:23-92, 110-121 (entropy_of_occupancy_grid,
  *                                _jensen_shannon_divergence)
  *   dusty_fps                    utils/sampling/fps/furthest_point_sampling.cpp:79-100
@@ -189,6 +194,47 @@ DUSTY_API int dusty_cov_mmd_1nna_finalize(const float* Mrr, const float* Mrg, co
  * The reference's optional sqrt of the distances is monotone and does not change the neighbour sets. */
 DUSTY_API int dusty_cov_mmd_knna_finalize(const float* Mrr, const float* Mrg, const float* Mgg, int nr, int ng, int k,
                                 float* out7, void* workspace, size_t workspace_bytes, void* stream);
+
+/* --------------------------------------------------------------------------------------------
+ * Approximate Earth Mover's Distance (reference utils/metrics/distance/emd/: the PSGN approxmatch)
+ * -------------------------------------------------------------------------------------------- */
+
+/* Scratch for dusty_emd_forward on (b,n,3) x (b,m,3). */
+DUSTY_API size_t dusty_emd_forward_workspace_bytes(int b, int n, int m);
+
+/* Approximate EMD of b independent cloud pairs, bit-equal to the reference's approxmatch + matchcost kernels.
+ *   xyz1 (b,n,3) f32, xyz2 (b,m,3) f32, contiguous; n, m >= 1.
+ *   cost (b) f32: sum_{k,l} |xyz1[k] - xyz2[l]| match[l][k] (not divided by the point count).
+ *   factors (b,10,n+m) f32 or NULL: the ten per-level ratio vectors (level v = 7 - j: ratioL (n), then
+ *   ratioR (m)) from which dusty_emd_backward rebuilds the match. No (b,m,n) match matrix is stored. */
+DUSTY_API int dusty_emd_forward(const float* xyz1, const float* xyz2, int b, int n, int m, float* cost,
+                                float* factors, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Gradient of sum(grad_cost * cost) with the match held constant (the reference's matchcostgrad1/2):
+ *   grad1[k] = grad_cost * sum_l match[l][k] (xyz1[k] - xyz2[l]) / max(|xyz1[k] - xyz2[l]|, 1e-20), grad2 the same
+ *   with the sign flipped. factors from dusty_emd_forward on the same clouds. grad1 (b,n,3) and grad2 (b,m,3) are
+ *   overwritten. No scratch is needed: workspace may be NULL. */
+DUSTY_API int dusty_emd_backward(const float* xyz1, const float* xyz2, int b, int n, int m, const float* grad_cost,
+                                 const float* factors, float* grad1, float* grad2,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+
+/* Scratch for dusty_emd_matrix on A (na,pa,3) x B (nb,pb,3). */
+DUSTY_API size_t dusty_emd_matrix_workspace_bytes(int na, int pa, int nb, int pb);
+
+/* Pairwise EMD matrix (compute_emd of cov_mmd_1nna.py, each entry bit-equal to the one-pair forward):
+ *   M[i,j] = cost(A[i], B[j]) * f32(1/pa), for rows i = row_begin, row_begin + row_stride, ... < row_end; M
+ *   row-major with leading dimension ldm (>= nb), NULL: not stored. EMD is not symmetric: every entry is computed.
+ * With keys (3*n_total u64, reset by dusty_nn_keys_reset) every entry also feeds the packed minima of
+ * dusty_chamfer_matrix_fused, so dusty_cov_mmd_1nna_from_keys gives the scores. Cloud i of A is stacked cloud
+ * stacked_offset_a + i, cloud j of B stacked_offset_b + j (reference clouds first). The 1-NN matrix
+ * [[M_rr, M_rg], [M_rg^T, M_gg]] is reduced column-wise (topk(dim=0)): entry (r, c) feeds keys[c] with index r when
+ * r != c; an M_rg entry (r < n_ref <= c) also feeds keys[r] with c, keys[n_total + c] with r and
+ * keys[2 n_total + r] with c. A launch is reference-by-reference, reference-by-generated or
+ * generated-by-generated; generated-by-reference (M_gr) is refused, since no score reads it. */
+DUSTY_API int dusty_emd_matrix(const float* A, int na, int pa, const float* B, int nb, int pb,
+                               int row_begin, int row_end, int row_stride, float* M, long long ldm,
+                               int stacked_offset_a, int stacked_offset_b, int n_ref, int n_total, uint64_t* keys,
+                               void* workspace, size_t workspace_bytes, void* stream);
 
 /* --------------------------------------------------------------------------------------------
  * JSD between occupancy histograms (next row 8f-2; reference utils/metrics/jsd.py:23-121)
