@@ -28,7 +28,6 @@
 //            index) returned is exactly the reference kernel's, for any finite input; the guard fires for
 //            ~0.1 % of the (row, tile) pairs on LiDAR-like clouds and costs < 0.5 %.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -38,8 +37,6 @@ namespace chamfer {
 constexpr int TPB = 256;
 constexpr int TILE = 2048;            // scan points per shared-memory tile (= float4 per tile)
 constexpr int CHUNK = 32;             // candidates per search chunk
-constexpr int PAIRS = CHUNK / 2;
-constexpr int SMEM_BYTES = 2 * TILE * 16;
 
 struct Params {
   const float4* scanX;      // scan-format clouds, X side (rows of the matrix / xyz1)
@@ -55,12 +52,12 @@ struct Params {
   // batch front end
   float* dist1; float* dist2;
   int* idx1; int* idx2;
-  // merged-origin clouds (MERGED instantiations): per-cloud {points kept, weight of the last kept point}, the
-  // per-chunk bounding boxes of sorted clouds (null: no pruning) and, for the batch front end, the map from a
-  // sorted position back to the original point index (the merged origin point maps to the first zero point)
+  // merged-origin clouds: per-cloud {points kept, weight of the last kept point}, the per-chunk bounding boxes of
+  // sorted clouds and, for the batch front end, the map from a sorted position back to the original point index
+  // (the merged origin point maps to the first zero point)
   const int2* metaX; const int2* metaY;
   const float4* boxX; const float4* boxY;
-  const float4* bbX; const float4* bbY;      // boxes of the blocks of 32 chunks (k-d ordered clouds, nn_walk_kernel)
+  const float4* bbX; const float4* bbY;      // boxes of the blocks of 32 chunks (sorted clouds, nn_walk_split_kernel)
   const int* permX; const int* permY;
   unsigned long long* visited;   // measurement only (null: off): (row, candidate) pairs the pruned search really evaluated
   // fused MMD/COV/1-NNA epilogue (matrix front end; null: off). keys = 3 arrays of n_total packed
@@ -101,11 +98,10 @@ __device__ __forceinline__ float search_window(float ax, float ay, float az, flo
 
 // The whole tile (npairs candidate pairs in scan format) against one row point, in the reference's rounding,
 // by all 32 lanes of a warp: minimum and, if wanted, the tile-relative position of the winner -- the lowest
-// position among bit-equal minima, or, for sorted clouds (perm != null: position of the tile's first candidate
-// in the map from positions to original indices), the position with the lowest original index.
+// position among bit-equal minima.
 template <bool WANT_INDEX>
 __device__ __forceinline__ void warp_tile_exact_min(const float4* tp, int npairs, float ax, float ay, float az, int lane,
-                                                    const int* perm, float& best, int& best_pos) {
+                                                    float& best, int& best_pos) {
   const f32x2 ax2 = pack2(ax, ax), ay2 = pack2(ay, ay), az2 = pack2(az, az);
   float e = __int_as_float(0x7f800000);
   int ei = 0x7fffffff;
@@ -117,8 +113,8 @@ __device__ __forceinline__ void warp_tile_exact_min(const float4* tp, int npairs
     float lo, hi;
     unpack2(fma2(dz, dz, fma2(dx, dx, mul2(dy, dy))), lo, hi);
     if (WANT_INDEX) {                       // q ascends: strict < keeps the lane's lowest position
-      if (lo < e || (perm && lo == e && ei != 0x7fffffff && perm[2 * q] < perm[ei])) { e = lo; ei = 2 * q; }
-      if (hi < e || (perm && hi == e && ei != 0x7fffffff && perm[2 * q + 1] < perm[ei])) { e = hi; ei = 2 * q + 1; }
+      if (lo < e) { e = lo; ei = 2 * q; }
+      if (hi < e) { e = hi; ei = 2 * q + 1; }
     } else {
       e = min3(e, lo, hi);
     }
@@ -129,7 +125,7 @@ __device__ __forceinline__ void warp_tile_exact_min(const float4* tp, int npairs
   best = m;
   if (WANT_INDEX) {
     const bool mine = e == m && ei != 0x7fffffff;
-    const unsigned key = mine ? (unsigned)(perm ? perm[ei] : ei) : 0x7fffffffu;
+    const unsigned key = mine ? (unsigned)ei : 0x7fffffffu;
     const unsigned kmin = __reduce_min_sync(0xffffffffu, key);
     const unsigned who = __ballot_sync(0xffffffffu, mine && key == kmin);
     best_pos = who ? __shfl_sync(0xffffffffu, ei, __ffs(who) - 1) : 0x7fffffff;
@@ -184,33 +180,48 @@ __device__ __forceinline__ void warp_cloud_exact_min(const float4* cloud, int nc
   }
 }
 
+// One matrix entry from its two directed sums: M[i,j] (+ mirror) and the fused MMD/COV/1-NNA reductions.
+__device__ __forceinline__ void emit_entry(const Params& p, int ci, int cj, double S0, double S1) {
+  const float v = (float)(S0 / (double)p.countX) + (float)(S1 / (double)p.countY);
+  if (p.M) {
+    p.M[(long long)(p.compact_rows ? (int)blockIdx.y : ci) * p.ldm + cj] = v;
+    if (p.symmetric && p.mirror && ci != cj) p.M[(long long)cj * p.ldm + ci] = v;
+  }
+  // fused _compute_cov_mmd / _compute_nna(k=1) reductions (reference cov_mmd_1nna.py:54-106): v >= 0, so
+  // (bits << 32 | index) orders by value, then by index -- torch's lowest-index tie rule on this path
+  if (p.keys) {
+    const int gi = p.offX + ci, gj = p.offY + cj;
+    if (gi != gj) {                                              // the +inf diagonal of _compute_nna
+      const unsigned long long vb = (unsigned long long)__float_as_uint(v) << 32;
+      atomicMin(p.keys + gj, vb | (unsigned)gi);
+      atomicMin(p.keys + gi, vb | (unsigned)gj);
+      const int lo = min(gi, gj), hi = max(gi, gj);
+      if (lo < p.n_ref && hi >= p.n_ref) {                       // an entry of M_rg: lo is the reference cloud
+        atomicMin(p.keys + p.n_total + hi, vb | (unsigned)lo);
+        atomicMin(p.keys + 2 * (long long)p.n_total + lo, vb | (unsigned)hi);
+      }
+    }
+  }
+}
+
 // NT threads per CTA. The register tile of R = 8 rows per thread is what makes the search FMA-bound
 // (one LDS.128 pair feeds 24 FFMA2), so small clouds keep R = 8 and shrink the CTA instead: 2048 rows
-// -> 256 threads, 1024 -> 128, 512 -> 64, 256 -> 32 (the matrix front end's table, pick_shape). Every
+// -> 256 threads, 1024 -> 128, 512 -> 64, 256 -> 32 (the matrix front end's table, dispatch_matrix). Every
 // shape keeps 16 warps of 128 registers per SM; the R < 8 instantiations (batch front end on small
 // batches, odd sizes) trade registers for residency because their CTAs are short.
-// TL = candidates per shared-memory tile. Pruned launches on sorted clouds use small CTAs with small tiles
-// (NT = 64, TL = 512): pruning is per warp, so in a wide CTA most warps find nothing to scan in a given tile and wait
-// at the tile barrier for the one or two that do (ncu: barrier stall 4.1 warps per issue with 8 warps per CTA);
-// two warps per CTA wait for each other only, and twelve such CTAs fit an SM.
-template <int R, bool MATRIX, bool MERGED, int NT = TPB, int TL = TILE>
-__global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) / NT : (R >= 8 ? 512 / NT : (R == 4 ? 3 : 4))) nn_kernel(const Params p) {
+// MERGED: merged-origin clouds (prep_merge_kernel) too large for the sort, in the matrix front end.
+template <int R, bool MATRIX, bool MERGED, int NT = TPB>
+__global__ void __launch_bounds__(NT, R >= 8 ? 512 / NT : (R == 4 ? 3 : 4)) nn_kernel(const Params p) {
+  static_assert(!MERGED || MATRIX, "merged origins are a matrix front end layout");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float4* const tiles = reinterpret_cast<float4*>(smem_raw);
   __shared__ uint64_t bars[2];
   __shared__ double red[NT / 32];
-  // merged + sorted clouds (prep_sort_kernel): per-chunk bounding boxes of the tile in flight (two buffers)
-  // and the box of each warp's rows; dist1 / dist2 carry the X / Y side box tables (null: no pruning)
-  __shared__ float4 sbox[MERGED ? 2 * 2 * (TL / CHUNK) : 1];
-  __shared__ float4 wbox[MERGED ? 2 * (NT / 32) : 1];
-  const float4* const bxX = MERGED ? p.boxX : nullptr;
-  const float4* const bxY = MERGED ? p.boxY : nullptr;
-  const bool prune = MERGED && bxX != nullptr;
 
   constexpr int RB = NT * R;
   // candidates per search chunk = the window the exact pass re-evaluates per row and tile. Small clouds (the
   // shrunken CTAs) take 16: the exact pass is a fixed cost per row, 14 % of the search at 512 points with 32.
-  constexpr int CH = (NT < TPB && !MERGED) ? CHUNK / 2 : CHUNK;      // merged clouds: one bounding box per 32 candidates
+  constexpr int CH = (NT < TPB && !MERGED) ? CHUNK / 2 : CHUNK;      // merged clouds: the DEFERRED pass reads whole chunks
   constexpr int PR = CH / 2;
   const int tid = threadIdx.x;
   const int lane = tid & 31;
@@ -226,8 +237,7 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
     ci = cj = blockIdx.y;
     dir_only = blockIdx.z;
     rb_only = blockIdx.x;
-    int rows_here = dir_only == 0 ? p.countX : p.countY;
-    if (MERGED) rows_here = (dir_only == 0 ? p.metaX[ci] : p.metaY[cj]).x;
+    const int rows_here = dir_only == 0 ? p.countX : p.countY;
     if (rb_only >= (rows_here + RB - 1) / RB) return;
   }
   const float4* const sx = p.scanX + (long long)ci * p.strideX;
@@ -246,7 +256,7 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
 #define K_paddedX (MERGED ? (mx.x + CHUNK - 1) / CHUNK * CHUNK : p.paddedX)
 #define K_paddedY (MERGED ? (my.x + CHUNK - 1) / CHUNK * CHUNK : p.paddedY)
 
-  const int ntX = (K_paddedX + TL - 1) / TL, ntY = (K_paddedY + TL - 1) / TL;
+  const int ntX = (K_paddedX + TILE - 1) / TILE, ntY = (K_paddedY + TILE - 1) / TILE;
   const int nrbX = (K_countX + RB - 1) / RB, nrbY = (K_countY + RB - 1) / RB;
   const int seg0 = nrbX * ntY;
   int pos_begin, pos_end;
@@ -256,58 +266,29 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
 
   // the two tile buffers are as large as the largest tile of this launch (launch_nn sizes the dynamic shared
   // memory the same way): small clouds leave room for more resident CTAs to hide the per-entry prologue
-  const int tstride = (R >= 8 && NT == TPB) ? TL : min(TL, max(p.paddedX, p.paddedY));
+  const int tstride = (R >= 8 && NT == TPB) ? TILE : min(TILE, max(p.paddedX, p.paddedY));
   if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_fence_init(); }
   __syncthreads();
 
-  // With pruning a row block starts on the tile at its own relative position in the (spatially sorted)
-  // other cloud, where its nearest neighbours most likely are: the bound it leaves prunes the other tiles.
-  auto tile_of = [&](int dir, int rb, int t) -> int {
-    if (!prune) return t;
-    const int nt = dir == 0 ? ntY : ntX, nrb = dir == 0 ? nrbX : nrbY;
-    return (t + rb * nt / nrb) % nt;
-  };
-  // tile stream: position -> (direction, row block, scan tile)
+  // tile stream: position -> (direction, scan tile)
   auto issue = [&](int pos, int buf) {
     int dir, t;
-    if (!MERGED) {
-      if (pos < seg0) { dir = 0; t = pos % ntY; } else { dir = 1; t = (pos - seg0) % ntX; }
-    } else {
-      int rb;
-      if (pos < seg0) { dir = 0; rb = pos / ntY; t = pos - rb * ntY; } else { dir = 1; const int q = pos - seg0; rb = q / ntX; t = q - rb * ntX; }
-      t = tile_of(dir, rb, t);
-    }
-    const float4* src = (dir == 0 ? sy : sx) + (long long)t * TL;
+    if (pos < seg0) { dir = 0; t = pos % ntY; } else { dir = 1; t = (pos - seg0) % ntX; }
+    const float4* src = (dir == 0 ? sy : sx) + (long long)t * TILE;
     const int padded = dir == 0 ? K_paddedY : K_paddedX;
-    const int npts = min(TL, padded - t * TL);
-    if (MERGED && prune) {
-      const float4* bsrc = (dir == 0 ? bxY + (long long)cj * (p.paddedY / CHUNK * 2) : bxX + (long long)ci * (p.paddedX / CHUNK * 2)) +
-                           t * (TL / CHUNK * 2);
-      const uint32_t bbytes = (uint32_t)(npts / CHUNK) * 32u;
-      mbar_expect_tx(&bars[buf], (uint32_t)npts * 16u + bbytes);
-      bulk_g2s(tiles + buf * tstride, src, (uint32_t)npts * 16u, &bars[buf]);
-      bulk_g2s(sbox + buf * (2 * (TL / CHUNK)), bsrc, bbytes, &bars[buf]);
-      return;
-    }
+    const int npts = min(TILE, padded - t * TILE);
     mbar_expect_tx(&bars[buf], (uint32_t)npts * 16u);
     bulk_g2s(tiles + buf * tstride, src, (uint32_t)npts * 16u, &bars[buf]);
   };
   if (tid == 0) issue(pos_begin, 0);
 
-  // Batch front end on sorted clouds: a candidate's position is not its index. Ties between bit-equal distances go
-  // to the lowest ORIGINAL index (the reference's rule, SURVEY.md S6), looked up only when a tie actually occurs.
-  auto before = [&](int dir, int posA, int posB) -> bool {
-    if (!MERGED) return posA < posB;
-    const int* pm = dir == 0 ? p.permY + (long long)cj * p.strideY : p.permX + (long long)ci * p.strideX;
-    return pm[posA] < pm[posB];
-  };
   f32x2 nax[R], nay[R], naz[R];     // {-2a, -2a}: search operands; ptxas folds the pair into FFMA2's scalar-broadcast form
   float eb[R];                      // exact running minimum over tiles
   int ei[R];                        // its index (batch front end only)
   // search state: best and runner-up chunk minima of |b|^2 - 2 a.b and the best chunk's number. Dense clouds
   // restart it for every tile (the exact pass follows the tile); merged clouds carry it across all tiles of a row
-  // block and defer the exact pass to the end (see DEFERRED below), an[] = |a|^2 turns it into a distance bound.
-  float cur[R], sec[R], an[R];
+  // block and defer the exact pass to the end (see DEFERRED below).
+  float cur[R], sec[R];
   int cid[R];
   double dsum = 0.0, S0 = 0.0;
 
@@ -336,113 +317,22 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
         naz[r] = pack2(mz, mz);
         eb[r] = __int_as_float(0x7f800000);
         ei[r] = 0;
-        if (MERGED) {
-          cur[r] = sec[r] = __int_as_float(0x7f800000); cid[r] = 0;
-          an[r] = 0.25f * fmaf(mz, mz, fmaf(mx, mx, my * my));
-        }
-      }
-      if (MERGED && prune) {            // bounding box of this warp's live rows (a = -0.5 * (-2a) exactly)
-        const float inf = __int_as_float(0x7f800000);
-        float l0 = inf, l1 = inf, l2 = inf, h0 = -inf, h1 = -inf, h2 = -inf;
-        #pragma unroll
-        for (int r = 0; r < R; ++r) {
-          if (K_ROW(r) < rowcount) {
-            float ax, ay, az, dummy;
-            unpack2(nax[r], ax, dummy); unpack2(nay[r], ay, dummy); unpack2(naz[r], az, dummy);
-            ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
-            l0 = fminf(l0, ax); l1 = fminf(l1, ay); l2 = fminf(l2, az);
-            h0 = fmaxf(h0, ax); h1 = fmaxf(h1, ay); h2 = fmaxf(h2, az);
-          }
-        }
-        #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-          l0 = fminf(l0, __shfl_xor_sync(0xffffffffu, l0, o)); h0 = fmaxf(h0, __shfl_xor_sync(0xffffffffu, h0, o));
-          l1 = fminf(l1, __shfl_xor_sync(0xffffffffu, l1, o)); h1 = fmaxf(h1, __shfl_xor_sync(0xffffffffu, h1, o));
-          l2 = fminf(l2, __shfl_xor_sync(0xffffffffu, l2, o)); h2 = fmaxf(h2, __shfl_xor_sync(0xffffffffu, h2, o));
-        }
-        if (lane == 0) { wbox[2 * (tid >> 5)] = make_float4(l0, l1, l2, 0.f); wbox[2 * (tid >> 5) + 1] = make_float4(h0, h1, h2, 0.f); }
-        __syncwarp();
+        if (MERGED) { cur[r] = sec[r] = __int_as_float(0x7f800000); cid[r] = 0; }
       }
     }
 
     mbar_wait(&bars[buf], (uint32_t)((it >> 1) & 1));
     const float4* const tp = tiles + buf * tstride;
-    const int te = MERGED ? tile_of(dir, rb, t) : t;     // which tile of the scanned cloud this buffer holds
-    const int nch = min(TL, scanpadded - te * TL) / CH;
+    const int nch = min(TILE, scanpadded - t * TILE) / CH;
 
     if (!MERGED || rb * RB + (tid >> 5) * (32 * R) < rowcount) {      // warp-uniform
-    // ---- pruning (merged + sorted clouds): chunks whose box is no closer to the box of this warp's rows than
-    //      every current minimum of those rows cannot lower any of them. LB is the reference's distance formula
-    //      on the per-axis gaps: each of its operations is monotone in |dx|,|dy|,|dz| and so is rounding, hence
-    //      LB <= d(a,b) in floating point for every row a of the warp and candidate b of the chunk.
-    unsigned long long vmask = ~0ull;
-    if (MERGED && prune) {
-      // DEFERRED: no exact minimum exists yet; cur + |a|^2 estimates the best candidate's distance within the search's
-      // rounding error u (21 |a|^2 + 15 D) (search_window), the reference formula adds 5 u D: 64 u (|a|^2 + D) on top
-      // is a rigorous upper bound of the row's final (exact) minimum, hence of anything a chunk must beat or tie.
-      float m = 0.0f;
-      #pragma unroll
-      for (int r = 0; r < R; ++r) {
-        if (K_ROW(r) < rowcount) {
-          const float dest = fmaxf(cur[r] + an[r], 0.0f);
-          m = fmaxf(m, fmaf(3.81469727e-6f /* 64 * 2^-24 */, an[r] + dest, dest) + 1e-36f);
-        }
-      }
-      const float ubmax = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m)));   // >= 0; +inf before the first tile
-      const float4 rl = wbox[2 * (tid >> 5)], rh = wbox[2 * (tid >> 5) + 1];
-      const float4* const sb = sbox + buf * (2 * (TL / CHUNK));
-      unsigned part[2];
-      #pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int c = h * 32 + lane;
-        bool visit = false;
-        if (c < nch) {
-          const float4 bl = sb[2 * c], bh = sb[2 * c + 1];
-          const float gx = max3(0.0f, bl.x - rh.x, rl.x - bh.x);
-          const float gy = max3(0.0f, bl.y - rh.y, rl.y - bh.y);
-          const float gz = max3(0.0f, bl.z - rh.z, rl.z - bh.z);
-          const float lb = fmaf(gz, gz, fmaf(gx, gx, __fmul_rn(gy, gy)));
-          visit = lb <= ubmax;      // a chunk that can only TIE the minimum may still hold the lower index (batch front end)
-        }
-        part[h] = __ballot_sync(0xffffffffu, visit);
-      }
-      vmask = (unsigned long long)part[0] | ((unsigned long long)part[1] << 32);
-    }
     // ---- search: which chunk of this tile holds the smallest |b|^2 - 2 a.b ----
     if (!MERGED) {
       #pragma unroll
       for (int r = 0; r < R; ++r) { cur[r] = sec[r] = __int_as_float(0x7f800000); cid[r] = 0; }
     }
-    const int cbase = MERGED ? te * (TL / CH) : 0;      // merged clouds number their chunks through the whole cloud
-    // second pruning level (sorted clouds): a chunk that passed the box-to-box test is scanned only if SOME row of the
-    // warp can still gain from it -- the row's own distance to the chunk's box (the same monotone formula, a point
-    // being a degenerate box) against the row's own bound: one far-away row no longer opens the chunk for all 32 R rows
-    float ubr[R];
-    if (MERGED && prune) {
-      #pragma unroll
-      for (int r = 0; r < R; ++r) {
-        const float dest = fmaxf(cur[r] + an[r], 0.0f);
-        ubr[r] = K_ROW(r) < rowcount ? fmaf(3.81469727e-6f, an[r] + dest, dest) + 1e-36f : -1.0f;      // dead rows never ask
-      }
-    }
-    int nvis = 0;
+    const int cbase = MERGED ? t * (TILE / CH) : 0;      // merged clouds number their chunks through the whole cloud
     for (int c = 0; c < nch; ++c) {
-      if (MERGED && !((vmask >> c) & 1ull)) continue;      // warp-uniform
-      if (MERGED && prune) {
-        const float4* const sb = sbox + buf * (2 * (TL / CHUNK));
-        const float4 bl = sb[2 * c], bh = sb[2 * c + 1];
-        bool need = false;
-        #pragma unroll
-        for (int r = 0; r < R; ++r) {
-          float ax, ay, az, dummy;
-          unpack2(nax[r], ax, dummy); unpack2(nay[r], ay, dummy); unpack2(naz[r], az, dummy);
-          ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
-          const float gx = max3(0.0f, bl.x - ax, ax - bh.x), gy = max3(0.0f, bl.y - ay, ay - bh.y), gz = max3(0.0f, bl.z - az, az - bh.z);
-          need |= fmaf(gz, gz, fmaf(gx, gx, __fmul_rn(gy, gy))) <= ubr[r];
-        }
-        if (!__any_sync(0xffffffffu, need)) continue;      // warp-uniform
-      }
-      ++nvis;
       const float4* cp = tp + c * CH;
       float cm[R];
       #pragma unroll
@@ -471,7 +361,7 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
 
     if (MERGED && p.visited != nullptr && lane == 0) {          // bench.py's executed-flop count for pruned workloads
       const int first = rb * RB + (tid >> 5) * (32 * R);
-      atomicAdd(p.visited, (unsigned long long)nvis * CH * (unsigned long long)min(32 * R, rowcount - first));
+      atomicAdd(p.visited, (unsigned long long)nch * CH * (unsigned long long)min(32 * R, rowcount - first));
     }
     // ---- exact: re-evaluate the winning chunk with the reference's rounding ----
     constexpr int G = R < 4 ? R : 4;
@@ -505,9 +395,9 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
           if (MATRIX) {
             e[r] = min3(e[r], lo, hi);
           } else {
-            const int i0 = te * TL + cid[g + r] * CH + 2 * kk;
-            if (lo < e[r] || (lo == e[r] && (eidx[r] == 0x7fffffff || before(dir, i0, eidx[r])))) { e[r] = lo; eidx[r] = i0; }
-            if (hi < e[r] || (hi == e[r] && (eidx[r] == 0x7fffffff || before(dir, i0 + 1, eidx[r])))) { e[r] = hi; eidx[r] = i0 + 1; }
+            const int i0 = t * TILE + cid[g + r] * CH + 2 * kk;
+            if (lo < e[r] || (lo == e[r] && (eidx[r] == 0x7fffffff || i0 < eidx[r]))) { e[r] = lo; eidx[r] = i0; }
+            if (hi < e[r] || (hi == e[r] && (eidx[r] == 0x7fffffff || i0 + 1 < eidx[r]))) { e[r] = hi; eidx[r] = i0 + 1; }
           }
         }
       }
@@ -515,8 +405,8 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
       for (int r = 0; r < G; ++r) {
         if (MATRIX) {
           eb[g + r] = fminf(eb[g + r], e[r]);
-        } else if (e[r] < eb[g + r] || (MERGED && e[r] == eb[g + r] && eidx[r] != 0x7fffffff && before(dir, eidx[r], ei[g + r]))) {
-          eb[g + r] = e[r];                        // dense clouds: tiles ascend, so the lowest index keeps ties by itself
+        } else if (e[r] < eb[g + r]) {
+          eb[g + r] = e[r];                        // tiles ascend, so the lowest index keeps ties by itself
           ei[g + r] = eidx[r];
         }
       }
@@ -536,16 +426,14 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
           flagged &= flagged - 1;
           float m;
           int mi = 0;
-          const int* tile_perm = nullptr;
-          if (MERGED && !MATRIX) tile_perm = (dir == 0 ? p.permY + (long long)cj * p.strideY : p.permX + (long long)ci * p.strideX) + te * TL;
           warp_tile_exact_min<!MATRIX>(tp, nch * PR, __shfl_sync(0xffffffffu, ax, src), __shfl_sync(0xffffffffu, ay, src),
-                                       __shfl_sync(0xffffffffu, az, src), lane, tile_perm, m, mi);
+                                       __shfl_sync(0xffffffffu, az, src), lane, m, mi);
           if (lane == src) {
             if (MATRIX) {
               eb[r] = fminf(eb[r], m);
             } else if (mi != 0x7fffffff) {
-              mi += te * TL;
-              if (m < eb[r] || (m == eb[r] && before(dir, mi, ei[r]))) { eb[r] = m; ei[r] = mi; }
+              mi += t * TILE;
+              if (m < eb[r] || (m == eb[r] && mi < ei[r])) { eb[r] = m; ei[r] = mi; }
             }
           }
         }
@@ -556,12 +444,9 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
 
     // ---- DEFERRED (merged clouds): after the last tile of a row block, the exact pass on each row's winning chunk
     //      and the guard over the whole cloud, both straight from global memory (L2): once per row block instead
-    //      of once per tile, which is what lets pruned launches use small tiles and small CTAs ----
+    //      of once per tile ----
     if (MERGED && t == nt - 1 && rb * RB + (tid >> 5) * (32 * R) < rowcount) {      // warp-uniform
       const float4* const cand = dir == 0 ? sy : sx;
-      const int* const cperm = MATRIX ? nullptr : (dir == 0 ? p.permY + (long long)cj * p.strideY : p.permX + (long long)ci * p.strideX);
-      const float4* const cboxes = !prune ? nullptr
-          : (dir == 0 ? bxY + (long long)cj * (p.paddedY / CHUNK * 2) : bxX + (long long)ci * (p.paddedX / CHUNK * 2));
       #pragma unroll
       for (int r = 0; r < R; ++r) {
         float ax, ay, az, dummy;
@@ -569,7 +454,6 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
         ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
         const bool live = K_ROW(r) < rowcount;
         float e = __int_as_float(0x7f800000);
-        int eidx = 0x7fffffff;
         if (live && cur[r] < __int_as_float(0x7f800000)) {
           const f32x2 ax2 = pack2(ax, ax), ay2 = pack2(ay, ay), az2 = pack2(az, az);
           const float4* cp = cand + (long long)cid[r] * CHUNK;
@@ -581,34 +465,20 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
             const f32x2 dz = sub2(pack2(q1.x, q1.y), az2);
             float lo, hi;
             unpack2(fma2(dz, dz, fma2(dx, dx, mul2(dy, dy))), lo, hi);
-            if (MATRIX) {
-              e = min3(e, lo, hi);
-            } else {
-              const int i0 = cid[r] * CHUNK + 2 * k;
-              if (lo < e || (lo == e && eidx != 0x7fffffff && cperm[i0] < cperm[eidx])) { e = lo; eidx = i0; }
-              if (hi < e || (hi == e && eidx != 0x7fffffff && cperm[i0 + 1] < cperm[eidx])) { e = hi; eidx = i0 + 1; }
-            }
+            e = min3(e, lo, hi);
           }
         }
         eb[r] = e;
-        ei[r] = eidx;
         const bool near_tie = live && sec[r] <= cur[r] + search_window(ax, ay, az, cur[r]);
         unsigned flagged = __ballot_sync(0xffffffffu, near_tie);
         while (flagged) {                         // warp-uniform
           const int src = __ffs(flagged) - 1;
           flagged &= flagged - 1;
           float m;
-          int mi = 0x7fffffff;
-          warp_cloud_exact_min<!MATRIX>(cand, scanpadded / CHUNK, cboxes, __shfl_sync(0xffffffffu, e, src),
-                                        __shfl_sync(0xffffffffu, ax, src), __shfl_sync(0xffffffffu, ay, src),
-                                        __shfl_sync(0xffffffffu, az, src), lane, cperm, m, mi);
-          if (lane == src) {
-            if (MATRIX) {
-              eb[r] = fminf(eb[r], m);
-            } else if (mi != 0x7fffffff && (m < eb[r] || (m == eb[r] && (ei[r] == 0x7fffffff || cperm[mi] < cperm[ei[r]])))) {
-              eb[r] = m; ei[r] = mi;
-            }
-          }
+          int mi;
+          warp_cloud_exact_min<false>(cand, scanpadded / CHUNK, nullptr, 0.0f, __shfl_sync(0xffffffffu, ax, src),
+                                      __shfl_sync(0xffffffffu, ay, src), __shfl_sync(0xffffffffu, az, src), lane, nullptr, m, mi);
+          if (lane == src) eb[r] = fminf(eb[r], m);
         }
       }
     }
@@ -625,15 +495,9 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
           } else {
             float* dist = dir == 0 ? p.dist1 : p.dist2;
             int* idx = dir == 0 ? p.idx1 : p.idx2;
-            if (MERGED) {      // per sorted position (stride = padded count); scattered to the original order afterwards
-              const long long o = (long long)ci * (dir == 0 ? p.strideX : p.strideY) + row;
-              dist[o] = eb[r];
-              idx[o] = (dir == 0 ? p.permY + (long long)cj * p.strideY : p.permX + (long long)ci * p.strideX)[ei[r] == 0x7fffffff ? 0 : ei[r]];
-            } else {
-              const long long o = (long long)ci * rowcount + row;
-              dist[o] = eb[r];
-              if (idx) idx[o] = ei[r] == 0x7fffffff ? 0 : ei[r];
-            }
+            const long long o = (long long)ci * rowcount + row;
+            dist[o] = eb[r];
+            if (idx) idx[o] = ei[r] == 0x7fffffff ? 0 : ei[r];
           }
         }
       }
@@ -644,28 +508,7 @@ __global__ void __launch_bounds__(NT, NT < TPB && MERGED ? (R >= 8 ? 512 : 640) 
 
   if (MATRIX) {
     const double S1 = block_sum<NT>(dsum, red);
-    if (tid == 0) {
-      const float v = (float)(S0 / (double)p.countX) + (float)(S1 / (double)p.countY);
-      if (p.M) {
-        p.M[(long long)(p.compact_rows ? (int)blockIdx.y : ci) * p.ldm + cj] = v;
-        if (p.symmetric && p.mirror && ci != cj) p.M[(long long)cj * p.ldm + ci] = v;
-      }
-      // fused _compute_cov_mmd / _compute_nna(k=1) reductions (reference cov_mmd_1nna.py:54-106): v >= 0, so
-      // (bits << 32 | index) orders by value, then by index -- torch's lowest-index tie rule on this path
-      if (p.keys) {
-        const int gi = p.offX + ci, gj = p.offY + cj;
-        if (gi != gj) {                                              // the +inf diagonal of _compute_nna
-          const unsigned long long vb = (unsigned long long)__float_as_uint(v) << 32;
-          atomicMin(p.keys + gj, vb | (unsigned)gi);
-          atomicMin(p.keys + gi, vb | (unsigned)gj);
-          const int lo = min(gi, gj), hi = max(gi, gj);
-          if (lo < p.n_ref && hi >= p.n_ref) {                       // an entry of M_rg: lo is the reference cloud
-            atomicMin(p.keys + p.n_total + hi, vb | (unsigned)lo);
-            atomicMin(p.keys + 2 * (long long)p.n_total + lo, vb | (unsigned)hi);
-          }
-        }
-      }
-    }
+    if (tid == 0) emit_entry(p, ci, cj, S0, S1);
   }
 }
 
@@ -710,7 +553,6 @@ __global__ void __launch_bounds__(256) prep_kernel(const float* __restrict__ xyz
 __global__ void __launch_bounds__(256) prep_merge_kernel(const float* __restrict__ xyz, int count, long long stride,
                                                          float4* __restrict__ out, int2* __restrict__ meta) {
   __shared__ int wsum[8];
-  __shared__ int s_total;
   const long long c = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const float* src = xyz + c * count * 3;
@@ -749,10 +591,11 @@ __global__ void __launch_bounds__(256) prep_merge_kernel(const float* __restrict
 
 // Merged origins + spatial order (clouds of at most SORT_CAP points): the kept points are sorted by a
 // Morton cell key (x, y interleaved at 7 bits each, z 1 bit, ties by original index, so the order is
-// deterministic) with a bitonic network in shared memory, written in scan format, and every 32-candidate
-// chunk gets its bounding box. The matrix kernel then skips a chunk whenever the gap between the chunk's
-// box and the box of a warp's 256 rows is already no smaller than every current minimum of those rows:
-// exact, because every operation of the distance is monotone in |dx|,|dy|,|dz| and so is rounding.
+// deterministic) or into k-d order (below) with bitonic networks in shared memory, written in scan format,
+// and every 32-candidate chunk and every block of 32 chunks gets its bounding box. The pair and walk kernels
+// skip a chunk whenever the gap between the chunk's box and a row or a row group's box is already no smaller
+// than the current minima of those rows: exact, because every operation of the distance is monotone in
+// |dx|,|dy|,|dz| and so is rounding.
 constexpr int SORT_CAP = 32768;
 constexpr int SORT_TPB = 1024;
 constexpr int WALK_BLOCKS = SORT_CAP / CHUNK / 32;      // blocks of 32 chunks per cloud (upper level of the best-first walk)
@@ -980,10 +823,10 @@ __global__ void __launch_bounds__(NT, NT == 1024 ? 1 : 6) prep_sort_kernel(const
     }
     float* q = dst + (size_t)(pos >> 1) * 8 + (pos & 1);     // {x0,x1,y0,y1}{z0,z1,n0,n1}
     q[0] = x; q[2] = y; q[4] = z; q[6] = n;
-    // consumers that walk chunks by box bound (block_boxes != null): the merged origin point stays outside its chunk's
-    // box (it would stretch the last leaf's box to the sensor) and the chunk is flagged in .w: always visited
-    const bool sep = block_boxes != nullptr && zeros > 0;
-    const bool real = pos < (sep ? total : kept);
+    // the merged origin point stays outside its chunk's box (it would stretch the last leaf's box to the sensor) and
+    // the chunk is flagged in .w: the walks always visit it
+    const bool sep = zeros > 0;
+    const bool real = pos < total;
     float l0 = real ? x : inf, l1 = real ? y : inf, l2 = real ? z : inf;
     float h0 = real ? x : -inf, h1 = real ? y : -inf, h2 = real ? z : -inf;
     #pragma unroll
@@ -998,23 +841,21 @@ __global__ void __launch_bounds__(NT, NT == 1024 ? 1 : 6) prep_sort_kernel(const
     }
   }
   if (tid == 0) meta[c] = make_int2(kept, zeros > 0 ? zeros : 1);
-  // ---- boxes of the blocks of 32 chunks (the upper level of nn_walk_kernel's best-first walk); empty: (+inf, -inf) ----
-  if (block_boxes != nullptr) {
-    __syncthreads();                            // this CTA's chunk boxes are visible
-    float4* const bb = block_boxes + c * (2 * WALK_BLOCKS);
-    const int nchunks = padded / CHUNK;
-    for (int b = warp; b < WALK_BLOCKS; b += NT / 32) {
-      const int chunk = b * 32 + lane;
-      float4 bl = make_float4(inf, inf, inf, 0.f), bh = make_float4(-inf, -inf, -inf, 0.f);
-      if (chunk < nchunks) { bl = bdst[2 * chunk]; bh = bdst[2 * chunk + 1]; }
-      #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        bl.x = fminf(bl.x, __shfl_xor_sync(0xffffffffu, bl.x, o)); bh.x = fmaxf(bh.x, __shfl_xor_sync(0xffffffffu, bh.x, o));
-        bl.y = fminf(bl.y, __shfl_xor_sync(0xffffffffu, bl.y, o)); bh.y = fmaxf(bh.y, __shfl_xor_sync(0xffffffffu, bh.y, o));
-        bl.z = fminf(bl.z, __shfl_xor_sync(0xffffffffu, bl.z, o)); bh.z = fmaxf(bh.z, __shfl_xor_sync(0xffffffffu, bh.z, o));
-      }
-      if (lane == 0) { bb[2 * b] = bl; bb[2 * b + 1] = bh; }
+  // ---- boxes of the blocks of 32 chunks (the upper level of nn_walk_split_kernel's best-first walk); empty: (+inf, -inf) ----
+  __syncthreads();                              // this CTA's chunk boxes are visible
+  float4* const bb = block_boxes + c * (2 * WALK_BLOCKS);
+  const int nchunks = padded / CHUNK;
+  for (int b = warp; b < WALK_BLOCKS; b += NT / 32) {
+    const int chunk = b * 32 + lane;
+    float4 bl = make_float4(inf, inf, inf, 0.f), bh = make_float4(-inf, -inf, -inf, 0.f);
+    if (chunk < nchunks) { bl = bdst[2 * chunk]; bh = bdst[2 * chunk + 1]; }
+    #pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      bl.x = fminf(bl.x, __shfl_xor_sync(0xffffffffu, bl.x, o)); bh.x = fmaxf(bh.x, __shfl_xor_sync(0xffffffffu, bh.x, o));
+      bl.y = fminf(bl.y, __shfl_xor_sync(0xffffffffu, bl.y, o)); bh.y = fmaxf(bh.y, __shfl_xor_sync(0xffffffffu, bh.y, o));
+      bl.z = fminf(bl.z, __shfl_xor_sync(0xffffffffu, bl.z, o)); bh.z = fmaxf(bh.z, __shfl_xor_sync(0xffffffffu, bh.z, o));
     }
+    if (lane == 0) { bb[2 * b] = bl; bb[2 * b + 1] = bh; }
   }
 }
 
@@ -1089,16 +930,16 @@ static int pick_r(int maxcount) {
   return 1;
 }
 
-template <int R, bool MATRIX, bool MERGED, int NT = TPB, int TL = TILE>
+template <int R, bool MATRIX, bool MERGED, int NT = TPB>
 static int launch_nn(const Params& p, dim3 grid, cudaStream_t st) {
   static bool configured[kMaxDevices] = {};   // per instantiation and device: the attribute is per context
   const int dev = current_device();
   if (!configured[dev]) {
-    DUSTY_CUDA(cudaFuncSetAttribute(nn_kernel<R, MATRIX, MERGED, NT, TL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * TL * 16));
+    DUSTY_CUDA(cudaFuncSetAttribute(nn_kernel<R, MATRIX, MERGED, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * TILE * 16));
     configured[dev] = true;
   }
-  const int tile_pts = (R >= 8 && NT == TPB) ? TL : std::min(TL, std::max(p.paddedX, p.paddedY));
-  nn_kernel<R, MATRIX, MERGED, NT, TL><<<grid, NT, 2 * (size_t)tile_pts * 16, st>>>(p);
+  const int tile_pts = (R >= 8 && NT == TPB) ? TILE : std::min(TILE, std::max(p.paddedX, p.paddedY));
+  nn_kernel<R, MATRIX, MERGED, NT><<<grid, NT, 2 * (size_t)tile_pts * 16, st>>>(p);
   DUSTY_AFTER_LAUNCH("chamfer nn_kernel");
   return 0;
 }
@@ -1112,13 +953,13 @@ static int dispatch_matrix(int maxcount, const Params& p, dim3 grid, cudaStream_
   return launch_nn<4, true, false, 32>(p, grid, st);
 }
 
-template <bool MATRIX, bool MERGED>
-static int dispatch_nn(int r, const Params& p, dim3 grid, cudaStream_t st) {
+// Dense batch front end: R rows per thread, see dusty_chamfer_forward.
+static int dispatch_batch(int r, const Params& p, dim3 grid, cudaStream_t st) {
   switch (r) {
-    case 8: return launch_nn<8, MATRIX, MERGED>(p, grid, st);
-    case 4: return launch_nn<4, MATRIX, MERGED>(p, grid, st);
-    case 2: return launch_nn<2, MATRIX, MERGED>(p, grid, st);
-    default: return launch_nn<1, MATRIX, MERGED>(p, grid, st);
+    case 8: return launch_nn<8, false, false>(p, grid, st);
+    case 4: return launch_nn<4, false, false>(p, grid, st);
+    case 2: return launch_nn<2, false, false>(p, grid, st);
+    default: return launch_nn<1, false, false>(p, grid, st);
   }
 }
 
@@ -1159,10 +1000,9 @@ __global__ void __launch_bounds__(256) unsort_kernel(const float* __restrict__ d
   if (idx) idx[g] = idx_sorted[o];
 }
 
-static SortSide sort_side(const float* xyz, long long clouds, int count, float4* out, int2* meta, float4* boxes, int* perm, int* inv,
-                          bool walkable) {
+static SortSide sort_side(const float* xyz, long long clouds, int count, float4* out, int2* meta, float4* boxes, int* perm, int* inv) {
   return SortSide{xyz, count, (long long)padded_of(count), out, meta, boxes, padded_of(count) / CHUNK * 2, perm, inv,
-                  walkable ? block_boxes_of(boxes, clouds, count) : nullptr};
+                  block_boxes_of(boxes, clouds, count)};
 }
 
 template <bool KD, int NT>
@@ -1180,26 +1020,17 @@ static int launch_prep_sort(const SortArgs& a, long long clouds, int maxcount, c
   return 0;
 }
 
-// walkable: for the pair / walk kernels (block boxes, origin kept out of its chunk's box); kd: k-d order (Morton otherwise).
-// clouds1 > 0: a second set in the same launch.
-static int run_prep_sort2(const SortSide& s0, long long clouds0, const SortSide& s1, long long clouds1, cudaStream_t st, bool walkable,
-                          bool kd) {
+// kd: k-d order (Morton otherwise). clouds1 > 0: a second set in the same launch.
+static int run_prep_sort2(const SortSide& s0, long long clouds0, const SortSide& s1, long long clouds1, cudaStream_t st, bool kd) {
   if (clouds0 + clouds1 == 0) return 0;
   if (clouds0 + clouds1 > 0x7fffffffLL) return fail_arg(DUSTY_EINVAL, "chamfer: too many clouds in one sort launch");
   SortArgs a{};
   a.s[0] = s0; a.s[1] = clouds1 > 0 ? s1 : s0; a.clouds0 = (int)clouds0;
   const int maxcount = clouds1 > 0 && s1.count > s0.count ? s1.count : s0.count;
-  static const bool small_ctas = [] { const char* e = getenv("DUSTY_CHAMFER_SORT_SMALL"); return !(e && e[0] == '0'); }();   // A/B
   const long long clouds = clouds0 + clouds1;
-  if (maxcount <= 4096 && small_ctas)
-    return walkable && kd ? launch_prep_sort<true, 256>(a, clouds, maxcount, st) : launch_prep_sort<false, 256>(a, clouds, maxcount, st);
-  return walkable && kd ? launch_prep_sort<true, SORT_TPB>(a, clouds, maxcount, st) : launch_prep_sort<false, SORT_TPB>(a, clouds, maxcount, st);
-}
-
-static int run_prep_sort(const float* xyz, long long clouds, int count, float4* out, int2* meta, float4* boxes, cudaStream_t st,
-                         int* perm = nullptr, int* inv = nullptr, bool walkable = false, bool kd = true) {
-  const SortSide s0 = sort_side(xyz, clouds, count, out, meta, boxes, perm, inv, walkable);
-  return run_prep_sort2(s0, clouds, s0, 0, st, walkable, kd);
+  if (maxcount <= 4096)
+    return kd ? launch_prep_sort<true, 256>(a, clouds, maxcount, st) : launch_prep_sort<false, 256>(a, clouds, maxcount, st);
+  return kd ? launch_prep_sort<true, SORT_TPB>(a, clouds, maxcount, st) : launch_prep_sort<false, SORT_TPB>(a, clouds, maxcount, st);
 }
 
 #include "chamfer_pair.cuh"
@@ -1219,11 +1050,10 @@ static unsigned long long* g_visited_counter = nullptr;
 // Un-sampled clouds in the batch front end (compute_cd on (B, H*W, 3) pairs, reference evaluate_reconstruction.py:
 // 124-131): the same treatment as the matrix front end -- zero points merged into one candidate, kept points
 // Morton-sorted with a box per chunk, chunks pruned by box distance -- plus the maps back to the original order.
+constexpr int BATCH_SORT_ABOVE = 4096;
 static bool forward_takes_sorted_path(int n, int m) {
-  static const bool enabled = [] { const char* e = getenv("DUSTY_CHAMFER_BATCH_SORT"); return !(e && e[0] == '0'); }();
-  static const int above = [] { const char* e = getenv("DUSTY_CHAMFER_BATCH_SORT_ABOVE"); return e ? atoi(e) : 4096; }();
   const int big = n > m ? n : m;
-  return enabled && big > above && big <= SORT_CAP;
+  return big > BATCH_SORT_ABOVE && big <= SORT_CAP;
 }
 
 namespace {
@@ -1275,15 +1105,12 @@ extern "C" int dusty_chamfer_forward(const float* xyz1, const float* xyz2, int b
   if (forward_takes_sorted_path(n, m)) {
     SortedSide X, Y;
     Y.carve(X.carve(static_cast<char*>(workspace), b, n), b, m);
-    static const bool walk = [] { const char* e = getenv("DUSTY_CHAMFER_WALK"); return !(e && e[0] == '0'); }();
     // Order of the batch front end's clouds: each is searched once, so the sort is most of the call. Measured, 8 / 32 / 128 pairs
-    // of 32768-point scans: Morton + tile kernel 0.87 / 1.25 / 2.87 ms, Morton + walk 0.96 / 1.19 / 2.27 ms, k-d + walk 3.45 /
-    // 3.52 / 4.12 ms (the k-d sort alone is 1.56 ms per launch: ten segmented sorts). The matrix front end, where a cloud is
-    // searched 2 N times, takes the k-d order. DUSTY_CHAMFER_BATCH_KD=1 for A/B runs. (With the split walk kernel -- 32-row groups,
-    // four times the CTAs -- Morton + walk is 0.78 / 1.04 / 2.02 ms.)
-    static const bool kd = [] { const char* e = getenv("DUSTY_CHAMFER_BATCH_KD"); return e && e[0] == '1'; }();
-    if (int rc = run_prep_sort2(sort_side(xyz1, b, n, X.scan, X.meta, X.boxes, X.perm, X.inv, walk), b,
-                                sort_side(xyz2, b, m, Y.scan, Y.meta, Y.boxes, Y.perm, Y.inv, walk), b, st, walk, kd)) return rc;
+    // of 32768-point scans with 64-row walk groups: Morton 0.96 / 1.19 / 2.27 ms, k-d 3.45 / 3.52 / 4.12 ms (the k-d sort alone
+    // is 1.56 ms per launch: ten segmented sorts); Morton with the 32-row groups of the split walk: 0.78 / 1.04 / 2.02 ms. The
+    // matrix front end, where a cloud is searched 2 N times, takes the k-d order.
+    if (int rc = run_prep_sort2(sort_side(xyz1, b, n, X.scan, X.meta, X.boxes, X.perm, X.inv), b,
+                                sort_side(xyz2, b, m, Y.scan, Y.meta, Y.boxes, Y.perm, Y.inv), b, st, false)) return rc;
     Params p{};
     p.scanX = X.scan; p.scanY = Y.scan;
     p.countX = n; p.countY = m;
@@ -1291,22 +1118,10 @@ extern "C" int dusty_chamfer_forward(const float* xyz1, const float* xyz2, int b
     p.strideX = p.paddedX; p.strideY = p.paddedY;
     p.dist1 = X.dist; p.dist2 = Y.dist; p.idx1 = X.idx; p.idx2 = Y.idx;
     p.metaX = X.meta; p.metaY = Y.meta; p.boxX = X.boxes; p.boxY = Y.boxes; p.permX = X.perm; p.permY = Y.perm;
+    p.bbX = block_boxes_of(X.boxes, b, n); p.bbY = block_boxes_of(Y.boxes, b, m);
     p.visited = g_visited_counter;
-    constexpr int R = 4;          // 128-row warps: the row boxes the pruning test uses stay tight (see dusty_chamfer_matrix)
-    const int big = n > m ? n : m;
-    constexpr int NTB = 64;       // two warps per CTA, 512-candidate tiles: see nn_kernel
-    if (walk) {
-      p.bbX = block_boxes_of(X.boxes, b, n); p.bbY = block_boxes_of(Y.boxes, b, m);
-      static const bool walk_split = [] { const char* e = getenv("DUSTY_CHAMFER_WALK_SPLIT"); return !(e && e[0] == '0'); }();   // A/B
-      if (walk_split) {
-        const int tasks = (n + 31) / 32 + (m + 31) / 32 + 2;      // 32-row groups of both directions (+ the merged origin rows)
-        if (int rc = launch_walk_split<false>(p, dim3((tasks + WALK_TPC - 1) / WALK_TPC, b, 1), st)) return rc;
-      } else {
-        const int tasks = (n + 63) / 64 + (m + 63) / 64 + 2;      // 64-row groups
-        if (int rc = launch_walk<2, 8, false>(p, dim3((tasks + WALK_TPC - 1) / WALK_TPC, b, 1), st)) return rc;
-      }
-    } else
-    if (int rc = launch_nn<R, false, true, NTB, 512>(p, dim3((big + NTB * R - 1) / (NTB * R), b, 2), st)) return rc;
+    const int tasks = (n + 31) / 32 + (m + 31) / 32 + 2;      // 32-row groups of both directions (+ the merged origin rows)
+    if (int rc = launch_walk_split<false>(p, dim3((tasks + WALK_TPC - 1) / WALK_TPC, b, 1), st)) return rc;
     unsort_kernel<<<(unsigned)(((long long)b * n + 255) / 256), 256, 0, st>>>(X.dist, X.idx, X.inv, b, n, p.strideX, dist1, idx1);
     DUSTY_AFTER_LAUNCH("chamfer unsort_kernel");
     unsort_kernel<<<(unsigned)(((long long)b * m + 255) / 256), 256, 0, st>>>(Y.dist, Y.idx, Y.inv, b, m, p.strideY, dist2, idx2);
@@ -1325,14 +1140,13 @@ extern "C" int dusty_chamfer_forward(const float* xyz1, const float* xyz2, int b
   p.dist1 = dist1; p.dist2 = dist2; p.idx1 = idx1; p.idx2 = idx2;
   // rows per thread: the largest R that still gives about one CTA per SM (a CTA covers 256 R rows of one
   // direction of one pair); few pairs of small clouds otherwise leave most of the GPU idle. Measured
-  // (tests/perf_chamfer_batch.py, 32 pairs of 2048 points): R = 8 (64 CTAs) 133 us, R = 4 (128 CTAs) 91 us,
+  // (32 pairs of 2048 points): R = 8 (64 CTAs) 133 us, R = 4 (128 CTAs) 91 us,
   // R = 1 (512 CTAs) 117 us -- smaller R feeds fewer FFMA2 per LDS, so stop as soon as the GPU is covered.
   const int big = n > m ? n : m;
   int r = pick_r(big);
   while (r > 1 && 2LL * b * ((big + TPB * r - 1) / (TPB * r)) < 120) r >>= 1;
-  if (const char* e = getenv("DUSTY_CHAMFER_R")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 4 || v == 8) r = v; }
   const int rbmax = (big + TPB * r - 1) / (TPB * r);
-  return dispatch_nn<false, false>(r, p, dim3(rbmax, b, 2), st);
+  return dispatch_batch(r, p, dim3(rbmax, b, 2), st);
 }
 
 extern "C" size_t dusty_chamfer_backward_workspace_bytes(int, int, int) { return 0; }
@@ -1406,30 +1220,16 @@ static int matrix_impl(const float* A, int na, int pa, const float* B, int nb, i
   float4* sb = symmetric ? sa : reinterpret_cast<float4*>(wsb);
   int2* mb = symmetric ? ma : reinterpret_cast<int2*>(wsb + align_up(scan_bytes(nb, pb), 256));
   float4* bb = symmetric ? ba : reinterpret_cast<float4*>(wsb + align_up(scan_bytes(nb, pb), 256) + meta_bytes(nb));
-  // merged clouds that fit the shared-memory sort are also put in spatial order with a box per chunk, and the
-  // kernel prunes chunks by box distance (DUSTY_CHAMFER_PRUNE=0 keeps the plain merged scan for A/B runs)
-  static const bool prune_enabled = [] { const char* e = getenv("DUSTY_CHAMFER_PRUNE"); return !(e && e[0] == '0'); }();
-  int merged_r = pick_r(pa > pb ? pa : pb);
-  static const bool pair_enabled = [] { const char* e = getenv("DUSTY_CHAMFER_PAIR"); return !(e && e[0] == '0'); }();
-  const bool pair = merge && prune_enabled && pair_enabled && pa <= PAIR_CAP && pb <= PAIR_CAP;
-  const bool sorted = merge && prune_enabled && pa <= SORT_CAP && pb <= SORT_CAP && (merged_r == 8 || pair);
-  if (sorted) {
-    // Pruning works per warp, and a warp owns 32 R consecutive sorted rows: fewer rows per thread give tighter row
-    // boxes (more chunks skipped) against fewer FFMA2 per LDS. Measured on the bench's un-sampled clouds, entries/s
-    // per GPU: R = 8 46.3 k, R = 4 61.0 k, R = 2 57.8 k, R = 1 39.0 k. DUSTY_CHAMFER_MERGED_R re-creates the A/B.
-    merged_r = 4;
-    if (const char* e = getenv("DUSTY_CHAMFER_MERGED_R")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 4 || v == 8) merged_r = v; }
-  }
-  // clouds that fit shared memory twice over (the evaluation's 2048 FPS samples): k-d order + the resident-pair kernel
-  // larger sorted clouds: k-d order + the two-level best-first walk from global memory (DUSTY_CHAMFER_WALK=0: Morton
-  // order + the tile-streaming nn_kernel, kept for A/B runs)
-  static const bool walk_enabled = [] { const char* e = getenv("DUSTY_CHAMFER_WALK"); return !(e && e[0] == '0'); }();
-  const bool walk = sorted && !pair && walk_enabled;
+  // Merged clouds that fit the shared-memory sort are put in k-d order with a box per chunk and per block of 32 chunks.
+  // Clouds that fit shared memory twice over (the evaluation's 2048 FPS samples) go to the resident-pair kernel, larger
+  // sorted ones to the two-level best-first walk from global memory, merged clouds beyond SORT_CAP to nn_kernel.
+  const bool pair = merge && pa <= PAIR_CAP && pb <= PAIR_CAP;
+  const bool walk = merge && !pair && pa <= SORT_CAP && pb <= SORT_CAP;
+  const bool sorted = pair || walk;
   if (!prepared) {
     if (sorted) {
-      const bool wk = pair || walk;
-      if (int rc = run_prep_sort2(sort_side(A, na, pa, sa, ma, ba, nullptr, nullptr, wk), na,
-                                  sort_side(B, nb, pb, sb, mb, bb, nullptr, nullptr, wk), symmetric ? 0 : nb, st, wk, true)) return rc;
+      if (int rc = run_prep_sort2(sort_side(A, na, pa, sa, ma, ba, nullptr, nullptr), na,
+                                  sort_side(B, nb, pb, sb, mb, bb, nullptr, nullptr), symmetric ? 0 : nb, st, true)) return rc;
     } else if (merge) {
       if (int rc = run_prep_merge(A, na, pa, sa, ma, st)) return rc;
       if (!symmetric) if (int rc = run_prep_merge(B, nb, pb, sb, mb, st)) return rc;
@@ -1454,26 +1254,9 @@ static int matrix_impl(const float* A, int na, int pa, const float* B, int nb, i
   if (merge) {
     p.metaX = ma; p.metaY = mb;
     if (sorted) { p.boxX = ba; p.boxY = bb; p.bbX = block_boxes_of(ba, na, pa); p.bbY = symmetric ? p.bbX : block_boxes_of(bb, nb, pb); }
-    // rows per lane, measured on 100 vs 100 un-sampled clouds: 1: 109.9 ms (1.7 % of the kept pairs visited), 2: 83.7 ms (2.3 %), 4: 85.9 ms (3.2 %)
-    static const bool walk_split = [] { const char* e = getenv("DUSTY_CHAMFER_WALK_SPLIT"); return !(e && e[0] == '0'); }();   // A/B
-    if (walk) return walk_split ? launch_walk_split<true>(p, grid, st) : launch_walk<2, 8, true>(p, grid, st);
-    if (pair) {
-      // Measured on the 1000 vs 1000 x 2048 evaluation (64-row groups, nn_pair_kernel<R, SUB, NW>): rows per lane R = 1 / 2 / 4:
-      // 444 / 418 / 536 ms; candidates per search window SUB = 8 / 16 / 32: 419 / 436 / 512 ms; warps per CTA NW = 4 / 6 / 8 / 10 / 12:
-      // 466 / 435 / 418 / 416 / 415 ms (a plateau: bound by issue slots and FFMA2/FMNMX3 dispatch, not by latency). The split
-      // kernel's 32-row groups: 392 ms. Only the two best shapes are instantiated.
-      static const bool pair_split = [] { const char* e = getenv("DUSTY_CHAMFER_PAIR_SPLIT"); return !(e && e[0] == '0'); }();
-      return pair_split ? launch_pair_split(p, grid, st) : launch_pair<2, 8>(p, grid, st);
-    }
-    static const bool narrow = [] { const char* e = getenv("DUSTY_CHAMFER_NARROW"); return !(e && e[0] == '0'); }();   // A/B switch
-    if (sorted && merged_r == 4 && narrow) {
-      // Measured on 100 vs 100 un-sampled clouds, entries/s per GPU. Round 1 layout (256 threads, 2048-candidate tiles, exact
-      // pass per tile) 58.6 k; exact pass deferred to the end of a row block 62.8 k; + two warps per CTA with 512-candidate
-      // tiles 69.5 k; + the per-row second pruning level 92.3 k (R = 8 with 32 or 64 threads 91.2 k, 128 threads with
-      // 1024-candidate tiles 93.0 k, R = 2 72.5 k: a plateau).
-      return launch_nn<4, true, true, 64, 512>(p, grid, st);
-    }
-    return dispatch_nn<true, true>(merged_r, p, grid, st);
+    if (pair) return launch_pair_split(p, grid, st);
+    if (walk) return launch_walk_split<true>(p, grid, st);
+    return launch_nn<8, true, true>(p, grid, st);
   }
   return dispatch_matrix(pa > pb ? pa : pb, p, grid, st);
 }

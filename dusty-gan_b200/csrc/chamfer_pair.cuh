@@ -3,282 +3,35 @@
 //
 // One CTA per matrix entry keeps BOTH clouds (scan format, 32 KB each at 2048 points) and their chunk boxes in shared
 // memory -- one round of four TMA bulk copies per entry instead of a tile stream per row block -- and its warps take
-// (direction, row group) tasks from a shared counter. A row group is 32 R consecutive rows of the k-d order, i.e. R
-// leaves of the row cloud's tree under one ancestor. For its group a warp
-//   1. bounds every candidate chunk from below by the distance between the chunk's box and the group's box (two
+// (direction, row group) tasks from a shared counter. A row group is 32 consecutive rows of the k-d order, i.e. one
+// leaf of the row cloud's tree. For its group a warp
+//   1. bounds every candidate chunk from below by the distance between the chunk's box and the leaf's box (two
 //      chunks per lane) and keeps the bounds as sortable keys;
 //   2. visits chunks BEST FIRST (one REDUX.MIN per pick): the nearest chunks tighten every row's running minimum
 //      immediately, and the walk ends at the first chunk whose bound exceeds the largest running minimum of the group;
-//   3. scans a picked chunk only if some row's own distance to the chunk's box is within that row's running minimum
-//      (the second pruning level of nn_kernel);
-//   4. finishes like nn_kernel's DEFERRED pass: the winning chunk of every row is re-evaluated in the reference's
-//      rounding, and a runner-up chunk inside the search's error window sends the row through an exact scan of every
-//      chunk its box bound cannot exclude.
+//   3. scans a picked chunk only if some row's own distance to the chunk's box is within that row's running minimum;
+//   4. finishes like nn_kernel's DEFERRED pass: the winning 8-candidate window of every row is re-evaluated in the
+//      reference's rounding, and a runner-up window inside the search's error window sends the row through an exact
+//      scan of every chunk its box bound cannot exclude.
 // Every bound is the reference's own distance formula on per-axis gaps (monotone, so it never exceeds a rounded pair
 // distance: oracle property test tests/test_oracle_golden.py), hence the results are the brute-force kernel's bit for
-// bit. Measured on the bench's 2048-point FPS clouds the walk evaluates 11 % of the pairs (Morton order + tile-order
-// visits of nn_kernel<4,1,1,64,512>: 38 %).
-// One matrix entry from its two directed sums: M[i,j] (+ mirror) and the fused MMD/COV/1-NNA reductions (see nn_kernel).
-__device__ __forceinline__ void emit_entry(const Params& p, int ci, int cj, double S0, double S1) {
-  const float v = (float)(S0 / (double)p.countX) + (float)(S1 / (double)p.countY);
-  if (p.M) {
-    p.M[(long long)(p.compact_rows ? (int)blockIdx.y : ci) * p.ldm + cj] = v;
-    if (p.symmetric && p.mirror && ci != cj) p.M[(long long)cj * p.ldm + ci] = v;
-  }
-  if (p.keys) {
-    const int gi = p.offX + ci, gj = p.offY + cj;
-    if (gi != gj) {
-      const unsigned long long vb = (unsigned long long)__float_as_uint(v) << 32;
-      atomicMin(p.keys + gj, vb | (unsigned)gi);
-      atomicMin(p.keys + gi, vb | (unsigned)gj);
-      const int lo = min(gi, gj), hi = max(gi, gj);
-      if (lo < p.n_ref && hi >= p.n_ref) {
-        atomicMin(p.keys + p.n_total + hi, vb | (unsigned)lo);
-        atomicMin(p.keys + 2 * (long long)p.n_total + lo, vb | (unsigned)hi);
-      }
-    }
-  }
-}
-
+// bit.
+//
+// The scan is bound by FFMA2/FMNMX3 dispatch (8.9 cycles per row and candidate pair), so the way to go faster is to
+// evaluate fewer pairs: on the bench's 2048-point FPS clouds 32-row groups visit 8.3 % of the pairs against 11.0 % for
+// 64-row groups. With one row per lane, though, every candidate pair costs two warp-uniform LDS.128 = four
+// shared-memory wavefronts per four arithmetic instructions and the kernel becomes shared-memory bound (444 ms against
+// 418 ms for two rows per lane on the 1000 vs 1000 x 2048 evaluation). So a lane keeps TWO rows (rows l and l + 16 of
+// the leaf, l = lane & 15; lanes l and l ^ 16 hold the same rows) and half-warp h reads the candidate pairs 8 h .. 8 h + 7
+// of the chunk -- an LDS.128 with one address per half-warp is still two wavefronts -- which halves the wavefronts per
+// arithmetic instruction. Each lane tracks (minimum, runner-up, window) of both rows over ITS half of the candidates;
+// the halves are merged with one shuffle per scanned chunk (pruning bound of the lane's own row: lane l + 16 h owns
+// row l + 16 h) and three at the end of the walk.
+// Shape, measured with 64-row groups on the same evaluation: 8 / 16 / 32 candidates per window 419 / 436 / 512 ms;
+// 4 / 6 / 8 / 10 / 12 warps per CTA 466 / 435 / 418 / 416 / 415 ms (a plateau: bound by issue slots, not by latency).
 constexpr int PAIR_CAP = 2048;
 constexpr int PAIR_NW = 8;                 // warps per CTA
 
-template <int R, int SUB, int NW = PAIR_NW>
-__global__ void __launch_bounds__(NW * 32, 3) nn_pair_kernel(const Params p) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  __shared__ uint64_t bar;
-  // per-task sums: a task's sum is formed in a fixed order inside its warp and the tasks are added in task order, so the
-  // entry does not depend on which warp happened to take which task
-  __shared__ double tsum[2 * (PAIR_CAP / (32 * R))];
-  __shared__ int next_task;
-  const int tid = threadIdx.x, lane = tid & 31;
-
-  const int ci = p.row_begin + blockIdx.y * p.row_stride;
-  const int cj = blockIdx.x;
-  if (p.symmetric && cj < ci) return;
-
-  const int2 mx = p.metaX[ci], my = p.metaY[cj];
-  const int padX = (mx.x + CHUNK - 1) / CHUNK * CHUNK, padY = (my.x + CHUNK - 1) / CHUNK * CHUNK;
-  float4* const sX = reinterpret_cast<float4*>(smem_raw);
-  float4* const sY = sX + p.paddedX;
-  float4* const bX = sY + p.paddedY;
-  float4* const bY = bX + p.paddedX / CHUNK * 2;
-  if (tid == 0) {
-    mbar_init(&bar, 1);
-    mbar_fence_init();
-    next_task = 0;
-    const uint32_t bytes = (uint32_t)(padX + padY) * 16u + (uint32_t)(padX / CHUNK + padY / CHUNK) * 32u;
-    mbar_expect_tx(&bar, bytes);
-    bulk_g2s(sX, p.scanX + (long long)ci * p.strideX, (uint32_t)padX * 16u, &bar);
-    bulk_g2s(sY, p.scanY + (long long)cj * p.strideY, (uint32_t)padY * 16u, &bar);
-    bulk_g2s(bX, p.boxX + (long long)ci * (p.paddedX / CHUNK * 2), (uint32_t)(padX / CHUNK) * 32u, &bar);
-    bulk_g2s(bY, p.boxY + (long long)cj * (p.paddedY / CHUNK * 2), (uint32_t)(padY / CHUNK) * 32u, &bar);
-  }
-  __syncthreads();
-  mbar_wait(&bar, 0);
-
-  constexpr int GR = 32 * R;                     // rows per group
-  const int ngX = (mx.x + GR - 1) / GR, ngY = (my.x + GR - 1) / GR;
-  const float inf = __int_as_float(0x7f800000);
-
-  for (;;) {
-    int task = 0;
-    if (lane == 0) task = atomicAdd(&next_task, 1);
-    task = __shfl_sync(0xffffffffu, task, 0);
-    if (task >= ngX + ngY) break;
-    const int dir = task >= ngX;
-    const int g = dir ? task - ngX : task;
-    const float4* const rows = dir ? sY : sX;
-    const float4* const cand = dir ? sX : sY;
-    const float4* const rbox = dir ? bY : bX;
-    const float4* const cbox = dir ? bX : bY;
-    const int rowcount = dir ? my.x : mx.x;
-    const int nrch = (dir ? padY : padX) / CHUNK;       // chunks of the row cloud
-    const int nch = (dir ? padX : padY) / CHUNK;        // chunks of the candidate cloud (<= 64)
-
-    // ---- rows (R leaves of the row cloud: rows r * 32 + lane of leaf g R + r) and the group's box ----
-    f32x2 nax[R], nay[R], naz[R];
-    float cur[R], sec[R], an[R], ubr[R];
-    int cid[R];
-    float gl0 = inf, gl1 = inf, gl2 = inf, gh0 = -inf, gh1 = -inf, gh2 = -inf;
-    #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const int row = g * GR + r * 32 + lane;
-      const int rr = row < rowcount ? row : 0;
-      const float* f = reinterpret_cast<const float*>(rows + (rr >> 1) * 2) + (rr & 1);
-      const float mx2 = -2.0f * f[0], my2 = -2.0f * f[2], mz2 = -2.0f * f[4];
-      nax[r] = pack2(mx2, mx2); nay[r] = pack2(my2, my2); naz[r] = pack2(mz2, mz2);
-      an[r] = 0.25f * fmaf(mz2, mz2, fmaf(mx2, mx2, my2 * my2));
-      cur[r] = sec[r] = inf; cid[r] = 0;
-      ubr[r] = row < rowcount ? inf : -1.0f;                 // dead rows never ask
-      if (g * R + r < nrch) {
-        const float4 bl = rbox[2 * (g * R + r)], bh = rbox[2 * (g * R + r) + 1];
-        gl0 = fminf(gl0, bl.x); gl1 = fminf(gl1, bl.y); gl2 = fminf(gl2, bl.z);
-        gh0 = fmaxf(gh0, bh.x); gh1 = fmaxf(gh1, bh.y); gh2 = fmaxf(gh2, bh.z);
-        if (bl.w != 0.0f) {          // the chunk also holds the merged origin point, kept outside its box
-          gl0 = fminf(gl0, 0.0f); gl1 = fminf(gl1, 0.0f); gl2 = fminf(gl2, 0.0f);
-          gh0 = fmaxf(gh0, 0.0f); gh1 = fmaxf(gh1, 0.0f); gh2 = fmaxf(gh2, 0.0f);
-        }
-      }
-    }
-    // ---- lower bound of every candidate chunk: key = (bound with its low 6 mantissa bits cleared) | chunk ----
-    const bool forced = cbox[2 * (nch - 1)].w != 0.0f;      // the last chunk holds the merged origin (outside its box): always visited
-    unsigned key[2];
-    #pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int c = h * 32 + lane;
-      key[h] = 0xffffffffu;
-      if (forced && c == nch - 1) {
-        key[h] = (unsigned)c;
-      } else if (c < nch) {
-        const float4 bl = cbox[2 * c], bh = cbox[2 * c + 1];
-        const float gx = max3(0.0f, bl.x - gh0, gl0 - bh.x), gy = max3(0.0f, bl.y - gh1, gl1 - bh.y), gz = max3(0.0f, bl.z - gh2, gl2 - bh.z);
-        const float lb = fmaf(gz, gz, fmaf(gx, gx, __fmul_rn(gy, gy)));
-        if (lb < inf) key[h] = (__float_as_uint(lb) & ~63u) | (unsigned)c;      // lb >= 0: the bit pattern orders like the value
-      }
-    }
-    float ubmax = inf;
-    int nvis = 0;
-    for (;;) {
-      const unsigned kwin = __reduce_min_sync(0xffffffffu, min(key[0], key[1]));
-      if (kwin == 0xffffffffu) break;
-      if (__uint_as_float(kwin & ~63u) > ubmax) break;      // (truncated) bound beyond every row's reach: so is the rest
-      const int c = (int)(kwin & 63u);
-      if (key[0] == kwin) key[0] = 0xffffffffu;
-      if (key[1] == kwin) key[1] = 0xffffffffu;
-      const float4 bl = cbox[2 * c], bh = cbox[2 * c + 1];
-      bool need = forced && c == nch - 1;
-      #pragma unroll
-      for (int r = 0; r < R; ++r) {
-        float ax, ay, az, dummy;
-        unpack2(nax[r], ax, dummy); unpack2(nay[r], ay, dummy); unpack2(naz[r], az, dummy);
-        ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
-        const float gx = max3(0.0f, bl.x - ax, ax - bh.x), gy = max3(0.0f, bl.y - ay, ay - bh.y), gz = max3(0.0f, bl.z - az, az - bh.z);
-        need |= fmaf(gz, gz, fmaf(gx, gx, __fmul_rn(gy, gy))) <= ubr[r];
-      }
-      if (!__any_sync(0xffffffffu, need)) continue;
-      ++nvis;
-      // search, tracked per SUB-candidate window: the exact pass re-reads only the winning window of each row (every
-      // lane another one: with whole chunks those loads, not the scan's broadcasts, saturated shared memory)
-      const float4* cp = cand + c * CHUNK;
-      #pragma unroll
-      for (int w = 0; w < CHUNK / SUB; ++w) {
-        float cm[R];
-        #pragma unroll
-        for (int k = w * (SUB / 2); k < (w + 1) * (SUB / 2); ++k) {
-          const float4 q0 = cp[2 * k], q1 = cp[2 * k + 1];
-          const f32x2 bx = pack2(q0.x, q0.y), by = pack2(q0.z, q0.w);
-          const f32x2 bz = pack2(q1.x, q1.y), bn = pack2(q1.z, q1.w);
-          #pragma unroll
-          for (int r = 0; r < R; ++r) {
-            f32x2 s = fma2(naz[r], bz, bn);
-            s = fma2(nay[r], by, s);
-            s = fma2(nax[r], bx, s);
-            float lo, hi;
-            unpack2(s, lo, hi);
-            cm[r] = (k == w * (SUB / 2)) ? fminf(lo, hi) : min3(cm[r], lo, hi);
-          }
-        }
-        #pragma unroll
-        for (int r = 0; r < R; ++r) {
-          const bool better = cm[r] < cur[r];
-          sec[r] = fminf(sec[r], better ? cur[r] : cm[r]);      // runner-up: the smallest minimum of any other window (NaN: all padding)
-          cur[r] = fminf(cur[r], cm[r]);
-          cid[r] = better ? c * (CHUNK / SUB) + w : cid[r];
-        }
-      }
-      float m = 0.0f;
-      #pragma unroll
-      for (int r = 0; r < R; ++r) {
-        // upper bound of the row's final exact minimum (see nn_kernel, DEFERRED): dest + 64 u (|a|^2 + dest)
-        if (ubr[r] >= 0.0f) {
-          const float dest = fmaxf(cur[r] + an[r], 0.0f);
-          ubr[r] = fmaf(3.81469727e-6f /* 64 * 2^-24 */, an[r] + dest, dest) + 1e-36f;
-          m = fmaxf(m, ubr[r]);
-        }
-      }
-      ubmax = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m)));
-    }
-    if (p.visited != nullptr && lane == 0)
-      atomicAdd(p.visited, (unsigned long long)nvis * CHUNK * (unsigned long long)min(GR, rowcount - g * GR));
-
-    // ---- exact pass on each row's winning window, guard over the whole candidate cloud ----
-    double dsum = 0.0;
-    #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      float ax, ay, az, dummy;
-      unpack2(nax[r], ax, dummy); unpack2(nay[r], ay, dummy); unpack2(naz[r], az, dummy);
-      ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
-      const int row = g * GR + r * 32 + lane;
-      const bool live = row < rowcount;
-      float e = inf;
-      if (live && cur[r] < inf) {
-        const f32x2 ax2 = pack2(ax, ax), ay2 = pack2(ay, ay), az2 = pack2(az, az);
-        const float4* cp = cand + cid[r] * SUB;
-        #pragma unroll
-        for (int k = 0; k < SUB / 2; ++k) {
-          const int kk = (k + lane) & (SUB / 2 - 1);      // lanes start on different banks
-          const float4 q0 = cp[2 * kk], q1 = cp[2 * kk + 1];
-          const f32x2 dx = sub2(pack2(q0.x, q0.y), ax2);
-          const f32x2 dy = sub2(pack2(q0.z, q0.w), ay2);
-          const f32x2 dz = sub2(pack2(q1.x, q1.y), az2);
-          float lo, hi;
-          unpack2(fma2(dz, dz, fma2(dx, dx, mul2(dy, dy))), lo, hi);
-          e = min3(e, lo, hi);
-        }
-      }
-      const bool near_tie = live && sec[r] <= cur[r] + search_window(ax, ay, az, cur[r]);
-      unsigned flagged = __ballot_sync(0xffffffffu, near_tie);
-      while (flagged) {                         // warp-uniform
-        const int src = __ffs(flagged) - 1;
-        flagged &= flagged - 1;
-        float m;
-        int mi;
-        warp_cloud_exact_min<false>(cand, nch, cbox, __shfl_sync(0xffffffffu, e, src), __shfl_sync(0xffffffffu, ax, src),
-                                    __shfl_sync(0xffffffffu, ay, src), __shfl_sync(0xffffffffu, az, src), lane, nullptr, m, mi);
-        if (lane == src) e = fminf(e, m);
-      }
-      if (live) dsum += (row == rowcount - 1 ? (double)(dir ? my.y : mx.y) : 1.0) * (double)e;
-    }
-    #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) dsum += __shfl_down_sync(0xffffffffu, dsum, o);
-    if (lane == 0) tsum[task] = dsum;
-  }
-
-  __syncthreads();
-  if (tid == 0) {
-    double S0 = 0.0, S1 = 0.0;
-    for (int t = 0; t < ngX; ++t) S0 += tsum[t];
-    for (int t = ngX; t < ngX + ngY; ++t) S1 += tsum[t];
-    emit_entry(p, ci, cj, S0, S1);
-  }
-}
-
-template <int R, int SUB, int NW = PAIR_NW>
-static int launch_pair(const Params& p, dim3 grid, cudaStream_t st) {
-  const size_t smem = (size_t)(p.paddedX + p.paddedY) * 16 + (size_t)(p.paddedX / CHUNK + p.paddedY / CHUNK) * 32;
-  static bool configured[kMaxDevices] = {};
-  const int dev = current_device();
-  if (!configured[dev]) {
-    DUSTY_CUDA(cudaFuncSetAttribute(nn_pair_kernel<R, SUB, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    2 * PAIR_CAP * 16 + 2 * (PAIR_CAP / CHUNK) * 32));
-    configured[dev] = true;
-  }
-  nn_pair_kernel<R, SUB, NW><<<grid, NW * 32, smem, st>>>(p);
-  DUSTY_AFTER_LAUNCH("chamfer nn_pair_kernel");
-  return 0;
-}
-
-// Split variant: 32-row groups (ONE leaf of the row cloud's k-d tree) without the shared-memory cost of one row per lane.
-// nn_pair_kernel's scan is bound by FFMA2/FMNMX3 dispatch (8.9 cycles per row and candidate pair), so the way to go faster
-// is to evaluate fewer pairs: 32-row groups visit 8.3 % of the pairs against 11.0 % for 64-row groups. With one row per
-// lane, though, every candidate pair costs two warp-uniform LDS.128 = four shared-memory wavefronts per four arithmetic
-// instructions and the kernel becomes shared-memory bound (nn_pair_kernel<1,8>: 444 ms against 418 ms). Here a lane keeps
-// TWO rows (rows l and l + 16 of the leaf, l = lane & 15; lanes l and l ^ 16 hold the same rows) and half-warp h reads the
-// candidate pairs 8 h .. 8 h + 7 of the chunk -- an LDS.128 with one address per half-warp is still two wavefronts --
-// so the wavefronts per arithmetic instruction are those of the two-rows-per-lane kernel. Each lane tracks (minimum,
-// runner-up, window) of both rows over ITS half of the candidates; the halves are merged with one shuffle per scanned
-// chunk (pruning bound of the lane's own row: lane l + 16 h owns row l + 16 h) and three at the end of the walk.
 __global__ void __launch_bounds__(PAIR_NW * 32, 3) nn_pair_split_kernel(const Params p) {
   constexpr int SUB = 8;
   constexpr int GR = 32;

@@ -1,264 +1,25 @@
-// Best-first Chamfer search for k-d ordered clouds of any size up to SORT_CAP (un-sampled range images: configs[4],
+// Best-first Chamfer search for sorted clouds of any size up to SORT_CAP (un-sampled range images: configs[4],
 // compute_cd on reconstruction pairs): included by chamfer.cu inside namespace dusty::chamfer.
 //
-// Same walk as nn_pair_kernel (chamfer_pair.cuh) with two changes for clouds that do not fit shared memory:
-//   * two levels: a lane first bounds one BLOCK of 32 chunks (a 1024-point subtree of the candidate cloud's k-d
-//     tree; at most 32 blocks, their boxes come from prep_sort_kernel) and the warp opens blocks best first; inside
-//     an open block a lane bounds one chunk and the warp scans chunks best first. Both levels stop at the first
-//     bound beyond the largest running minimum of the warp's 64 rows;
-//   * candidates, boxes and rows are read from global memory through L1 (the kernel uses little shared memory,
-//     so L1 keeps ~200 KB): row groups are taken in k-d order, so the warps of a CTA work on neighbouring groups and
-//     walk overlapping chunks. (The split variant below -- the default -- stages the chunk it scans through 512 bytes
-//     of per-warp shared memory: a half-warp-uniform LDG.128 costs far more L1 wavefronts than the same LDS.128.)
-// nn_kernel<4,1,1,64,512> streams every tile of the candidate cloud past every row block (33 MB of L2 -> shared
-// memory traffic per entry at 16 k points, tiles visited in storage order); the walk reads the chunks it scans.
+// The walk of nn_pair_split_kernel (chamfer_pair.cuh) -- 32-row groups, two rows per lane, the two half-warps on the two
+// halves of a candidate chunk, lane l + 16 h owns row l + 16 h -- with two changes for clouds that do not fit shared memory:
+//   * two levels: a lane first bounds one BLOCK of 32 chunks (1024 consecutive points of the candidate cloud, a subtree
+//     of its k-d tree in k-d order; at most 32 blocks, their boxes come from prep_sort_kernel) and the warp opens blocks
+//     best first; inside an open block a lane bounds one chunk and the warp scans chunks best first. Both levels stop
+//     at the first bound beyond the largest running minimum of the warp's 32 rows;
+//   * candidates, boxes and rows are read from global memory through L1 (the kernel uses little shared memory, so L1
+//     keeps ~200 KB): row groups are taken in sorted order, so the warps of a CTA work on neighbouring groups and walk
+//     overlapping chunks. The chunk a warp scans is staged through 512 bytes of per-warp shared memory: a
+//     half-warp-uniform LDG.128 costs far more L1 wavefronts than the same LDS.128.
+// The walk reads only the chunks it scans -- on the bench's un-sampled clouds 1.7 % of the kept pairs (64-row groups:
+// 2.3 %) -- where streaming every tile of the candidate cloud past every row block moves 33 MB from L2 to shared memory
+// per entry at 16 k points.
 // MATRIX: one CTA per matrix entry, per-task sums added in task order (deterministic under the dynamic task
-// order). Batch front end: a CTA takes WALK_TPC consecutive tasks of one pair; per-point (dist, idx) go to the sorted
-// positions and unsort_kernel puts them back (ties between bit-equal distances: lowest original index, through perm).
+// order). Batch front end (Morton order): a CTA takes WALK_TPC consecutive tasks of one pair; per-point (dist, idx) go to
+// the sorted positions and unsort_kernel puts them back (ties between bit-equal distances: lowest original index, through
+// perm).
 constexpr int WALK_NW = 8;                  // warps per CTA
 constexpr int WALK_TPC = 8;                 // tasks per CTA in the batch front end (one per warp: few pairs must still fill the GPU)
-constexpr int WALK_MAXTASKS = 2 * (SORT_CAP / 64 + 1);
-
-template <int R, int SUB, bool MATRIX>
-__global__ void __launch_bounds__(WALK_NW * 32, 3) nn_walk_kernel(const Params p) {
-  __shared__ double tsum[MATRIX ? WALK_MAXTASKS : 1];
-  __shared__ int next_task;
-  const int tid = threadIdx.x, lane = tid & 31;
-  int ci, cj;
-  if (MATRIX) {
-    ci = p.row_begin + blockIdx.y * p.row_stride;
-    cj = blockIdx.x;
-    if (p.symmetric && cj < ci) return;
-  } else {
-    ci = cj = blockIdx.y;
-  }
-  const int2 mx = p.metaX[ci], my = p.metaY[cj];
-  const int padX = (mx.x + CHUNK - 1) / CHUNK * CHUNK, padY = (my.x + CHUNK - 1) / CHUNK * CHUNK;
-  const float4* const sX = p.scanX + (long long)ci * p.strideX;
-  const float4* const sY = p.scanY + (long long)cj * p.strideY;
-  const float4* const bX = p.boxX + (long long)ci * (p.paddedX / CHUNK * 2);
-  const float4* const bY = p.boxY + (long long)cj * (p.paddedY / CHUNK * 2);
-  const float4* const bbX = p.bbX + (long long)ci * (2 * WALK_BLOCKS);
-  const float4* const bbY = p.bbY + (long long)cj * (2 * WALK_BLOCKS);
-
-  constexpr int GR = 32 * R;
-  const int ngX = (mx.x + GR - 1) / GR, ngY = (my.x + GR - 1) / GR;
-  int task_begin = 0, task_end = ngX + ngY;
-  if (!MATRIX) {
-    task_begin = blockIdx.x * WALK_TPC;
-    task_end = min(task_end, task_begin + WALK_TPC);
-    if (task_begin >= task_end) return;
-  }
-  if (tid == 0) next_task = task_begin;
-  __syncthreads();
-  const float inf = __int_as_float(0x7f800000);
-
-  for (;;) {
-    int task = 0;
-    if (lane == 0) task = atomicAdd(&next_task, 1);
-    task = __shfl_sync(0xffffffffu, task, 0);
-    if (task >= task_end) break;
-    const int dir = task >= ngX;
-    const int g = dir ? task - ngX : task;
-    const float4* const rows = dir ? sY : sX;
-    const float4* const cand = dir ? sX : sY;
-    const float4* const rbox = dir ? bY : bX;
-    const float4* const cbox = dir ? bX : bY;
-    const float4* const cblk = dir ? bbX : bbY;
-    const int* const cperm = MATRIX ? nullptr : (dir ? p.permX + (long long)ci * p.strideX : p.permY + (long long)cj * p.strideY);
-    const int rowcount = dir ? my.x : mx.x;
-    const int nrch = (dir ? padY : padX) / CHUNK;
-    const int nch = (dir ? padX : padY) / CHUNK;
-    const int nblk = (nch + 31) / 32;
-
-    f32x2 nax[R], nay[R], naz[R];
-    float cur[R], sec[R], an[R], ubr[R];
-    int cid[R];
-    float gl0 = inf, gl1 = inf, gl2 = inf, gh0 = -inf, gh1 = -inf, gh2 = -inf;
-    #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const int row = g * GR + r * 32 + lane;
-      const int rr = row < rowcount ? row : 0;
-      const float* f = reinterpret_cast<const float*>(rows + (rr >> 1) * 2) + (rr & 1);
-      const float mx2 = -2.0f * f[0], my2 = -2.0f * f[2], mz2 = -2.0f * f[4];
-      nax[r] = pack2(mx2, mx2); nay[r] = pack2(my2, my2); naz[r] = pack2(mz2, mz2);
-      an[r] = 0.25f * fmaf(mz2, mz2, fmaf(mx2, mx2, my2 * my2));
-      cur[r] = sec[r] = inf; cid[r] = 0;
-      ubr[r] = row < rowcount ? inf : -1.0f;
-      if (g * R + r < nrch) {
-        const float4 bl = rbox[2 * (g * R + r)], bh = rbox[2 * (g * R + r) + 1];
-        gl0 = fminf(gl0, bl.x); gl1 = fminf(gl1, bl.y); gl2 = fminf(gl2, bl.z);
-        gh0 = fmaxf(gh0, bh.x); gh1 = fmaxf(gh1, bh.y); gh2 = fmaxf(gh2, bh.z);
-        if (bl.w != 0.0f) {          // the chunk also holds the merged origin point, kept outside its box
-          gl0 = fminf(gl0, 0.0f); gl1 = fminf(gl1, 0.0f); gl2 = fminf(gl2, 0.0f);
-          gh0 = fmaxf(gh0, 0.0f); gh1 = fmaxf(gh1, 0.0f); gh2 = fmaxf(gh2, 0.0f);
-        }
-      }
-    }
-    auto box_key = [&](const float4& bl, const float4& bh, unsigned id) -> unsigned {
-      const float gx = max3(0.0f, bl.x - gh0, gl0 - bh.x), gy = max3(0.0f, bl.y - gh1, gl1 - bh.y), gz = max3(0.0f, bl.z - gh2, gl2 - bh.z);
-      const float lb = fmaf(gz, gz, fmaf(gx, gx, __fmul_rn(gy, gy)));
-      return lb < inf ? (__float_as_uint(lb) & ~31u) | id : 0xffffffffu;      // bound with 5 mantissa bits cleared | id
-    };
-    const bool forced = cbox[2 * (nch - 1)].w != 0.0f;      // the last chunk holds the merged origin (outside its box): always visited
-    unsigned bkey = 0xffffffffu;                 // upper level: one block of 32 chunks per lane
-    if (lane < nblk) bkey = forced && lane == nblk - 1 ? (unsigned)lane : box_key(cblk[2 * lane], cblk[2 * lane + 1], (unsigned)lane);
-    float ubmax = inf;
-    int nvis = 0;
-    for (;;) {
-      const unsigned bwin = __reduce_min_sync(0xffffffffu, bkey);
-      if (bwin == 0xffffffffu || __uint_as_float(bwin & ~31u) > ubmax) break;
-      const int blk = (int)(bwin & 31u);
-      if (bkey == bwin) bkey = 0xffffffffu;
-      unsigned key = 0xffffffffu;                // lower level: one chunk of the open block per lane
-      const int cl = blk * 32 + lane;
-      if (cl < nch) key = forced && cl == nch - 1 ? (unsigned)lane : box_key(cbox[2 * cl], cbox[2 * cl + 1], (unsigned)lane);
-      for (;;) {
-        const unsigned kwin = __reduce_min_sync(0xffffffffu, key);
-        if (kwin == 0xffffffffu || __uint_as_float(kwin & ~31u) > ubmax) break;
-        const int c = blk * 32 + (int)(kwin & 31u);
-        if (key == kwin) key = 0xffffffffu;
-        const float4 bl = cbox[2 * c], bh = cbox[2 * c + 1];
-        bool need = forced && c == nch - 1;
-        #pragma unroll
-        for (int r = 0; r < R; ++r) {
-          float ax, ay, az, dummy;
-          unpack2(nax[r], ax, dummy); unpack2(nay[r], ay, dummy); unpack2(naz[r], az, dummy);
-          ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
-          const float gx = max3(0.0f, bl.x - ax, ax - bh.x), gy = max3(0.0f, bl.y - ay, ay - bh.y), gz = max3(0.0f, bl.z - az, az - bh.z);
-          need |= fmaf(gz, gz, fmaf(gx, gx, __fmul_rn(gy, gy))) <= ubr[r];
-        }
-        if (!__any_sync(0xffffffffu, need)) continue;
-        ++nvis;
-        const float4* cp = cand + (long long)c * CHUNK;
-        #pragma unroll
-        for (int w = 0; w < CHUNK / SUB; ++w) {
-          float cm[R];
-          #pragma unroll
-          for (int k = w * (SUB / 2); k < (w + 1) * (SUB / 2); ++k) {
-            const float4 q0 = __ldg(cp + 2 * k), q1 = __ldg(cp + 2 * k + 1);
-            const f32x2 bx = pack2(q0.x, q0.y), by = pack2(q0.z, q0.w);
-            const f32x2 bz = pack2(q1.x, q1.y), bn = pack2(q1.z, q1.w);
-            #pragma unroll
-            for (int r = 0; r < R; ++r) {
-              f32x2 s = fma2(naz[r], bz, bn);
-              s = fma2(nay[r], by, s);
-              s = fma2(nax[r], bx, s);
-              float lo, hi;
-              unpack2(s, lo, hi);
-              cm[r] = (k == w * (SUB / 2)) ? fminf(lo, hi) : min3(cm[r], lo, hi);
-            }
-          }
-          #pragma unroll
-          for (int r = 0; r < R; ++r) {
-            const bool better = cm[r] < cur[r];
-            sec[r] = fminf(sec[r], better ? cur[r] : cm[r]);      // (an all-padding window has cm = NaN: ignored)
-            cur[r] = fminf(cur[r], cm[r]);
-            cid[r] = better ? c * (CHUNK / SUB) + w : cid[r];
-          }
-        }
-        float m = 0.0f;
-        #pragma unroll
-        for (int r = 0; r < R; ++r) {
-          if (ubr[r] >= 0.0f) {
-            const float dest = fmaxf(cur[r] + an[r], 0.0f);
-            ubr[r] = fmaf(3.81469727e-6f /* 64 * 2^-24 */, an[r] + dest, dest) + 1e-36f;
-            m = fmaxf(m, ubr[r]);
-          }
-        }
-        ubmax = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m)));
-      }
-    }
-    if (p.visited != nullptr && lane == 0)
-      atomicAdd(p.visited, (unsigned long long)nvis * CHUNK * (unsigned long long)min(GR, rowcount - g * GR));
-
-    // ---- exact pass on each row's winning window, guard over the whole candidate cloud ----
-    double dsum = 0.0;
-    #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      float ax, ay, az, dummy;
-      unpack2(nax[r], ax, dummy); unpack2(nay[r], ay, dummy); unpack2(naz[r], az, dummy);
-      ax *= -0.5f; ay *= -0.5f; az *= -0.5f;
-      const int row = g * GR + r * 32 + lane;
-      const bool live = row < rowcount;
-      float e = inf;
-      int eidx = 0x7fffffff;
-      if (live && cur[r] < inf) {
-        const f32x2 ax2 = pack2(ax, ax), ay2 = pack2(ay, ay), az2 = pack2(az, az);
-        const float4* cp = cand + (long long)cid[r] * SUB;
-        #pragma unroll
-        for (int k = 0; k < SUB / 2; ++k) {
-          const float4 q0 = __ldg(cp + 2 * k), q1 = __ldg(cp + 2 * k + 1);
-          const f32x2 dx = sub2(pack2(q0.x, q0.y), ax2);
-          const f32x2 dy = sub2(pack2(q0.z, q0.w), ay2);
-          const f32x2 dz = sub2(pack2(q1.x, q1.y), az2);
-          float lo, hi;
-          unpack2(fma2(dz, dz, fma2(dx, dx, mul2(dy, dy))), lo, hi);
-          if (MATRIX) {
-            e = min3(e, lo, hi);
-          } else {
-            const int i0 = cid[r] * SUB + 2 * k;
-            if (lo < e || (lo == e && eidx != 0x7fffffff && cperm[i0] < cperm[eidx])) { e = lo; eidx = i0; }
-            if (hi < e || (hi == e && eidx != 0x7fffffff && cperm[i0 + 1] < cperm[eidx])) { e = hi; eidx = i0 + 1; }
-          }
-        }
-      }
-      const bool near_tie = live && sec[r] <= cur[r] + search_window(ax, ay, az, cur[r]);
-      unsigned flagged = __ballot_sync(0xffffffffu, near_tie);
-      while (flagged) {                         // warp-uniform
-        const int src = __ffs(flagged) - 1;
-        flagged &= flagged - 1;
-        float m;
-        int mi = 0x7fffffff;
-        warp_cloud_exact_min<!MATRIX>(cand, nch, cbox, __shfl_sync(0xffffffffu, e, src), __shfl_sync(0xffffffffu, ax, src),
-                                      __shfl_sync(0xffffffffu, ay, src), __shfl_sync(0xffffffffu, az, src), lane, cperm, m, mi);
-        if (lane == src) {
-          if (MATRIX) {
-            e = fminf(e, m);
-          } else if (mi != 0x7fffffff && (m < e || (m == e && (eidx == 0x7fffffff || cperm[mi] < cperm[eidx])))) {
-            e = m; eidx = mi;
-          }
-        }
-      }
-      if (live) {
-        if (MATRIX) {
-          dsum += (row == rowcount - 1 ? (double)(dir ? my.y : mx.y) : 1.0) * (double)e;
-        } else {                // per sorted position (stride = padded count); unsort_kernel restores the original order
-          const long long o = (long long)ci * (dir ? p.strideY : p.strideX) + row;
-          (dir ? p.dist2 : p.dist1)[o] = e;
-          (dir ? p.idx2 : p.idx1)[o] = cperm[eidx == 0x7fffffff ? 0 : eidx];
-        }
-      }
-    }
-    if (MATRIX) {
-      #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) dsum += __shfl_down_sync(0xffffffffu, dsum, o);
-      if (lane == 0) tsum[task] = dsum;
-    }
-  }
-
-  if (MATRIX) {
-    __syncthreads();
-    if (tid == 0) {
-      double S0 = 0.0, S1 = 0.0;
-      for (int t = 0; t < ngX; ++t) S0 += tsum[t];
-      for (int t = ngX; t < ngX + ngY; ++t) S1 += tsum[t];
-      emit_entry(p, ci, cj, S0, S1);
-    }
-  }
-}
-
-template <int R, int SUB, bool MATRIX>
-static int launch_walk(const Params& p, dim3 grid, cudaStream_t st) {
-  nn_walk_kernel<R, SUB, MATRIX><<<grid, WALK_NW * 32, 0, st>>>(p);
-  DUSTY_AFTER_LAUNCH("chamfer nn_walk_kernel");
-  return 0;
-}
-
-// Split variant (the default): 32-row groups -- one leaf of the row cloud's k-d tree -- with two rows per lane; the two
-// half-warps read different halves of a candidate chunk. See nn_pair_split_kernel (chamfer_pair.cuh) for the reasoning:
-// fewer pairs visited (1.7 % instead of 2.3 % of the kept pairs on the bench's un-sampled clouds) at the L1 wavefronts per
-// arithmetic instruction of the two-rows-per-lane kernel. Lane l + 16 h owns row l + 16 h of its group.
 constexpr int WALK_SPLIT_MAXTASKS = 2 * (SORT_CAP / 32 + 1);
 
 template <bool MATRIX>

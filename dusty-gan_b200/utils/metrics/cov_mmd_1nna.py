@@ -50,10 +50,10 @@ FUSED_EPILOGUE = True
 # Clouds with more points than this go through the sorted search (flag DUSTY_MATRIX_MERGE_ORIGIN of the C ABI): all
 # exactly-zero points of a cloud -- the dropped pixels of an un-sampled range image (reference
 # evaluate_reconstruction.py:124-131, SURVEY.md S7) -- are scanned as ONE point of that multiplicity, the other points
-# are put in spatial (Morton) order with a bounding box per 32 of them, and the kernel skips every candidate chunk
-# that an exact box bound rules out. Results are unchanged (the bound is evaluated in the kernel's own rounding); on
-# LiDAR clouds the search visits 11 % (un-sampled) to 38 % (2048 FPS samples) of the pairs: 1.8x the brute-force
-# kernel on the 1000 vs 1000 x 2048 evaluation. The choice depends on the shape only, so a given input always takes the
+# are put in k-d order with a bounding box per 32 of them, and the kernel visits candidate chunks nearest first and
+# skips every chunk that an exact box bound rules out. Results are unchanged (the bound is evaluated in the kernel's
+# own rounding); on LiDAR clouds the search visits 1.7 % (un-sampled, of the kept pairs) to 8.2 % (2048 FPS samples)
+# of the pairs: 5.4x the brute-force kernel on the 1000 vs 1000 x 2048 evaluation. The choice depends on the shape only, so a given input always takes the
 # same path (and every row shard of a matrix the same one). Smaller clouds keep the brute-force kernel: its register
 # tile, not pruning, is what pays there. Set it to a huge value to force the brute-force kernel (bench.py does, for
 # the roofline of that kernel).

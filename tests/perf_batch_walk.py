@@ -9,4 +9,4 @@ ref = bench.make_clouds(B, 2, head, lidar, dev, 1, True)
 gen = bench.make_clouds(B, 1, head, lidar, dev, 1, True)
 d = chamfer_distance(ref, gen)
 ms = statistics.median(bench.time_events(lambda: chamfer_distance(ref, gen), 10, 3))
-print("batch %d x 32768: %.1f us" % (B, ms * 1e3), os.environ.get("DUSTY_CHAMFER_WALK"), os.environ.get("DUSTY_CHAMFER_BATCH_KD"))
+print("batch %d x 32768: %.1f us" % (B, ms * 1e3))

@@ -1,4 +1,4 @@
-"""A/B of the resident-pair kernels on the evaluation's shape (env: DUSTY_CHAMFER_PAIR, DUSTY_CHAMFER_PAIR_SPLIT; N, P, ABOVE)."""
+"""Timing of the resident-pair kernel on the evaluation's shape (env: N, P, ABOVE); not a test."""
 import os, sys, statistics, ctypes as C
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -17,6 +17,5 @@ ms = statistics.median(bench.time_events(run, 3, 1))
 cnt = C.c_uint64()
 _lib.load().dusty_chamfer_count_pairs(1, None); run(); _lib.load().dusty_chamfer_count_pairs(0, C.byref(cnt))
 E2 = N * (2 * N + 1)
-print("PAIR=%s SPLIT=%s N=%d P=%d: %.1f ms  %.0f entries/s  visited %.4f  scores %s" % (
-    os.environ.get("DUSTY_CHAMFER_PAIR", "1"), os.environ.get("DUSTY_CHAMFER_PAIR_SPLIT", "1"), N, P, ms, 3 * N * N / ms * 1e3,
-    cnt.value / (E2 * 2 * P * P), pr))
+print("N=%d P=%d: %.1f ms  %.0f entries/s  visited %.4f  scores %s" % (
+    N, P, ms, 3 * N * N / ms * 1e3, cnt.value / (E2 * 2 * P * P), pr))

@@ -1,5 +1,5 @@
-"""A/B of the best-first walk on un-sampled clouds (env DUSTY_CHAMFER_WALK): matrix front end (configs[4] shape) and
-batch front end (8 pairs x 32768 points); not a test."""
+"""Timing of the best-first walk on un-sampled clouds: matrix front end (configs[4] shape, env N) and batch front end
+(8 pairs x 32768 points); not a test."""
 import os, sys, statistics, ctypes as C
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -18,11 +18,11 @@ cnt = C.c_uint64()
 _lib.load().dusty_chamfer_count_pairs(1, None); run(); _lib.load().dusty_chamfer_count_pairs(0, C.byref(cnt))
 kept = torch.cat([(c != 0).any(-1).sum(1) + ((c == 0).all(-1).any(1)).long() for c in (ref, gen)]).double()
 kept_pairs = float((kept.sum() ** 2 + (kept ** 2).sum()) / 2) * 2
-print("WALK=%s matrix N=%d: %.1f ms  %.0f entries/s  visited %.4f of kept pairs  %s" % (
-    os.environ.get("DUSTY_CHAMFER_WALK", "1"), N, ms, 3 * N * N / ms * 1e3, cnt.value / kept_pairs,
+print("matrix N=%d: %.1f ms  %.0f entries/s  visited %.4f of kept pairs  %s" % (
+    N, ms, 3 * N * N / ms * 1e3, cnt.value / kept_pairs,
     {k: pr[k] for k in ("mmd-cd", "cov-cd", "1-nn-accuracy-cd")}))
 a, b = ref[:8].contiguous(), gen[:8].contiguous()
 d = chamfer_distance(a, b)
 ms = statistics.median(bench.time_events(lambda: chamfer_distance(a, b), 10, 3))
-print("WALK=%s batch 8 x 32768: %.1f us  %.0f pairs/s  checksum %.9g %.9g" % (
-    os.environ.get("DUSTY_CHAMFER_WALK", "1"), ms * 1e3, 8 / ms * 1e3, d[0].double().sum().item(), d[1].double().sum().item()))
+print("batch 8 x 32768: %.1f us  %.0f pairs/s  checksum %.9g %.9g" % (
+    ms * 1e3, 8 / ms * 1e3, d[0].double().sum().item(), d[1].double().sum().item()))

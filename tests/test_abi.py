@@ -142,12 +142,8 @@ def test_hot_kernels_keep_their_occupancy_shape():
     for frag in ("nn_kernelILi8ELb1ELb0ELi128", "nn_kernelILi8ELb1ELb0ELi64", "nn_kernelILi8ELb1ELb0ELi32"):
         n = one(frag)
         assert int(usage[n]) <= 128 and int(local[n]) == 0, frag
-    for frag in ("nn_kernelILi4ELb1ELb1ELi64ELi512", "nn_kernelILi4ELb0ELb1ELi64ELi512"):      # pruned search on sorted clouds:
-        n = one(frag)                                                                           # ten 2-warp CTAs per SM
-        assert int(usage[n]) <= 102 and int(local[n]) <= 32, frag
-    for frag in ("nn_pair_split_kernel", "nn_pair_kernelILi2ELi8E"):      # resident-pair kernels: three 8-warp CTAs per SM
-        pair = one(frag)
-        assert int(usage[pair]) <= 85 and int(local[pair]) <= 16       # (the stack bytes belong to the double-division subroutine of the epilogue)
+    pair = one("nn_pair_split_kernel")                                 # resident-pair kernel: three 8-warp CTAs per SM
+    assert int(usage[pair]) <= 85 and int(local[pair]) <= 16           # (the stack bytes belong to the double-division subroutine of the epilogue)
     assert int(usage[one("head_project_kernelILi1ELb0E")]) <= 32         # 8 CTAs of 256 threads per SM
     assert int(usage[one("head_project_kernelILi2ELb0E")]) <= 36         # DUSty-II: 7 CTAs per SM
     assert int(usage[one("head_project_kernelILi1ELb1E")]) <= 48         # with compaction: 5 CTAs per SM, 16 KB smem each

@@ -200,10 +200,10 @@ def test_matrix_sorted_search_is_the_default_above_256_points():
                                             (2048, 2048, 0.4), (2048, 65, 0.5), (33, 2048, 0.2), (2048, 2049, 0.0)])
 def test_matrix_resident_pair_kernel_against_oracle(pa, pb, dropped):
     """Clouds of at most 2048 points with merged origins: k-d ordered by prep_sort_kernel<true>, searched by
-    nn_pair_kernel (both clouds in shared memory, best-first chunk walk). Every entry against the CUDA-rounding
-    oracle, for point counts that are not multiples of the 64-row groups or the 32-candidate chunks, clouds with
+    nn_pair_split_kernel (both clouds in shared memory, best-first chunk walk). Every entry against the CUDA-rounding
+    oracle, for point counts that are not multiples of the 32-row groups or the 32-candidate chunks, clouds with
     and without dropped (0,0,0) points, degenerate clouds, and 2049 points (one past the kernel's capacity: the
-    Morton-sorted tile kernel). Two runs are bit-identical although warps take their row groups dynamically."""
+    two-level walk nn_walk_split_kernel). Two runs are bit-identical although warps take their row groups dynamically."""
     a = lidar_like_clouds(4, pa, 700 + pa, dropped=dropped); b = lidar_like_clouds(3, pb, 800 + pb, dropped=dropped)
     b[1] = b[1][0]                                           # every point the same
     if dropped:

@@ -63,7 +63,7 @@ def test_configs3_dusty2_clouds_64_vs_64_every_entry_and_score():
 
 def test_configs4_unsampled_clouds_through_the_sorted_and_pruned_path():
     """configs[4] shape: un-sampled 64x512 clouds (32 768 points, dropped pixels at the origin) through
-    chamfer_matrix's default path for them: origin points merged, kept points Morton-sorted, chunks pruned by
+    chamfer_matrix's default path for them: origin points merged, kept points in k-d order, chunks pruned by
     box distance. 3 vs 2 clouds from the DUSty-I head, every entry against the oracle on all 32 768 points."""
     from dusty_gan_b200.utils.metrics.cov_mmd_1nna import chamfer_matrix
     a, b = head_clouds(1, 3, 401), head_clouds(1, 2, 402)
@@ -75,7 +75,7 @@ def test_configs4_unsampled_clouds_through_the_sorted_and_pruned_path():
     S = chamfer_matrix(a)
     assert torch.equal(S, S.t()) and bool((S.diagonal() == 0).all())
     assert_matrix(S, native.pairwise_cd(a.cpu().numpy(), None))
-    # the same entries with pruning off and with merging off: all three instantiations agree to the ulp
+    # the same entries with merging off: both paths agree to the ulp
     for kw in (dict(merge_origin=False),):
         assert_matrix(chamfer_matrix(a, b, **kw), native.pairwise_cd(a.cpu().numpy(), b.cpu().numpy()))
 
