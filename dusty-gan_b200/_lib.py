@@ -94,6 +94,10 @@ SIGNATURES = {
     "dusty_head_project_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "dusty_head_project": (C.c_int, [C.POINTER(HeadParams), c_float_p, c_float_p, c_float_p, c_float_p, c_float_p,
                                      c_float_p, c_int_p, c_int_p, c_float_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dusty_head_project_backward_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "dusty_head_project_backward": (C.c_int, [C.POINTER(HeadParams), c_float_p, c_float_p, c_float_p, c_float_p,
+                                              c_float_p, c_float_p, c_float_p, c_float_p, c_float_p, C.c_void_p,
+                                              C.c_size_t, C.c_void_p]),
     "dusty_inv_to_xyz": (C.c_int, [C.POINTER(HeadParams), c_float_p, c_float_p, c_float_p, C.c_void_p]),
     "dusty_scan_preprocess": (C.c_int, [C.POINTER(ScanParams), c_float_p, c_float_p, c_float_p, c_float_p, c_float_p,
                                         c_float_p, C.c_void_p]),

@@ -13,6 +13,10 @@
 // functions ATen's CUDA kernels call), so masks and points are bit-identical to the reference
 // run on the same GPU. HBM traffic per pixel: read depth + confidence, write mask + depth + xyz
 // = 28 B (DUSty-I) / 36 B (DUSty-II); the noise map and the trig table are small and L2 resident.
+//
+// The backward (head_backward_kernel) is the gradient autograd produces through the same chain. It saves nothing:
+// it rebuilds every forward value with the forward's helpers from the same inputs and noise, and rounds the chain
+// rule where autograd's kernels round it.
 #include <algorithm>
 #include <cstdlib>
 
@@ -488,6 +492,184 @@ __global__ void __launch_bounds__(TPB) gumbel_sigmoid_kernel(const float* __rest
                          gate_value(cv.z, g.mode, na.z, nb.z, p), gate_value(cv.w, g.mode, na.w, nb.w, p)));
 }
 
+// ---- backward of head_project_kernel ----
+struct BwdArgs {
+  dusty_head_params p;
+  GateDev gp, gi;
+  const float* depth;
+  const float* conf;
+  const float* trig;
+  const float* grad_mask;     // (b,C,h,w) or NULL
+  const float* grad_depth;    // (b,1,h,w) or NULL
+  const float* grad_points;   // layout p.points_layout; NULL unless the PROJ instantiation runs
+  float* grad_depth_in;
+  float* grad_conf;
+  float* tau_partial;         // one float per CTA, or NULL when d/d inv_tau is not wanted
+  int npix;
+  int segs_per_image;
+};
+
+// Gradient of GumbelSigmoid with respect to its logit, given the gradient g of its (straight-through or soft)
+// output. The soft value is rebuilt from the same noise and in the same rounding as gate_value. The term
+// d soft / d inv_tau is added to tau; a gate without noise is (logit > 0): no gradient.
+__device__ __forceinline__ float gate_grad(float logit, int mode, float na, float nb, float g, const dusty_head_params& p,
+                                           float& tau) {
+  if (mode == DUSTY_NOISE_NONE) return 0.0f;
+  const float l = mode == DUSTY_NOISE_UNIFORM ? logistic_from_uniform(na, nb, p.eps) : na;
+  const float xl = __fadd_rn(logit, l);
+  const float soft = __frcp_rn(__fadd_rn(1.0f, expf(-__fmul_rn(xl, p.inv_tau))));
+  const float gx = __fmul_rn(__fmul_rn(g, __fsub_rn(1.0f, soft)), soft);     // ATen sigmoid_backward: (g * (1 - y)) * y
+  tau = __fadd_rn(tau, __fmul_rn(gx, xl));
+  return __fmul_rn(gx, p.inv_tau);
+}
+
+__device__ __forceinline__ float4 ldg_or_zero(const float* base, long long off) {
+  return base ? ldg_stream(reinterpret_cast<const float4*>(base + off)) : make_float4(0, 0, 0, 0);
+}
+
+// One 4-pixel group per thread, the forward's grid. Every forward value (gates, mask, dout, inv, validity) is
+// recomputed with the forward's helpers from the same inputs and noise, hence bit-identical to what the forward
+// returned. PROJ adds the projection's gradient; interleaved grad_points arrive through the forward's per-warp
+// transpose run backwards (coalesced 512-byte loads per warp instruction).
+template <int C, bool PROJ>
+__global__ void __launch_bounds__(TPB, PROJ ? 3 : 4) head_backward_kernel(const BwdArgs a) {
+  __shared__ __align__(16) float stage[PROJ ? (TPB / 32) * 384 : 4];
+  __shared__ float wtau[TPB / 32];
+  const dusty_head_params& p = a.p;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const long long img = blockIdx.x / a.segs_per_image;
+  const int seg = (int)(blockIdx.x - (unsigned)img * a.segs_per_image);
+  const int npix = a.npix;
+  const int pix = seg * GROUP + tid * 4;
+  float tau = 0.0f;
+  float4 gpx = make_float4(0, 0, 0, 0), gpy = gpx, gpz = gpx;
+  if (PROJ) {
+    if (p.points_layout == 0) {
+      if (pix < npix) {
+        const float* g = a.grad_points + img * 3 * npix + pix;
+        gpx = ldg_stream(reinterpret_cast<const float4*>(g));
+        gpy = ldg_stream(reinterpret_cast<const float4*>(g + npix));
+        gpz = ldg_stream(reinterpret_cast<const float4*>(g + 2 * npix));
+      }
+    } else {
+      const int wpix = seg * GROUP + warp * 128;
+      float4 v0 = make_float4(0, 0, 0, 0), v1 = v0, v2 = v0;
+      if (wpix + 128 <= npix) {                         // whole warp in range (uniform)
+        const float4* g = reinterpret_cast<const float4*>(a.grad_points + (img * npix + wpix) * 3);
+        float4* wst = reinterpret_cast<float4*>(stage + warp * 384);
+        wst[lane] = ldg_stream(g + lane);
+        wst[lane + 32] = ldg_stream(g + lane + 32);
+        wst[lane + 64] = ldg_stream(g + lane + 64);
+        __syncwarp();
+        v0 = wst[lane * 3]; v1 = wst[lane * 3 + 1]; v2 = wst[lane * 3 + 2];
+      } else if (pix < npix) {
+        const float4* g = reinterpret_cast<const float4*>(a.grad_points + (img * npix + pix) * 3);
+        v0 = ldg_stream(g); v1 = ldg_stream(g + 1); v2 = ldg_stream(g + 2);
+      }
+      gpx = make_float4(v0.x, v0.w, v1.z, v2.y);
+      gpy = make_float4(v0.y, v1.x, v1.w, v2.z);
+      gpz = make_float4(v0.z, v1.y, v2.x, v2.w);
+    }
+  }
+  if (pix < npix) {
+    const float* conf0 = a.conf + img * C * npix;
+    const float4 dv = ldg_stream(reinterpret_cast<const float4*>(a.depth + img * npix + pix));
+    const float4 cv = ldg_stream(reinterpret_cast<const float4*>(conf0 + pix));
+    const float4 c1 = C == 2 ? ldg_stream(reinterpret_cast<const float4*>(conf0 + npix + pix)) : make_float4(0, 0, 0, 0);
+    const float4 gd = ldg_or_zero(a.grad_depth, img * npix + pix);
+    const float4 gm0 = ldg_or_zero(a.grad_mask, img * C * npix + pix);
+    const float4 gm1 = C == 2 ? ldg_or_zero(a.grad_mask, img * C * npix + npix + pix) : make_float4(0, 0, 0, 0);
+    float4 na = make_float4(0, 0, 0, 0), nb = na, ia = na, ib = na;
+    if (a.gp.mode != DUSTY_NOISE_NONE) na = load_noise(a.gp, a.gp.a, img, pix);
+    if (a.gp.mode == DUSTY_NOISE_UNIFORM) nb = load_noise(a.gp, a.gp.b, img, pix);
+    if (C == 2 && a.gi.mode != DUSTY_NOISE_NONE) ia = load_noise(a.gi, a.gi.a, img, pix);
+    if (C == 2 && a.gi.mode == DUSTY_NOISE_UNIFORM) ib = load_noise(a.gi, a.gi.b, img, pix);
+    const float din[4] = {dv.x, dv.y, dv.z, dv.w}, cp[4] = {cv.x, cv.y, cv.z, cv.w}, ci[4] = {c1.x, c1.y, c1.z, c1.w};
+    const float gdv[4] = {gd.x, gd.y, gd.z, gd.w}, gmp[4] = {gm0.x, gm0.y, gm0.z, gm0.w}, gmi[4] = {gm1.x, gm1.y, gm1.z, gm1.w};
+    const float nav[4] = {na.x, na.y, na.z, na.w}, nbv[4] = {nb.x, nb.y, nb.z, nb.w};
+    const float iav[4] = {ia.x, ia.y, ia.z, ia.w}, ibv[4] = {ib.x, ib.y, ib.z, ib.w};
+    float grng[4] = {0.f, 0.f, 0.f, 0.f};
+    if (PROJ) {
+      // d/d range of ((r cos el) cos az, (r cos el) sin az, r sin el): autograd's operand order, and the order in
+      // which its engine adds the three branches (z, then y, then x)
+      const float4 ce = *reinterpret_cast<const float4*>(a.trig + pix);
+      const float4 se = *reinterpret_cast<const float4*>(a.trig + npix + pix);
+      const float4 ca = *reinterpret_cast<const float4*>(a.trig + 2 * npix + pix);
+      const float4 sa = *reinterpret_cast<const float4*>(a.trig + 3 * npix + pix);
+      const float cev[4] = {ce.x, ce.y, ce.z, ce.w}, sev[4] = {se.x, se.y, se.z, se.w};
+      const float cav[4] = {ca.x, ca.y, ca.z, ca.w}, sav[4] = {sa.x, sa.y, sa.z, sa.w};
+      const float gx[4] = {gpx.x, gpx.y, gpx.z, gpx.w}, gy[4] = {gpy.x, gpy.y, gpy.z, gpy.w}, gz[4] = {gpz.x, gpz.y, gpz.z, gpz.w};
+      #pragma unroll
+      for (int q = 0; q < 4; ++q)
+        grng[q] = __fadd_rn(__fadd_rn(__fmul_rn(gz[q], sev[q]), __fmul_rn(__fmul_rn(gy[q], sav[q]), cev[q])),
+                            __fmul_rn(__fmul_rn(gx[q], cav[q]), cev[q]));
+    }
+    float gdin[4], gc0[4], gc1[4];
+    #pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const float mp = gate_value(cp[q], a.gp.mode, nav[q], nbv[q], p);
+      const float mi = C == 2 ? gate_value(ci[q], a.gi.mode, iav[q], ibv[q], p) : 1.0f;
+      const float mk = C == 2 ? __fmul_rn(mp, mi) : mp;
+      float gdout = gdv[q];
+      if (PROJ) {
+        const float dout = __fadd_rn(__fmul_rn(mk, din[q]), __fmul_rn(__fsub_rn(1.0f, mk), p.drop_const));
+        const float pre = __fmul_rn(__fadd_rn(dout, 1.0f), 0.5f);
+        const float inv = pre < 0.0f ? 0.0f : (pre > 1.0f ? 1.0f : pre);
+        bool valid;
+        range_from_inv(inv, p, valid);
+        const float rcp = __frcp_rn(__fadd_rn(__fmul_rn(inv, p.disp_scale), p.disp_shift));
+        float g = __fmul_rn(grng[q], valid ? 1.0f : 0.0f);
+        g = __fmul_rn(__fmul_rn(__fmul_rn(g, p.inv_max_depth), p.range), p.inv_range);
+        g = __fmul_rn(-g, __fmul_rn(rcp, rcp));                       // reciprocal_backward: -g * (y * y)
+        g = __fmul_rn(g, p.disp_scale);
+        g = (pre >= 0.0f && pre <= 1.0f) ? g : 0.0f;                  // clamp_backward keeps the bounds
+        gdout = __fadd_rn(gdout, __fmul_rn(g, 0.5f));
+      }
+      gdin[q] = __fmul_rn(gdout, mk);
+      // d/d mask of mask * depth + (1 - mask) * drop_const; DUSty-I adds it to the mask's own gradient in the order
+      // autograd does: (grad_mask - g * drop_const) + g * depth
+      const float gdrop = __fmul_rn(gdout, p.drop_const), gblend = __fmul_rn(gdout, din[q]);
+      if (C == 1) {
+        gc0[q] = gate_grad(cp[q], a.gp.mode, nav[q], nbv[q], __fadd_rn(__fsub_rn(gmp[q], gdrop), gblend), p, tau);
+      } else {
+        const float gm = __fsub_rn(gblend, gdrop);
+        gc0[q] = gate_grad(cp[q], a.gp.mode, nav[q], nbv[q], __fadd_rn(__fmul_rn(gm, mi), gmp[q]), p, tau);
+        gc1[q] = gate_grad(ci[q], a.gi.mode, iav[q], ibv[q], __fadd_rn(__fmul_rn(gm, mp), gmi[q]), p, tau);
+      }
+    }
+    float* gco = a.grad_conf + img * C * npix + pix;
+    stg_stream(reinterpret_cast<float4*>(a.grad_depth_in + img * npix + pix), make_float4(gdin[0], gdin[1], gdin[2], gdin[3]));
+    stg_stream(reinterpret_cast<float4*>(gco), make_float4(gc0[0], gc0[1], gc0[2], gc0[3]));
+    if (C == 2) stg_stream(reinterpret_cast<float4*>(gco + npix), make_float4(gc1[0], gc1[1], gc1[2], gc1[3]));
+  }
+  if (a.tau_partial == nullptr) return;
+  // per-CTA partial of d/d inv_tau: fixed shuffle tree, then the 8 warp sums in warp order
+  #pragma unroll
+  for (int o = 16; o > 0; o >>= 1) tau = __fadd_rn(tau, __shfl_xor_sync(0xffffffffu, tau, o));
+  if (lane == 0) wtau[warp] = tau;
+  __syncthreads();
+  if (tid == 0) {
+    float s = 0.0f;
+    #pragma unroll
+    for (int w = 0; w < TPB / 32; ++w) s = __fadd_rn(s, wtau[w]);
+    a.tau_partial[blockIdx.x] = s;
+  }
+}
+
+// d/d inv_tau = sum of the per-CTA partials: one CTA, fixed order (strided per thread, then a fixed tree), in double.
+__global__ void __launch_bounds__(TPB) head_backward_tau_kernel(const float* __restrict__ partial, int n, float* __restrict__ out) {
+  __shared__ double s[TPB];
+  double acc = 0.0;
+  for (int i = threadIdx.x; i < n; i += TPB) acc += (double)partial[i];
+  s[threadIdx.x] = acc;
+  __syncthreads();
+  for (int o = TPB / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *out = (float)s[0];
+}
+
 static int check_params(const dusty_head_params* p, const char* who) {
   if (!p) return fail_arg(DUSTY_EINVAL, "%s: null params", who);
   if (p->b < 0 || p->h <= 0 || p->w <= 0) return fail_arg(DUSTY_EINVAL, "%s: bad shape b=%d h=%d w=%d", who, p->b, p->h, p->w);
@@ -584,6 +766,61 @@ extern "C" int dusty_head_project(const dusty_head_params* p, const float* depth
     else head_project_kernel<2, false><<<(unsigned)ctas, TPB, 0, st>>>(a);
   }
   DUSTY_AFTER_LAUNCH("head_project_kernel");
+  return 0;
+}
+
+extern "C" size_t dusty_head_project_backward_workspace_bytes(int b, int h, int w) {
+  if (b <= 0 || h <= 0 || w <= 0) return 0;
+  const long long segs = ((long long)h * w + GROUP - 1) / GROUP;
+  return align_up((size_t)b * segs * sizeof(float), 256);      // one partial of d/d inv_tau per CTA
+}
+
+extern "C" int dusty_head_project_backward(const dusty_head_params* p, const float* depth, const float* confidence,
+                                           const float* trig, const float* grad_mask, const float* grad_depth,
+                                           const float* grad_points, float* grad_depth_in, float* grad_confidence,
+                                           float* grad_inv_tau, void* workspace, size_t workspace_bytes, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (int rc = check_params(p, "head_project_backward")) return rc;
+  if (p->conf_channels != 1 && p->conf_channels != 2)
+    return fail_arg(DUSTY_EINVAL, "head_project_backward: conf_channels must be 1 or 2");
+  if (p->b == 0) return 0;
+  if (!depth || !confidence || !grad_depth_in || !grad_confidence || (grad_points && !trig))
+    return fail_arg(DUSTY_EINVAL, "head_project_backward: null pointer");
+  if (!aligned16(depth) || !aligned16(confidence) || (trig && !aligned16(trig)) || !aligned16(grad_mask) ||
+      !aligned16(grad_depth) || !aligned16(grad_points) || !aligned16(grad_depth_in) || !aligned16(grad_confidence))
+    return fail_arg(DUSTY_EALIGN, "head_project_backward: tensors must be 16-byte aligned");
+  if (int rc = check_gate(p->gate_pixel, "pixel")) return rc;
+  if (p->conf_channels == 2) if (int rc = check_gate(p->gate_image, "image")) return rc;
+  const size_t ws_need = dusty_head_project_backward_workspace_bytes(p->b, p->h, p->w);
+  if (grad_inv_tau && (!workspace || workspace_bytes < ws_need))
+    return fail_arg(DUSTY_ENOSPACE, "head_project_backward: grad_inv_tau needs %zu workspace bytes", ws_need);
+  BwdArgs a{};
+  a.p = *p;
+  a.gp = GateDev{p->gate_pixel.mode, p->gate_pixel.noise_a, p->gate_pixel.noise_b, p->gate_pixel.batch_stride, (int)p->gate_pixel.pixel_stride};
+  a.gi = GateDev{p->gate_image.mode, p->gate_image.noise_a, p->gate_image.noise_b, p->gate_image.batch_stride, (int)p->gate_image.pixel_stride};
+  if (p->conf_channels == 1) a.gi.mode = DUSTY_NOISE_NONE;
+  a.depth = depth; a.conf = confidence; a.trig = trig;
+  a.grad_mask = grad_mask; a.grad_depth = grad_depth; a.grad_points = grad_points;
+  a.grad_depth_in = grad_depth_in; a.grad_conf = grad_confidence;
+  a.tau_partial = grad_inv_tau ? static_cast<float*>(workspace) : nullptr;
+  a.npix = p->h * p->w;
+  a.segs_per_image = (a.npix + GROUP - 1) / GROUP;
+  const long long ctas = (long long)p->b * a.segs_per_image;
+  if (ctas > 0x7fffffffLL) return fail_arg(DUSTY_EINVAL, "head_project_backward: grid too large");
+  if (int rc = check_device()) return rc;
+  const bool proj = grad_points != nullptr;
+  if (p->conf_channels == 1) {
+    if (proj) head_backward_kernel<1, true><<<(unsigned)ctas, TPB, 0, st>>>(a);
+    else head_backward_kernel<1, false><<<(unsigned)ctas, TPB, 0, st>>>(a);
+  } else {
+    if (proj) head_backward_kernel<2, true><<<(unsigned)ctas, TPB, 0, st>>>(a);
+    else head_backward_kernel<2, false><<<(unsigned)ctas, TPB, 0, st>>>(a);
+  }
+  DUSTY_AFTER_LAUNCH("head_backward_kernel");
+  if (grad_inv_tau) {
+    head_backward_tau_kernel<<<1, TPB, 0, st>>>(a.tau_partial, (int)ctas, grad_inv_tau);
+    DUSTY_AFTER_LAUNCH("head_backward_tau_kernel");
+  }
   return 0;
 }
 

@@ -5,13 +5,16 @@ Same class names, constructor arguments, attribute names (``fixed_noise``, ``dro
 ``utils.setup``'s fixed-noise forward pre-hook (reference utils/__init__.py:141-149) is registered on the
 GumbelSigmoid modules; the fused heads do not call those modules, so ``_head_call`` runs their pre-hooks
 itself before reading ``fixed_noise`` (``tests/test_gpu_head.py::test_setup_fixed_noise_hook_*``). The
-element-wise chains run as single CUDA kernels through the C ABI.
+element-wise chains run as single CUDA kernels through the C ABI, and so does their backward: ``maskout``,
+``forward`` and ``pipeline.maskout_and_project(..., differentiable=True)`` carry gradients to the backbone's
+``depth`` and ``confidence`` (and to a learnable temperature) through ``dusty_head_project_backward``.
 """
 import ctypes as C
 
 import numpy as np
 import torch
 from torch import nn
+from torch.autograd.function import once_differentiable
 
 from .. import _lib
 
@@ -194,11 +197,54 @@ def _drop_value(module):
     return cached[1]
 
 
+class _HeadFn(torch.autograd.Function):
+    """``dusty_head_project`` as an autograd op: (depth, confidence, temperature weight) -> (mask, depth, points).
+    ``launch`` runs the forward kernel into ``outputs``. The backward kernel rebuilds every forward value from the
+    same inputs and noise, so the forward keeps only its inputs, its parameters (``params``, whose noise pointers
+    stay valid because ``keep`` holds the noise tensors), the trig table and the gate module."""
+
+    @staticmethod
+    def forward(ctx, depth, conf, weight, launch, outputs, params, trig, keep, gate):
+        ctx.set_materialize_grads(False)
+        launch()
+        ctx.params, ctx.trig, ctx.keep, ctx.gate = params, trig, keep, gate
+        ctx.save_for_backward(depth, conf, weight)
+        return outputs
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_mask, g_depth, g_points):
+        depth, conf, weight = ctx.saved_tensors
+        lib = _lib.load()
+        grads = [None if g is None else g.contiguous() for g in (g_mask, g_depth, g_points)]
+        grad_depth = torch.empty_like(depth)
+        grad_conf = torch.empty_like(conf)
+        want_tau = weight is not None and ctx.needs_input_grad[2]
+        grad_tau = torch.empty((), device=depth.device, dtype=torch.float32) if want_tau else None
+        p = ctx.params
+        ws_bytes = lib.dusty_head_project_backward_workspace_bytes(p.b, p.h, p.w) if want_tau else 0
+        ws = _lib.workspace(ws_bytes, depth.device) if want_tau else None
+        with torch.cuda.device(depth.device):
+            _lib.check(lib.dusty_head_project_backward(
+                C.byref(p), _lib.ptr(depth), _lib.ptr(conf), _lib.ptr(ctx.trig if grads[2] is not None else None),
+                *(_lib.ptr(g) for g in grads), _lib.ptr(grad_depth), _lib.ptr(grad_conf), _lib.ptr(grad_tau),
+                _lib.ptr(ws), ws_bytes, _lib.stream_of(depth)), "dusty_head_project_backward")
+        grad_weight = None
+        if want_tau:       # inv_tau = softplus(weight) + 1/tau_max (reference models/dusty.py:39-41)
+            with torch.enable_grad():
+                (grad_weight,) = torch.autograd.grad(ctx.gate._inverse_tau_tensor(), ctx.gate.weight, grad_tau)
+        return (grad_depth if ctx.needs_input_grad[0] else None, grad_conf if ctx.needs_input_grad[1] else None,
+                grad_weight, None, None, None, None, None, None)
+
+
 def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1, compact=False, buffers=None):
     """Shared body of maskout (lidar=None) and the fused generate->points path (lidar given).
     ``buffers`` may hold preallocated ``mask``, ``depth``, ``points`` (and, for ``compact``, ``valid_count``,
     ``valid_index``, ``valid_points``, ``workspace``) tensors to write into (steady-state callers reuse them; the
-    evaluate loop of the reference reallocates every batch)."""
+    evaluate loop of the reference reallocates every batch).
+
+    When grad mode is on and ``depth`` or ``confidence`` requires grad, the launch runs inside ``_HeadFn``: the
+    returned mask, depth and points then carry gradients (compaction outputs excepted)."""
     buffers = buffers or {}
     assert isinstance(output, dict)
     assert "confidence" in output
@@ -210,9 +256,11 @@ def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1,
     if depth.dim() != 4 or depth.shape[1] != 1 or conf.shape != (depth.shape[0], channels, *depth.shape[2:]):
         raise ValueError(f"expected depth (B,1,H,W) and confidence (B,{channels},H,W), got "
                          f"{tuple(depth.shape)} and {tuple(conf.shape)}")
-    if torch.is_grad_enabled() and (depth.requires_grad or conf.requires_grad):
-        raise NotImplementedError("the fused head is forward-only (evaluate path runs under no_grad, reference "
-                                  "evaluate_synthesis.py:24); use GumbelSigmoid for a differentiable gate")
+    differentiable = torch.is_grad_enabled() and (depth.requires_grad or conf.requires_grad)
+    if differentiable and channels == 2 and module.training and module.gumbel_pixel.tau is None:
+        raise NotImplementedError("DUSty2 with a learnable temperature (tau=None) in training mode: the fused kernel "
+                                  "reads one inv_tau for both gates, so the gradients of the two gates' weights "
+                                  "cannot be separated")
     d, c = depth.contiguous(), conf.contiguous()
     B, _, H, W = d.shape
     p = _lib.HeadParams()
@@ -267,11 +315,17 @@ def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1,
     ws = (buffers.get("workspace") if buffers.get("workspace") is not None else _lib.workspace(ws_bytes, d.device)) if compact else None
     if ws is not None and ws.numel() < ws_bytes:
         raise ValueError("preallocated workspace is too small")
-    with torch.cuda.device(d.device):
-        _lib.check(lib.dusty_head_project(C.byref(p), _lib.ptr(d), _lib.ptr(c), _lib.ptr(trig), _lib.ptr(mask),
-                                          _lib.ptr(dout), _lib.ptr(points), _lib.ptr(count), _lib.ptr(index),
-                                          _lib.ptr(compacted), _lib.ptr(ws), ws_bytes, _lib.stream_of(d)),
-                   "dusty_head_project")
+    def launch():
+        with torch.cuda.device(d.device):
+            _lib.check(lib.dusty_head_project(C.byref(p), _lib.ptr(d), _lib.ptr(c), _lib.ptr(trig), _lib.ptr(mask),
+                                              _lib.ptr(dout), _lib.ptr(points), _lib.ptr(count), _lib.ptr(index),
+                                              _lib.ptr(compacted), _lib.ptr(ws), ws_bytes, _lib.stream_of(d)),
+                       "dusty_head_project")
+    if differentiable:
+        mask, dout, points = _HeadFn.apply(d, c, gm.weight if gm.tau is None else None, launch, (mask, dout, points),
+                                           p, trig, keep, gm)
+    else:
+        launch()
     output["depth_orig"] = depth
     output["mask"] = mask
     output["depth"] = dout

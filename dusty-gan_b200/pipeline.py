@@ -9,6 +9,8 @@ and the real-data side of the same script (evaluate_synthesis.py:49-57, 69-110):
 
     raw (64,2048,4) scans -> preprocess_reals (one kernel) -> downsample_point_clouds -> {"2d","3d"} cache
 """
+import contextlib
+
 import torch
 
 from .datasets.kitti import preprocess_scans
@@ -16,14 +18,22 @@ from .models.dusty import _head_call
 from .utils.sampling.fps import downsample_point_clouds
 
 
-@torch.no_grad()
-def maskout_and_project(head, output, lidar, tol=0.0, threshold=0.5, compact=False, buffers=None):
+def maskout_and_project(head, output, lidar, tol=0.0, threshold=0.5, compact=False, buffers=None,
+                        differentiable=False):
     """``head`` is a DUSty1/DUSty2 module, ``output`` the backbone's dict. Returns the dict updated like
     ``maskout`` plus ``points`` (B,H*W,3) -- the contiguous layout FPS consumes -- and, with
     ``compact=True``, ``valid_count`` (B,), ``valid_index`` (B,H*W) and ``valid_points`` (B,H*W,3):
-    the valid pixels of each image in ascending pixel order (what ``points[i][valid[i]]`` selects)."""
-    out, points, count, index, compacted = _head_call(head, output, threshold, lidar=lidar, tol=tol,
-                                                      points_layout=1, compact=compact, buffers=buffers)
+    the valid pixels of each image in ascending pixel order (what ``points[i][valid[i]]`` selects).
+
+    Runs under ``no_grad`` unless ``differentiable=True``; then ``depth``, ``mask`` and ``points`` carry gradients
+    to ``output["depth"]`` and ``output["confidence"]`` (the inversion loss of demo.py:510-515 back-propagates a
+    Chamfer loss on the points to the latent). Compaction outputs have no gradient, so ``compact=True`` is refused
+    there."""
+    if differentiable and compact:
+        raise ValueError("maskout_and_project: compact=True has no gradient; use differentiable=False")
+    with contextlib.nullcontext() if differentiable else torch.no_grad():
+        out, points, count, index, compacted = _head_call(head, output, threshold, lidar=lidar, tol=tol,
+                                                          points_layout=1, compact=compact, buffers=buffers)
     out["points"] = points
     if compact:
         out["valid_count"], out["valid_index"], out["valid_points"] = count, index, compacted

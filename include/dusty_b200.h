@@ -40,6 +40,8 @@
  *   dusty_head_project           models/dusty.py:45-59,77-91,107-127 (GumbelSigmoid.forward,
  *                                DUSty1.maskout, DUSty2.maskout) fused with utils/__init__.py:76-79
  *                                (tanh_to_sigmoid + clamp) and utils/lidar.py:38-68 (inv_to_xyz)
+ *   dusty_head_project_backward  the autograd backward of the same chain (the straight-through mask gradient),
+ *                                e.g. demo.py:510-515's inversion loss and the generator step of trainers/dcgan_amp.py
  *   dusty_inv_to_xyz             utils/lidar.py:61-68     (Coordinate.inv_to_xyz alone)
  *   dusty_scan_preprocess        datasets/kitti.py:54-78 (KITTIOdometry.preprocess + transform's nearest
  *                                resize) fused with evaluate_synthesis.py:49-57 (preprocess_reals:
@@ -339,6 +341,24 @@ DUSTY_API size_t dusty_head_project_workspace_bytes(int b, int h, int w);
 DUSTY_API int dusty_head_project(const dusty_head_params* p, const float* depth, const float* confidence,
                        const float* trig, float* out_mask, float* out_depth, float* out_points,
                        int32_t* out_count, int32_t* out_index, float* out_compact,
+                       void* workspace, size_t workspace_bytes, void* stream);
+
+/* Backward of dusty_head_project: the gradient autograd gives through the reference's op chain (GumbelSigmoid's
+ * straight-through estimator, the mask blend, tanh_to_sigmoid + clamp, inv_to_xyz), with every forward value
+ * recomputed bit-identically from the forward's inputs; nothing is saved by the forward.
+ *   p, depth, confidence: exactly what the forward received, gate noise pointers included.
+ *   Upstream gradients, each NULL for zero: grad_mask (b,C,h,w), grad_depth (b,1,h,w), grad_points in
+ *   p->points_layout. trig (4,h,w) is required when grad_points is given.
+ *   grad_depth_in (b,1,h,w), grad_confidence (b,C,h,w): overwritten. Channel 1 of a DUSty-II gate without noise
+ *   (DUSTY_NOISE_NONE, eval mode) is 0.
+ *   grad_inv_tau: NULL, or one float that receives d loss / d p->inv_tau summed over every gate with noise; it
+ *   needs dusty_head_project_backward_workspace_bytes() of workspace and is reduced in a fixed order (no atomics),
+ *   so repeated calls give bit-identical results.
+ *   All tensor pointers must be 16-byte aligned and w a multiple of 4. */
+DUSTY_API size_t dusty_head_project_backward_workspace_bytes(int b, int h, int w);
+DUSTY_API int dusty_head_project_backward(const dusty_head_params* p, const float* depth, const float* confidence,
+                       const float* trig, const float* grad_mask, const float* grad_depth, const float* grad_points,
+                       float* grad_depth_in, float* grad_confidence, float* grad_inv_tau,
                        void* workspace, size_t workspace_bytes, void* stream);
 
 /* Projection only: inv (b,1,h,w) in [0,1] (already tanh_to_sigmoid'ed and clamped) -> xyz. */
