@@ -18,14 +18,14 @@ c_int_p = C.c_void_p
 
 
 class Gate(C.Structure):
-    _fields_ = [("mode", C.c_int32), ("reserved", C.c_int32), ("noise_a", C.c_void_p), ("noise_b", C.c_void_p),
-                ("batch_stride", C.c_int64), ("pixel_stride", C.c_int64)]
+    _fields_ = [("mode", C.c_int32), ("hard", C.c_int32), ("noise_a", C.c_void_p), ("noise_b", C.c_void_p),
+                ("batch_stride", C.c_int64), ("pixel_stride", C.c_int64), ("inv_tau", C.c_float), ("eps", C.c_float)]
 
 
 class HeadParams(C.Structure):
     _fields_ = [("b", C.c_int32), ("h", C.c_int32), ("w", C.c_int32), ("conf_channels", C.c_int32),
                 ("gate_pixel", Gate), ("gate_image", Gate),
-                ("inv_tau", C.c_float), ("threshold", C.c_float), ("eps", C.c_float), ("drop_const", C.c_float),
+                ("threshold", C.c_float), ("drop_const", C.c_float),
                 ("tol", C.c_float), ("disp_scale", C.c_float), ("disp_shift", C.c_float), ("min_depth", C.c_float),
                 ("inv_range", C.c_float), ("range", C.c_float), ("inv_max_depth", C.c_float),
                 ("points_layout", C.c_int32)]
@@ -38,7 +38,7 @@ class ScanParams(C.Structure):
                 ("disp_lo", C.c_float), ("inv_disp_range", C.c_float), ("drop_const", C.c_float)]
 
 
-ABI_VERSION = 2          # DUSTY_B200_ABI_VERSION of include/dusty_b200.h
+ABI_VERSION = 3          # DUSTY_B200_ABI_VERSION of include/dusty_b200.h
 NOISE_NONE, NOISE_LOGISTIC, NOISE_UNIFORM = 0, 1, 2
 MATRIX_SYMMETRIC, MATRIX_MIRROR, MATRIX_COMPACT_ROWS, MATRIX_PREPARED, MATRIX_MERGE_ORIGIN = 1, 2, 4, 8, 16
 
@@ -89,8 +89,7 @@ SIGNATURES = {
     "dusty_gather_points_grad": (C.c_int, [c_float_p, c_int_p, C.c_int, C.c_int, C.c_int, C.c_int, c_float_p,
                                            C.c_void_p]),
     "dusty_logistic_noise": (C.c_int, [c_float_p, c_float_p, C.c_float, C.c_size_t, c_float_p, C.c_void_p]),
-    "dusty_gumbel_sigmoid": (C.c_int, [c_float_p, C.POINTER(Gate), C.c_float, C.c_float, C.c_float, C.c_int, C.c_int,
-                                       c_float_p, C.c_void_p]),
+    "dusty_gumbel_sigmoid": (C.c_int, [c_float_p, C.POINTER(Gate), C.c_float, C.c_int, C.c_int, c_float_p, C.c_void_p]),
     "dusty_head_project_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "dusty_head_project": (C.c_int, [C.POINTER(HeadParams), c_float_p, c_float_p, c_float_p, c_float_p, c_float_p,
                                      c_float_p, c_int_p, c_int_p, c_float_p, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -28,12 +28,16 @@ namespace head {
 constexpr int TPB = 256;
 constexpr int GROUP = TPB * 4;          // pixels per CTA (1024)
 
+// One gate as the kernels read it: its noise (dusty_gate) and its own scalars
 struct GateDev {
   int mode;
+  int hard;
   const float* a;
   const float* b;
   long long bstride;
   int pstride;
+  float inv_tau;
+  float eps;
 };
 
 struct Args {
@@ -60,14 +64,16 @@ __device__ __forceinline__ float logistic_from_uniform(float u1, float u2, float
   return -logf(__fadd_rn(__fdiv_rn(l1, l2), eps));
 }
 
-// GumbelSigmoid.forward for one logit; returns the straight-through forward value.
-__device__ __forceinline__ float gate_value(float logit, int mode, float na, float nb, const dusty_head_params& p) {
-  if (mode == DUSTY_NOISE_NONE) return logit > 0.0f ? 1.0f : 0.0f;
-  const float l = mode == DUSTY_NOISE_UNIFORM ? logistic_from_uniform(na, nb, p.eps) : na;
-  const float x = __fmul_rn(__fadd_rn(logit, l), p.inv_tau);
+// GumbelSigmoid.forward of gate g for one logit: the straight-through value, or the soft one when !g.hard.
+// The gate is taken by value: a reference into the kernel's parameter costs the 32-register forward kernels 8-16
+// more bytes of spills.
+__device__ __forceinline__ float gate_value(float logit, const GateDev g, float na, float nb, float threshold) {
+  if (g.mode == DUSTY_NOISE_NONE) return logit > 0.0f ? 1.0f : 0.0f;
+  const float l = g.mode == DUSTY_NOISE_UNIFORM ? logistic_from_uniform(na, nb, g.eps) : na;
+  const float x = __fmul_rn(__fadd_rn(logit, l), g.inv_tau);
   const float soft = __frcp_rn(__fadd_rn(1.0f, expf(-x)));     // == 1.0f / y: both are the correctly rounded quotient
-  if (p.threshold != p.threshold) return soft;               // NaN threshold: GumbelSigmoid(hard=False)
-  const float hard = soft > p.threshold ? 1.0f : 0.0f;
+  if (!g.hard) return soft;                                    // GumbelSigmoid(hard=False)
+  const float hard = soft > threshold ? 1.0f : 0.0f;           // a NaN threshold gives 0, as in the reference
   return __fadd_rn(__fsub_rn(hard, soft), soft);
 }
 
@@ -134,16 +140,16 @@ __global__ void __launch_bounds__(TPB, C == 1 ? 8 : 7) head_project_kernel(const
     float4 na = make_float4(0, 0, 0, 0), nb = na;
     if (a.gp.mode != DUSTY_NOISE_NONE) na = load_noise(a.gp, a.gp.a, img, pix);
     if (a.gp.mode == DUSTY_NOISE_UNIFORM) nb = load_noise(a.gp, a.gp.b, img, pix);
-    float mp[4] = {gate_value(cv.x, a.gp.mode, na.x, nb.x, p), gate_value(cv.y, a.gp.mode, na.y, nb.y, p),
-                   gate_value(cv.z, a.gp.mode, na.z, nb.z, p), gate_value(cv.w, a.gp.mode, na.w, nb.w, p)};
+    float mp[4] = {gate_value(cv.x, a.gp, na.x, nb.x, p.threshold), gate_value(cv.y, a.gp, na.y, nb.y, p.threshold),
+                   gate_value(cv.z, a.gp, na.z, nb.z, p.threshold), gate_value(cv.w, a.gp, na.w, nb.w, p.threshold)};
     float mk[4] = {mp[0], mp[1], mp[2], mp[3]};
     stg_stream(reinterpret_cast<float4*>(omask0 + pix), make_float4(mp[0], mp[1], mp[2], mp[3]));
     if (C == 2) {
       float4 ia = make_float4(0, 0, 0, 0), ib = ia;
       if (a.gi.mode != DUSTY_NOISE_NONE) ia = load_noise(a.gi, a.gi.a, img, pix);
       if (a.gi.mode == DUSTY_NOISE_UNIFORM) ib = load_noise(a.gi, a.gi.b, img, pix);
-      const float mi[4] = {gate_value(c1.x, a.gi.mode, ia.x, ib.x, p), gate_value(c1.y, a.gi.mode, ia.y, ib.y, p),
-                           gate_value(c1.z, a.gi.mode, ia.z, ib.z, p), gate_value(c1.w, a.gi.mode, ia.w, ib.w, p)};
+      const float mi[4] = {gate_value(c1.x, a.gi, ia.x, ib.x, p.threshold), gate_value(c1.y, a.gi, ia.y, ib.y, p.threshold),
+                           gate_value(c1.z, a.gi, ia.z, ib.z, p.threshold), gate_value(c1.w, a.gi, ia.w, ib.w, p.threshold)};
       stg_stream(reinterpret_cast<float4*>(omask0 + npix + pix), make_float4(mi[0], mi[1], mi[2], mi[3]));
       #pragma unroll
       for (int q = 0; q < 4; ++q) mk[q] = __fmul_rn(mp[q], mi[q]);
@@ -332,16 +338,16 @@ __global__ void __launch_bounds__(IMG_TPB, 2) head_project_image_kernel(const Ar
       if (noise_tile) na = *reinterpret_cast<const float4*>(tab + 4 * IMG_STEP);
       else if (a.gp.mode != DUSTY_NOISE_NONE) na = load_noise(a.gp, a.gp.a, img, pix);
       if (a.gp.mode == DUSTY_NOISE_UNIFORM) nb = load_noise(a.gp, a.gp.b, img, pix);
-      float mp[4] = {gate_value(ccur.x, a.gp.mode, na.x, nb.x, p), gate_value(ccur.y, a.gp.mode, na.y, nb.y, p),
-                     gate_value(ccur.z, a.gp.mode, na.z, nb.z, p), gate_value(ccur.w, a.gp.mode, na.w, nb.w, p)};
+      float mp[4] = {gate_value(ccur.x, a.gp, na.x, nb.x, p.threshold), gate_value(ccur.y, a.gp, na.y, nb.y, p.threshold),
+                     gate_value(ccur.z, a.gp, na.z, nb.z, p.threshold), gate_value(ccur.w, a.gp, na.w, nb.w, p.threshold)};
       float mk[4] = {mp[0], mp[1], mp[2], mp[3]};
       stg_stream(reinterpret_cast<float4*>(omask0 + pix), make_float4(mp[0], mp[1], mp[2], mp[3]));
       if (C == 2) {
         float4 ia = make_float4(0, 0, 0, 0), ib = ia;
         if (a.gi.mode != DUSTY_NOISE_NONE) ia = load_noise(a.gi, a.gi.a, img, pix);
         if (a.gi.mode == DUSTY_NOISE_UNIFORM) ib = load_noise(a.gi, a.gi.b, img, pix);
-        const float mi[4] = {gate_value(c1cur.x, a.gi.mode, ia.x, ib.x, p), gate_value(c1cur.y, a.gi.mode, ia.y, ib.y, p),
-                             gate_value(c1cur.z, a.gi.mode, ia.z, ib.z, p), gate_value(c1cur.w, a.gi.mode, ia.w, ib.w, p)};
+        const float mi[4] = {gate_value(c1cur.x, a.gi, ia.x, ib.x, p.threshold), gate_value(c1cur.y, a.gi, ia.y, ib.y, p.threshold),
+                             gate_value(c1cur.z, a.gi, ia.z, ib.z, p.threshold), gate_value(c1cur.w, a.gi, ia.w, ib.w, p.threshold)};
         stg_stream(reinterpret_cast<float4*>(omask0 + npix + pix), make_float4(mi[0], mi[1], mi[2], mi[3]));
         #pragma unroll
         for (int q = 0; q < 4; ++q) mk[q] = __fmul_rn(mp[q], mi[q]);
@@ -479,7 +485,7 @@ __global__ void __launch_bounds__(TPB) logistic_noise_kernel(const float* __rest
 }
 
 __global__ void __launch_bounds__(TPB) gumbel_sigmoid_kernel(const float* __restrict__ logits, const GateDev g,
-                                                             const dusty_head_params p, int npix, float* __restrict__ out) {
+                                                             float threshold, int npix, float* __restrict__ out) {
   const long long img = blockIdx.y;
   const int pix = (blockIdx.x * TPB + threadIdx.x) * 4;
   if (pix >= npix) return;
@@ -488,8 +494,8 @@ __global__ void __launch_bounds__(TPB) gumbel_sigmoid_kernel(const float* __rest
   if (g.mode != DUSTY_NOISE_NONE) na = load_noise(g, g.a, img, pix);
   if (g.mode == DUSTY_NOISE_UNIFORM) nb = load_noise(g, g.b, img, pix);
   stg_stream(reinterpret_cast<float4*>(out + img * npix + pix),
-             make_float4(gate_value(cv.x, g.mode, na.x, nb.x, p), gate_value(cv.y, g.mode, na.y, nb.y, p),
-                         gate_value(cv.z, g.mode, na.z, nb.z, p), gate_value(cv.w, g.mode, na.w, nb.w, p)));
+             make_float4(gate_value(cv.x, g, na.x, nb.x, threshold), gate_value(cv.y, g, na.y, nb.y, threshold),
+                         gate_value(cv.z, g, na.z, nb.z, threshold), gate_value(cv.w, g, na.w, nb.w, threshold)));
 }
 
 // ---- backward of head_project_kernel ----
@@ -504,23 +510,22 @@ struct BwdArgs {
   const float* grad_points;   // layout p.points_layout; NULL unless the PROJ instantiation runs
   float* grad_depth_in;
   float* grad_conf;
-  float* tau_partial;         // one float per CTA, or NULL when d/d inv_tau is not wanted
+  float* tau_partial;         // per gate, one float per CTA (pixel gate, then image gate), or NULL when d/d inv_tau is not wanted
   int npix;
   int segs_per_image;
 };
 
-// Gradient of GumbelSigmoid with respect to its logit, given the gradient g of its (straight-through or soft)
-// output. The soft value is rebuilt from the same noise and in the same rounding as gate_value. The term
-// d soft / d inv_tau is added to tau; a gate without noise is (logit > 0): no gradient.
-__device__ __forceinline__ float gate_grad(float logit, int mode, float na, float nb, float g, const dusty_head_params& p,
-                                           float& tau) {
-  if (mode == DUSTY_NOISE_NONE) return 0.0f;
-  const float l = mode == DUSTY_NOISE_UNIFORM ? logistic_from_uniform(na, nb, p.eps) : na;
+// Gradient of gate gt's GumbelSigmoid with respect to its logit, given the gradient g of its (straight-through or
+// soft) output. The soft value is rebuilt from the same noise and in the same rounding as gate_value. The term
+// d soft / d inv_tau is added to the gate's own accumulator tau; a gate without noise is (logit > 0): no gradient.
+__device__ __forceinline__ float gate_grad(float logit, const GateDev gt, float na, float nb, float g, float& tau) {
+  if (gt.mode == DUSTY_NOISE_NONE) return 0.0f;
+  const float l = gt.mode == DUSTY_NOISE_UNIFORM ? logistic_from_uniform(na, nb, gt.eps) : na;
   const float xl = __fadd_rn(logit, l);
-  const float soft = __frcp_rn(__fadd_rn(1.0f, expf(-__fmul_rn(xl, p.inv_tau))));
+  const float soft = __frcp_rn(__fadd_rn(1.0f, expf(-__fmul_rn(xl, gt.inv_tau))));
   const float gx = __fmul_rn(__fmul_rn(g, __fsub_rn(1.0f, soft)), soft);     // ATen sigmoid_backward: (g * (1 - y)) * y
   tau = __fadd_rn(tau, __fmul_rn(gx, xl));
-  return __fmul_rn(gx, p.inv_tau);
+  return __fmul_rn(gx, gt.inv_tau);
 }
 
 __device__ __forceinline__ float4 ldg_or_zero(const float* base, long long off) {
@@ -534,14 +539,14 @@ __device__ __forceinline__ float4 ldg_or_zero(const float* base, long long off) 
 template <int C, bool PROJ>
 __global__ void __launch_bounds__(TPB, PROJ ? 3 : 4) head_backward_kernel(const BwdArgs a) {
   __shared__ __align__(16) float stage[PROJ ? (TPB / 32) * 384 : 4];
-  __shared__ float wtau[TPB / 32];
+  __shared__ float wtau[C][TPB / 32];
   const dusty_head_params& p = a.p;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long img = blockIdx.x / a.segs_per_image;
   const int seg = (int)(blockIdx.x - (unsigned)img * a.segs_per_image);
   const int npix = a.npix;
   const int pix = seg * GROUP + tid * 4;
-  float tau = 0.0f;
+  float tau_p = 0.0f, tau_i = 0.0f;         // d/d inv_tau of the pixel and the image gate
   float4 gpx = make_float4(0, 0, 0, 0), gpy = gpx, gpz = gpx;
   if (PROJ) {
     if (p.points_layout == 0) {
@@ -607,8 +612,8 @@ __global__ void __launch_bounds__(TPB, PROJ ? 3 : 4) head_backward_kernel(const 
     float gdin[4], gc0[4], gc1[4];
     #pragma unroll
     for (int q = 0; q < 4; ++q) {
-      const float mp = gate_value(cp[q], a.gp.mode, nav[q], nbv[q], p);
-      const float mi = C == 2 ? gate_value(ci[q], a.gi.mode, iav[q], ibv[q], p) : 1.0f;
+      const float mp = gate_value(cp[q], a.gp, nav[q], nbv[q], p.threshold);
+      const float mi = C == 2 ? gate_value(ci[q], a.gi, iav[q], ibv[q], p.threshold) : 1.0f;
       const float mk = C == 2 ? __fmul_rn(mp, mi) : mp;
       float gdout = gdv[q];
       if (PROJ) {
@@ -630,11 +635,11 @@ __global__ void __launch_bounds__(TPB, PROJ ? 3 : 4) head_backward_kernel(const 
       // autograd does: (grad_mask - g * drop_const) + g * depth
       const float gdrop = __fmul_rn(gdout, p.drop_const), gblend = __fmul_rn(gdout, din[q]);
       if (C == 1) {
-        gc0[q] = gate_grad(cp[q], a.gp.mode, nav[q], nbv[q], __fadd_rn(__fsub_rn(gmp[q], gdrop), gblend), p, tau);
+        gc0[q] = gate_grad(cp[q], a.gp, nav[q], nbv[q], __fadd_rn(__fsub_rn(gmp[q], gdrop), gblend), tau_p);
       } else {
         const float gm = __fsub_rn(gblend, gdrop);
-        gc0[q] = gate_grad(cp[q], a.gp.mode, nav[q], nbv[q], __fadd_rn(__fmul_rn(gm, mi), gmp[q]), p, tau);
-        gc1[q] = gate_grad(ci[q], a.gi.mode, iav[q], ibv[q], __fadd_rn(__fmul_rn(gm, mp), gmi[q]), p, tau);
+        gc0[q] = gate_grad(cp[q], a.gp, nav[q], nbv[q], __fadd_rn(__fmul_rn(gm, mi), gmp[q]), tau_p);
+        gc1[q] = gate_grad(ci[q], a.gi, iav[q], ibv[q], __fadd_rn(__fmul_rn(gm, mp), gmi[q]), tau_i);
       }
     }
     float* gco = a.grad_conf + img * C * npix + pix;
@@ -643,22 +648,30 @@ __global__ void __launch_bounds__(TPB, PROJ ? 3 : 4) head_backward_kernel(const 
     if (C == 2) stg_stream(reinterpret_cast<float4*>(gco + npix), make_float4(gc1[0], gc1[1], gc1[2], gc1[3]));
   }
   if (a.tau_partial == nullptr) return;
-  // per-CTA partial of d/d inv_tau: fixed shuffle tree, then the 8 warp sums in warp order
+  // per-CTA partial of d/d inv_tau for each gate: fixed shuffle tree, then the 8 warp sums in warp order
   #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) tau = __fadd_rn(tau, __shfl_xor_sync(0xffffffffu, tau, o));
-  if (lane == 0) wtau[warp] = tau;
+  for (int o = 16; o > 0; o >>= 1) {
+    tau_p = __fadd_rn(tau_p, __shfl_xor_sync(0xffffffffu, tau_p, o));
+    if (C == 2) tau_i = __fadd_rn(tau_i, __shfl_xor_sync(0xffffffffu, tau_i, o));
+  }
+  if (lane == 0) {
+    wtau[0][warp] = tau_p;
+    if (C == 2) wtau[C - 1][warp] = tau_i;
+  }
   __syncthreads();
-  if (tid == 0) {
+  if (tid < C) {                         // thread 0: pixel gate, thread 1: image gate
     float s = 0.0f;
     #pragma unroll
-    for (int w = 0; w < TPB / 32; ++w) s = __fadd_rn(s, wtau[w]);
-    a.tau_partial[blockIdx.x] = s;
+    for (int w = 0; w < TPB / 32; ++w) s = __fadd_rn(s, wtau[tid][w]);
+    a.tau_partial[tid * gridDim.x + blockIdx.x] = s;
   }
 }
 
-// d/d inv_tau = sum of the per-CTA partials: one CTA, fixed order (strided per thread, then a fixed tree), in double.
+// d/d inv_tau of gate blockIdx.x = sum of its n per-CTA partials: one CTA per gate, fixed order (strided per thread,
+// then a fixed tree), in double.
 __global__ void __launch_bounds__(TPB) head_backward_tau_kernel(const float* __restrict__ partial, int n, float* __restrict__ out) {
   __shared__ double s[TPB];
+  partial += (long long)blockIdx.x * n;
   double acc = 0.0;
   for (int i = threadIdx.x; i < n; i += TPB) acc += (double)partial[i];
   s[threadIdx.x] = acc;
@@ -667,7 +680,7 @@ __global__ void __launch_bounds__(TPB) head_backward_tau_kernel(const float* __r
     if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
     __syncthreads();
   }
-  if (threadIdx.x == 0) *out = (float)s[0];
+  if (threadIdx.x == 0) out[blockIdx.x] = (float)s[0];
 }
 
 static int check_params(const dusty_head_params* p, const char* who) {
@@ -681,6 +694,7 @@ static int check_params(const dusty_head_params* p, const char* who) {
 
 static int check_gate(const dusty_gate& g, const char* name) {
   if (g.mode < DUSTY_NOISE_NONE || g.mode > DUSTY_NOISE_UNIFORM) return fail_arg(DUSTY_EINVAL, "head_project: %s gate mode %d", name, g.mode);
+  if (g.hard != 0 && g.hard != 1) return fail_arg(DUSTY_EINVAL, "head_project: %s gate hard must be 0 or 1", name);
   if (g.mode != DUSTY_NOISE_NONE && !g.noise_a) return fail_arg(DUSTY_EINVAL, "head_project: %s gate needs noise_a", name);
   if (g.mode == DUSTY_NOISE_UNIFORM && !g.noise_b) return fail_arg(DUSTY_EINVAL, "head_project: %s gate needs noise_b", name);
   if (g.pixel_stride != 0 && g.pixel_stride != 1) return fail_arg(DUSTY_EINVAL, "head_project: %s gate pixel_stride must be 0 or 1", name);
@@ -689,6 +703,10 @@ static int check_gate(const dusty_gate& g, const char* name) {
       return fail_arg(DUSTY_EALIGN, "head_project: %s gate noise must be 16-byte aligned with batch_stride %% 4 == 0", name);
   }
   return 0;
+}
+
+static GateDev gate_dev(const dusty_gate& g) {
+  return GateDev{g.mode, g.hard, g.noise_a, g.noise_b, g.batch_stride, (int)g.pixel_stride, g.inv_tau, g.eps};
 }
 
 }  // namespace head
@@ -723,8 +741,8 @@ extern "C" int dusty_head_project(const dusty_head_params* p, const float* depth
   if (p->conf_channels == 2) if (int rc = check_gate(p->gate_image, "image")) return rc;
   Args a{};
   a.p = *p;
-  a.gp = GateDev{p->gate_pixel.mode, p->gate_pixel.noise_a, p->gate_pixel.noise_b, p->gate_pixel.batch_stride, (int)p->gate_pixel.pixel_stride};
-  a.gi = GateDev{p->gate_image.mode, p->gate_image.noise_a, p->gate_image.noise_b, p->gate_image.batch_stride, (int)p->gate_image.pixel_stride};
+  a.gp = gate_dev(p->gate_pixel);
+  a.gi = gate_dev(p->gate_image);
   if (p->conf_channels == 1) a.gi.mode = DUSTY_NOISE_NONE;
   a.depth = depth; a.conf = confidence; a.trig = trig;
   a.out_mask = out_mask; a.out_depth = out_depth; a.out_points = out_points;
@@ -772,7 +790,7 @@ extern "C" int dusty_head_project(const dusty_head_params* p, const float* depth
 extern "C" size_t dusty_head_project_backward_workspace_bytes(int b, int h, int w) {
   if (b <= 0 || h <= 0 || w <= 0) return 0;
   const long long segs = ((long long)h * w + GROUP - 1) / GROUP;
-  return align_up((size_t)b * segs * sizeof(float), 256);      // one partial of d/d inv_tau per CTA
+  return align_up(2 * (size_t)b * segs * sizeof(float), 256);      // one partial of d/d inv_tau per gate and CTA
 }
 
 extern "C" int dusty_head_project_backward(const dusty_head_params* p, const float* depth, const float* confidence,
@@ -796,8 +814,8 @@ extern "C" int dusty_head_project_backward(const dusty_head_params* p, const flo
     return fail_arg(DUSTY_ENOSPACE, "head_project_backward: grad_inv_tau needs %zu workspace bytes", ws_need);
   BwdArgs a{};
   a.p = *p;
-  a.gp = GateDev{p->gate_pixel.mode, p->gate_pixel.noise_a, p->gate_pixel.noise_b, p->gate_pixel.batch_stride, (int)p->gate_pixel.pixel_stride};
-  a.gi = GateDev{p->gate_image.mode, p->gate_image.noise_a, p->gate_image.noise_b, p->gate_image.batch_stride, (int)p->gate_image.pixel_stride};
+  a.gp = gate_dev(p->gate_pixel);
+  a.gi = gate_dev(p->gate_image);
   if (p->conf_channels == 1) a.gi.mode = DUSTY_NOISE_NONE;
   a.depth = depth; a.conf = confidence; a.trig = trig;
   a.grad_mask = grad_mask; a.grad_depth = grad_depth; a.grad_points = grad_points;
@@ -818,14 +836,14 @@ extern "C" int dusty_head_project_backward(const dusty_head_params* p, const flo
   }
   DUSTY_AFTER_LAUNCH("head_backward_kernel");
   if (grad_inv_tau) {
-    head_backward_tau_kernel<<<1, TPB, 0, st>>>(a.tau_partial, (int)ctas, grad_inv_tau);
+    head_backward_tau_kernel<<<(unsigned)p->conf_channels, TPB, 0, st>>>(a.tau_partial, (int)ctas, grad_inv_tau);
     DUSTY_AFTER_LAUNCH("head_backward_tau_kernel");
   }
   return 0;
 }
 
-extern "C" int dusty_gumbel_sigmoid(const float* logits, const dusty_gate* gate, float inv_tau, float threshold, float eps,
-                                    int b, int npix, float* out, void* stream) {
+extern "C" int dusty_gumbel_sigmoid(const float* logits, const dusty_gate* gate, float threshold, int b, int npix, float* out,
+                                    void* stream) {
   if (b < 0 || npix <= 0 || npix % 4 != 0) return fail_arg(DUSTY_EINVAL, "gumbel_sigmoid: bad shape b=%d npix=%d", b, npix);
   if (b == 0) return 0;
   if (b > 65535) return fail_arg(DUSTY_EINVAL, "gumbel_sigmoid: batch %d exceeds 65535", b);
@@ -833,10 +851,8 @@ extern "C" int dusty_gumbel_sigmoid(const float* logits, const dusty_gate* gate,
   if (!logits || !gate || !out) return fail_arg(DUSTY_EINVAL, "gumbel_sigmoid: null pointer");
   if (!aligned16(logits) || !aligned16(out)) return fail_arg(DUSTY_EALIGN, "gumbel_sigmoid: tensors must be 16-byte aligned");
   if (int rc = check_gate(*gate, "gumbel")) return rc;
-  dusty_head_params p{};
-  p.inv_tau = inv_tau; p.threshold = threshold; p.eps = eps;
-  const GateDev g{gate->mode, gate->noise_a, gate->noise_b, gate->batch_stride, (int)gate->pixel_stride};
-  gumbel_sigmoid_kernel<<<dim3((npix / 4 + TPB - 1) / TPB, b), TPB, 0, static_cast<cudaStream_t>(stream)>>>(logits, g, p, npix, out);
+  gumbel_sigmoid_kernel<<<dim3((npix / 4 + TPB - 1) / TPB, b), TPB, 0, static_cast<cudaStream_t>(stream)>>>(
+      logits, gate_dev(*gate), threshold, npix, out);
   DUSTY_AFTER_LAUNCH("gumbel_sigmoid_kernel");
   return 0;
 }

@@ -7,7 +7,7 @@ GumbelSigmoid modules; the fused heads do not call those modules, so ``_head_cal
 itself before reading ``fixed_noise`` (``tests/test_gpu_head.py::test_setup_fixed_noise_hook_*``). The
 element-wise chains run as single CUDA kernels through the C ABI, and so does their backward: ``maskout``,
 ``forward`` and ``pipeline.maskout_and_project(..., differentiable=True)`` carry gradients to the backbone's
-``depth`` and ``confidence`` (and to a learnable temperature) through ``dusty_head_project_backward``.
+``depth`` and ``confidence`` (and to each gate's learnable temperature) through ``dusty_head_project_backward``.
 """
 import ctypes as C
 
@@ -35,7 +35,8 @@ def _run_forward_pre_hooks(module, logits):
 
 
 def _gate_struct(module, logits):
-    """Describe how ``module`` (a GumbelSigmoid) supplies its noise for ``logits`` (B,1,H,W).
+    """Describe ``module`` (a GumbelSigmoid) for ``logits`` (B,1,H,W): its own temperature, eps and ``hard`` flag,
+    and how it supplies its noise.
 
     Returns (Gate, keepalive tensors). With ``fixed_noise`` set the same (1,1,H,W) map is shared by
     the whole batch (reference models/dusty.py:48-50); otherwise fresh U1, U2 are drawn with the
@@ -43,6 +44,9 @@ def _gate_struct(module, logits):
     """
     B, _, H, W = logits.shape
     g = _lib.Gate()
+    g.hard = 1 if module.hard else 0
+    g.inv_tau = module._inv_tau()
+    g.eps = np.float32(module.eps)
     if module.fixed_noise is not None:
         noise = module.fixed_noise
         _lib.require_cuda(noise, "fixed_noise")
@@ -84,10 +88,8 @@ class _GumbelSigmoidFn(torch.autograd.Function):
         out = torch.empty_like(x)
         lib = _lib.load()
         with torch.cuda.device(x.device):
-            thr = np.float32(threshold) if module.hard else np.float32("nan")      # NaN: the kernel returns the soft mask
-            _lib.check(lib.dusty_gumbel_sigmoid(_lib.ptr(x), C.byref(gate), module._inv_tau(), thr,
-                                                np.float32(module.eps), B, H * W, _lib.ptr(out), _lib.stream_of(x)),
-                       "dusty_gumbel_sigmoid")
+            _lib.check(lib.dusty_gumbel_sigmoid(_lib.ptr(x), C.byref(gate), np.float32(threshold), B, H * W,
+                                                _lib.ptr(out), _lib.stream_of(x)), "dusty_gumbel_sigmoid")
         ctx.module = module
         # the soft mask is re-derived in backward from (logits, noise); keep the noise alive
         if gate.mode == _lib.NOISE_UNIFORM:
@@ -198,30 +200,32 @@ def _drop_value(module):
 
 
 class _HeadFn(torch.autograd.Function):
-    """``dusty_head_project`` as an autograd op: (depth, confidence, temperature weight) -> (mask, depth, points).
-    ``launch`` runs the forward kernel into ``outputs``. The backward kernel rebuilds every forward value from the
-    same inputs and noise, so the forward keeps only its inputs, its parameters (``params``, whose noise pointers
-    stay valid because ``keep`` holds the noise tensors), the trig table and the gate module."""
+    """``dusty_head_project`` as an autograd op: (depth, confidence, pixel gate's temperature weight, image gate's
+    temperature weight) -> (mask, depth, points). ``launch`` runs the forward kernel into ``outputs``. The backward
+    kernel rebuilds every forward value from the same inputs and noise, so the forward keeps only its inputs, its
+    parameters (``params``, whose noise pointers stay valid because ``keep`` holds the noise tensors), the trig table
+    and the gate modules (``gates``: pixel gate, image gate or None)."""
 
     @staticmethod
-    def forward(ctx, depth, conf, weight, launch, outputs, params, trig, keep, gate):
+    def forward(ctx, depth, conf, weight_pixel, weight_image, launch, outputs, params, trig, keep, gates):
         ctx.set_materialize_grads(False)
         launch()
-        ctx.params, ctx.trig, ctx.keep, ctx.gate = params, trig, keep, gate
-        ctx.save_for_backward(depth, conf, weight)
+        ctx.params, ctx.trig, ctx.keep, ctx.gates = params, trig, keep, gates
+        ctx.save_for_backward(depth, conf)
         return outputs
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g_mask, g_depth, g_points):
-        depth, conf, weight = ctx.saved_tensors
+        depth, conf = ctx.saved_tensors
         lib = _lib.load()
         grads = [None if g is None else g.contiguous() for g in (g_mask, g_depth, g_points)]
         grad_depth = torch.empty_like(depth)
         grad_conf = torch.empty_like(conf)
-        want_tau = weight is not None and ctx.needs_input_grad[2]
-        grad_tau = torch.empty((), device=depth.device, dtype=torch.float32) if want_tau else None
+        want_tau = ctx.needs_input_grad[2] or ctx.needs_input_grad[3]
         p = ctx.params
+        # d loss / d inv_tau of each gate: pixel, then (DUSty-II) image
+        grad_tau = torch.empty(p.conf_channels, device=depth.device, dtype=torch.float32) if want_tau else None
         ws_bytes = lib.dusty_head_project_backward_workspace_bytes(p.b, p.h, p.w) if want_tau else 0
         ws = _lib.workspace(ws_bytes, depth.device) if want_tau else None
         with torch.cuda.device(depth.device):
@@ -229,12 +233,13 @@ class _HeadFn(torch.autograd.Function):
                 C.byref(p), _lib.ptr(depth), _lib.ptr(conf), _lib.ptr(ctx.trig if grads[2] is not None else None),
                 *(_lib.ptr(g) for g in grads), _lib.ptr(grad_depth), _lib.ptr(grad_conf), _lib.ptr(grad_tau),
                 _lib.ptr(ws), ws_bytes, _lib.stream_of(depth)), "dusty_head_project_backward")
-        grad_weight = None
-        if want_tau:       # inv_tau = softplus(weight) + 1/tau_max (reference models/dusty.py:39-41)
-            with torch.enable_grad():
-                (grad_weight,) = torch.autograd.grad(ctx.gate._inverse_tau_tensor(), ctx.gate.weight, grad_tau)
+        grad_weights = [None, None]
+        for i, gate in enumerate(ctx.gates):
+            if ctx.needs_input_grad[2 + i]:     # inv_tau = softplus(weight) + 1/tau_max (reference models/dusty.py:39-41)
+                with torch.enable_grad():
+                    (grad_weights[i],) = torch.autograd.grad(gate._inverse_tau_tensor(), gate.weight, grad_tau[i])
         return (grad_depth if ctx.needs_input_grad[0] else None, grad_conf if ctx.needs_input_grad[1] else None,
-                grad_weight, None, None, None, None, None, None)
+                *grad_weights, None, None, None, None, None, None)
 
 
 def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1, compact=False, buffers=None):
@@ -257,10 +262,6 @@ def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1,
         raise ValueError(f"expected depth (B,1,H,W) and confidence (B,{channels},H,W), got "
                          f"{tuple(depth.shape)} and {tuple(conf.shape)}")
     differentiable = torch.is_grad_enabled() and (depth.requires_grad or conf.requires_grad)
-    if differentiable and channels == 2 and module.training and module.gumbel_pixel.tau is None:
-        raise NotImplementedError("DUSty2 with a learnable temperature (tau=None) in training mode: the fused kernel "
-                                  "reads one inv_tau for both gates, so the gradients of the two gates' weights "
-                                  "cannot be separated")
     d, c = depth.contiguous(), conf.contiguous()
     B, _, H, W = d.shape
     p = _lib.HeadParams()
@@ -270,6 +271,7 @@ def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1,
         _run_forward_pre_hooks(module.gumbel, c)
         p.gate_pixel, k = _gate_struct(module.gumbel, c)
         keep.append(k)
+        gates = (module.gumbel, None)
     else:
         _run_forward_pre_hooks(module.gumbel_pixel, c[:, :1])
         p.gate_pixel, k = _gate_struct(module.gumbel_pixel, c[:, :1])
@@ -278,12 +280,11 @@ def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1,
             _run_forward_pre_hooks(module.gumbel_image, c[:, 1:])
             p.gate_image, k = _gate_struct(module.gumbel_image, c[:, 1:])
             keep.append(k)
+            gates = (module.gumbel_pixel, module.gumbel_image)
         else:
             p.gate_image.mode = _lib.NOISE_NONE     # (logit > 0), reference models/dusty.py:120
-    gm = module.gumbel if channels == 1 else module.gumbel_pixel
-    p.inv_tau = gm._inv_tau()
+            gates = (module.gumbel_pixel, None)
     p.threshold = np.float32(threshold)
-    p.eps = np.float32(gm.eps)
     p.drop_const = np.float32(_drop_value(module))
     p.points_layout = points_layout
     mask = buffers["mask"] if "mask" in buffers else torch.empty_like(c)
@@ -322,8 +323,8 @@ def _head_call(module, output, threshold, lidar=None, tol=1e-8, points_layout=1,
                                               _lib.ptr(compacted), _lib.ptr(ws), ws_bytes, _lib.stream_of(d)),
                        "dusty_head_project")
     if differentiable:
-        mask, dout, points = _HeadFn.apply(d, c, gm.weight if gm.tau is None else None, launch, (mask, dout, points),
-                                           p, trig, keep, gm)
+        weights = [g.weight if g is not None and g.tau is None else None for g in gates]
+        mask, dout, points = _HeadFn.apply(d, c, *weights, launch, (mask, dout, points), p, trig, keep, gates)
     else:
         launch()
     output["depth_orig"] = depth

@@ -58,7 +58,7 @@
 extern "C" {
 #endif
 
-#define DUSTY_B200_ABI_VERSION 2
+#define DUSTY_B200_ABI_VERSION 3
 
 #if defined(__GNUC__)
 #define DUSTY_API __attribute__((visibility("default")))
@@ -286,18 +286,23 @@ DUSTY_API int dusty_gather_points_grad(const float* grad_out, const int32_t* idx
 DUSTY_API int dusty_logistic_noise(const float* u1, const float* u2, float eps, size_t count, float* out,
                          void* stream);
 
-/* How the relaxed-Bernoulli noise of one Gumbel-sigmoid gate is supplied. */
+/* One Gumbel-sigmoid gate (GumbelSigmoid, models/dusty.py:6-62): how its relaxed-Bernoulli noise is supplied, and
+ * the gate's own scalars. DUSty-II has two gates, and each keeps its own temperature, eps and output kind. */
 #define DUSTY_NOISE_NONE     0   /* gate is (logit > 0), DUSty2's eval-mode image gate */
 #define DUSTY_NOISE_LOGISTIC 1   /* noise_a holds l */
-#define DUSTY_NOISE_UNIFORM  2   /* noise_a, noise_b hold U1, U2; l is derived as above */
+#define DUSTY_NOISE_UNIFORM  2   /* noise_a, noise_b hold U1, U2; l as dusty_logistic_noise forms it, with the gate's eps */
 
 typedef struct dusty_gate {
   int32_t mode;             /* DUSTY_NOISE_* */
-  int32_t reserved;
+  int32_t hard;             /* 1: straight-through (hard - soft) + soft, hard = soft > threshold; 0: the soft mask
+                               (GumbelSigmoid(hard=False), models/dusty.py:58-59) */
   const float* noise_a;     /* l or U1 */
   const float* noise_b;     /* U2 or NULL */
   int64_t batch_stride;     /* elements between images in noise_a/b; 0 = one map shared by the batch */
   int64_t pixel_stride;     /* 1 = per-pixel map; 0 = one value per image */
+  float inv_tau;            /* f32(1.0/tau): ATen CUDA forms x/scalar as x * f32(1/double(scalar)); for the learnable
+                               temperature (tau=None, models/dusty.py:39-41) the f32 value of softplus(weight) + 1/tau_max */
+  float eps;                /* 1e-10; used when mode == DUSTY_NOISE_UNIFORM */
 } dusty_gate;
 
 typedef struct dusty_head_params {
@@ -305,9 +310,7 @@ typedef struct dusty_head_params {
   int32_t conf_channels;    /* 1 (DUSty-I) or 2 (DUSty-II: channel 0 pixel gate, channel 1 image gate) */
   dusty_gate gate_pixel;
   dusty_gate gate_image;    /* ignored when conf_channels == 1 */
-  float inv_tau;            /* f32(1.0/tau): ATen CUDA forms x/scalar as x * f32(1/double(scalar)) */
-  float threshold;          /* mask_soft > threshold */
-  float eps;                /* 1e-10 */
+  float threshold;          /* mask_soft > threshold, the same for both gates as in the reference */
   float drop_const;         /* generator-side drop value, -1 */
   /* projection constants, exactly the f32 scalars the reference's element-wise kernels receive */
   float tol;                /* |inv - 0| > tol */
@@ -320,13 +323,12 @@ typedef struct dusty_head_params {
   int32_t points_layout;    /* 0: xyz planar (b,3,h,w) like inv_to_xyz; 1: interleaved (b,h*w,3) */
 } dusty_head_params;
 
-/* GumbelSigmoid.forward alone (models/dusty.py:45-59): out = (hard - soft) + soft with
- * soft = 1/(1+exp(-((logit + l) * inv_tau))), hard = soft > threshold. A NaN threshold selects the soft output
- * (GumbelSigmoid(hard=False), models/dusty.py:58-59). inv_tau is f32(1/tau), or for the learnable temperature
- * (tau=None, :39-41) the f32 value of softplus(weight) + 1/tau_max. logits/out (b,1,h*w) f32, 16-byte aligned,
- * npix a multiple of 4. */
-DUSTY_API int dusty_gumbel_sigmoid(const float* logits, const dusty_gate* gate, float inv_tau, float threshold,
-                         float eps, int b, int npix, float* out, void* stream);
+/* GumbelSigmoid.forward alone (models/dusty.py:45-59): soft = 1/(1+exp(-((logit + l) * gate->inv_tau))); out is
+ * (hard - soft) + soft with hard = soft > threshold when gate->hard, else soft. A NaN threshold is an ordinary
+ * threshold: no soft value exceeds it, so a hard gate returns exact zeros, as the reference does.
+ * logits/out (b,1,h*w) f32, 16-byte aligned, npix a multiple of 4. */
+DUSTY_API int dusty_gumbel_sigmoid(const float* logits, const dusty_gate* gate, float threshold, int b, int npix,
+                         float* out, void* stream);
 
 /* Fused point-drop head + projection.
  *   depth (b,1,h,w), confidence (b,C,h,w): generator outputs (tanh range).
@@ -351,9 +353,9 @@ DUSTY_API int dusty_head_project(const dusty_head_params* p, const float* depth,
  *   p->points_layout. trig (4,h,w) is required when grad_points is given.
  *   grad_depth_in (b,1,h,w), grad_confidence (b,C,h,w): overwritten. Channel 1 of a DUSty-II gate without noise
  *   (DUSTY_NOISE_NONE, eval mode) is 0.
- *   grad_inv_tau: NULL, or one float that receives d loss / d p->inv_tau summed over every gate with noise; it
- *   needs dusty_head_project_backward_workspace_bytes() of workspace and is reduced in a fixed order (no atomics),
- *   so repeated calls give bit-identical results.
+ *   grad_inv_tau: NULL, or conf_channels floats: d loss / d gate_pixel.inv_tau, then (DUSty-II) d loss /
+ *   d gate_image.inv_tau; 0 for a gate without noise. It needs dusty_head_project_backward_workspace_bytes() of
+ *   workspace, and each float is reduced in a fixed order (no atomics), so repeated calls give bit-identical results.
  *   All tensor pointers must be 16-byte aligned and w a multiple of 4. */
 DUSTY_API size_t dusty_head_project_backward_workspace_bytes(int b, int h, int w);
 DUSTY_API int dusty_head_project_backward(const dusty_head_params* p, const float* depth, const float* confidence,

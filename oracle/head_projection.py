@@ -17,29 +17,37 @@ def logistic_noise(u1, u2, eps=1e-10):
     return -torch.log(torch.log(u1 + eps) / torch.log(u2 + eps) + eps)
 
 
-def gumbel_sigmoid(logits, noise, tau=1.0, threshold=0.5):
-    """reference models/dusty.py:45-59 (hard=True): noise is the logistic sample, fixed or fresh."""
+def gumbel_sigmoid(logits, noise, tau=1.0, threshold=0.5, hard=True):
+    """reference models/dusty.py:38-59: noise is the logistic sample, fixed or fresh. ``tau`` is a Python scalar
+    temperature (``x / tau``), or a 0-dim tensor holding the learnable inverse temperature
+    ``softplus(weight) + 1/tau_max`` (tau=None, :39-41: ``x * inverse_tau``). ``hard=False`` returns the soft mask."""
     x = logits + (noise.expand(logits.shape[0], -1, -1, -1) if noise.shape[0] == 1 else noise)
-    soft = torch.sigmoid(x / tau)
-    hard = (soft > threshold).float()
-    return hard - soft.detach() + soft
+    soft = torch.sigmoid(x * tau if isinstance(tau, torch.Tensor) else x / tau)
+    if not hard:
+        return soft
+    mask_hard = (soft > threshold).float()
+    return mask_hard - soft.detach() + soft
 
 
-def maskout_dusty1(depth, confidence, noise, tau=1.0, threshold=0.5, drop_const=-1.0):
+def maskout_dusty1(depth, confidence, noise, tau=1.0, threshold=0.5, drop_const=-1.0, hard=True):
     """reference models/dusty.py:77-91 -> (mask, depth_out)."""
     dc = torch.tensor(drop_const).float().to(depth.device)
-    mask = gumbel_sigmoid(confidence, noise, tau, threshold)
+    mask = gumbel_sigmoid(confidence, noise, tau, threshold, hard)
     return mask, mask * depth + (1 - mask) * dc
 
 
-def maskout_dusty2(depth, confidence, noise_pixel, tau=1.0, threshold=0.5, drop_const=-1.0, noise_image=None):
-    """reference models/dusty.py:107-127 -> (mask (B,2,H,W), depth_out); eval mode when noise_image is None."""
+def maskout_dusty2(depth, confidence, noise_pixel, tau=1.0, threshold=0.5, drop_const=-1.0, noise_image=None,
+                   hard=True, tau_image=None, hard_image=None):
+    """reference models/dusty.py:107-127 -> (mask (B,2,H,W), depth_out); eval mode when noise_image is None.
+    ``tau``/``hard`` are the pixel gate's; the image gate has its own ``tau_image``/``hard_image`` (None: the pixel
+    gate's). Both gates see the same threshold, as in the reference."""
     dc = torch.tensor(drop_const).float().to(depth.device)
-    mask_pixel = gumbel_sigmoid(confidence[:, [0]], noise_pixel, tau, threshold)
+    mask_pixel = gumbel_sigmoid(confidence[:, [0]], noise_pixel, tau, threshold, hard)
     if noise_image is None:
         mask_image = (confidence[:, [1]] > 0.0).float()
     else:
-        mask_image = gumbel_sigmoid(confidence[:, [1]], noise_image, tau, threshold)
+        mask_image = gumbel_sigmoid(confidence[:, [1]], noise_image, tau if tau_image is None else tau_image, threshold,
+                                    hard if hard_image is None else hard_image)
     mask = mask_pixel * mask_image
     return torch.cat([mask_pixel, mask_image], dim=1), mask * depth + (1 - mask) * dc
 

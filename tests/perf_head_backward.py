@@ -1,6 +1,7 @@
 """Speed of dusty_head_project_backward (not a test): batch 256 of 64x512 range images, DUSty-I / DUSty-II, fixed
-and fresh noise, maskout alone and with the fused projection, against autograd through the reference's op chain
-(oracle.head_projection) on the same GPU.
+and fresh noise, maskout alone and with the fused projection, without and with the gradients of the gates'
+temperatures (``grad_inv_tau``: one per-CTA partial per gate, then one reduction pass), against autograd through the
+reference's op chain (oracle.head_projection) on the same GPU.
 
     python tests/perf_head_backward.py
 
@@ -65,6 +66,7 @@ def time_per_call(fns, reps=5, calls=20):
 
 def gate(mode_fixed, per_pixel, noise):
     g = _lib.Gate()
+    g.hard, g.inv_tau, g.eps = 1, np.float32(1.0), np.float32(1e-10)
     if mode_fixed:
         g.mode, g.noise_a, g.noise_b, g.batch_stride = _lib.NOISE_LOGISTIC, noise[0].data_ptr(), None, 0
     else:
@@ -99,6 +101,8 @@ def main():
                      "gm": torch.randn(B, kind, H, W, device=dev, generator=gen),
                      "gp": torch.randn(B, H * W, 3, device=dev, generator=gen)}
                 s["out_d"], s["out_c"] = torch.empty_like(s["depth"]), torch.empty_like(s["conf"])
+                s["out_tau"] = torch.empty(kind, device=dev)
+                s["ws"] = _lib.workspace(lib.dusty_head_project_backward_workspace_bytes(B, H, W), dev)
                 if noise == "fresh":
                     s["np"] = [torch.rand(B, 1, H, W, device=dev, generator=gen) for _ in range(2)]
                     s["ni"] = [torch.rand(B, 1, 1, 1, device=dev, generator=gen) for _ in range(2)]
@@ -108,17 +112,19 @@ def main():
                 p.b, p.h, p.w, p.conf_channels, p.points_layout = B, H, W, kind, 1
                 p.gate_pixel = gate(noise == "fixed", True, s["np"])
                 p.gate_image = gate(noise == "fixed", False, s["ni"])
-                p.inv_tau, p.threshold, p.eps, p.drop_const = np.float32(1.0), np.float32(0.5), np.float32(1e-10), np.float32(-1.0)
+                p.threshold, p.drop_const = np.float32(0.5), np.float32(-1.0)
                 _projection_fields(p, lidar, 0.0)
                 s["p"] = p
                 sets.append(s)
             for proj in (False, True):
-                def launch(s=None, proj=proj):
+                def launch(s=None, proj=proj, tau=False):
                     _lib.check(lib.dusty_head_project_backward(
                         C.byref(s["p"]), _lib.ptr(s["depth"]), _lib.ptr(s["conf"]), _lib.ptr(trig), _lib.ptr(s["gm"]),
                         _lib.ptr(s["gd"]), _lib.ptr(s["gp"] if proj else None), _lib.ptr(s["out_d"]),
-                        _lib.ptr(s["out_c"]), None, None, 0, _lib.stream_of(s["depth"])), "dusty_head_project_backward")
+                        _lib.ptr(s["out_c"]), _lib.ptr(s["out_tau"] if tau else None), _lib.ptr(s["ws"] if tau else None),
+                        s["ws"].numel() if tau else 0, _lib.stream_of(s["depth"])), "dusty_head_project_backward")
                 t = time_per_call([lambda s=s: launch(s) for s in sets])
+                t_tau = time_per_call([lambda s=s: launch(s, tau=True) for s in sets])
                 nbytes = 4 + 4 * kind + 4 + 4 * kind + (12 if proj else 0) + (8 if noise == "fresh" else 0) + 4 + 4 * kind
                 gbs = nbytes * B * H * W / t / 1e9
                 # the same backward through autograd of the reference's op chain
@@ -137,7 +143,8 @@ def main():
                     grads.append(s["gp"])
                 t_ref = time_per_call([lambda: torch.autograd.backward(outs, grads, retain_graph=True)], reps=3, calls=5)
                 del outs, grads, mask, dout, d, c
-                row = {"dusty": kind, "noise": noise, "projection": proj, "us": round(t * 1e6, 1), "bytes_per_px": nbytes,
+                row = {"dusty": kind, "noise": noise, "projection": proj, "us": round(t * 1e6, 1),
+                       "us_with_grad_inv_tau": round(t_tau * 1e6, 1), "bytes_per_px": nbytes,
                        "GB_s": round(gbs), "frac_hbm_copy": round(gbs / peak, 3), "oracle_autograd_us": round(t_ref * 1e6, 1),
                        "speedup": round(t_ref / t, 1)}
                 rows.append(row)

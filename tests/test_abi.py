@@ -30,7 +30,7 @@ def test_library_exports_every_declared_symbol():
     assert exported == declared_symbols()
     assert sorted(_lib.SIGNATURES) == declared_symbols()
     lib = _lib.load()
-    assert lib.dusty_abi_version() == _lib.ABI_VERSION == 2
+    assert lib.dusty_abi_version() == _lib.ABI_VERSION == 3
     assert lib.dusty_launch_count() == 0 or lib.dusty_launch_count() > 0
 
 
@@ -122,6 +122,28 @@ def test_header_is_plain_c_and_a_c_program_links(tmp_path):
     subprocess.check_call(["gcc", "-std=c99", "-pedantic", "-Werror", "-fsyntax-only", "-x", "c",
                            os.path.join(ROOT, "include", "dusty_b200.h")])
     assert os.path.exists(_build_c_demo(tmp_path))
+
+
+def test_struct_layouts_match_the_ctypes_mirrors(tmp_path):
+    """Every Python call passes the parameter structs by pointer through the ctypes mirrors in _lib.py: their size and
+    each field's offset must be what a C compiler makes of include/dusty_b200.h."""
+    import ctypes
+    from dusty_gan_b200 import _lib
+    mirrors = {"dusty_gate": _lib.Gate, "dusty_head_params": _lib.HeadParams, "dusty_scan_params": _lib.ScanParams}
+    lines = ["#include <stddef.h>", "#include <stdio.h>", '#include "dusty_b200.h"', "int main(void) {"]
+    want = []
+    for cname, cls in mirrors.items():
+        lines.append(f'  printf("{cname} sizeof %zu\\n", sizeof({cname}));')
+        want.append(f"{cname} sizeof {ctypes.sizeof(cls)}")
+        for field, _ in cls._fields_:
+            lines.append(f'  printf("{cname}.{field} %zu\\n", offsetof({cname}, {field}));')
+            want.append(f"{cname}.{field} {getattr(cls, field).offset}")
+    lines += ["  return 0;", "}"]
+    src, exe = tmp_path / "layout.c", str(tmp_path / "layout")
+    src.write_text("\n".join(lines) + "\n")
+    subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), str(src),
+                           "-o", exe])
+    assert subprocess.check_output([exe], text=True).splitlines() == want
 
 
 def test_hot_kernels_keep_their_occupancy_shape():

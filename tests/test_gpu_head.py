@@ -1,10 +1,12 @@
 """Fused head + projection: bit-exact against the reference's op chain (oracle.head_projection) run
 on the same GPU, and against the golden CPU vectors up to ATen's CPU/CUDA last-ulp differences."""
+import math
+
 import numpy as np
 import pytest
 import torch
 
-from helpers import head_inputs
+from helpers import head_inputs, oracle_head_maskout, oracle_head_noise
 from oracle import head_projection as hp
 
 pytestmark = pytest.mark.gpu
@@ -66,6 +68,79 @@ def test_fixed_noise_bit_exact_on_device(kind, shape, compaction, monkeypatch):
         assert_bit_equal(fused["valid_points"][b, :k], pts[b][valid[b]], "compacted points")
 
 
+def _diverged_weights(head):
+    with torch.no_grad():
+        head.gumbel_pixel.weight.fill_(0.37)
+        head.gumbel_image.weight.fill_(-1.2)
+
+
+# name -> (kind, training, tau of the constructor, per-gate setup): each gate's own temperature, eps and hard flag
+GATE_CASES = {
+    "dusty1_learnable": (1, False, None, lambda h: h.gumbel.weight.data.fill_(0.37)),
+    "dusty1_soft": (1, False, 1.0, lambda h: setattr(h.gumbel, "hard", False)),
+    "dusty2_diverged_learnable": (2, True, None, _diverged_weights),
+    "dusty2_image_tau": (2, True, 0.7, lambda h: setattr(h.gumbel_image, "tau", 1.9)),
+    "dusty2_soft_pixel": (2, True, 1.0, lambda h: setattr(h.gumbel_pixel, "hard", False)),
+    "dusty2_soft_image": (2, True, 1.0, lambda h: setattr(h.gumbel_image, "hard", False)),
+    "dusty2_image_eps": (2, True, 1.0, lambda h: setattr(h.gumbel_image, "eps", 0.05)),
+}
+
+
+@pytest.mark.parametrize("noise", ["fixed", "fresh"])
+@pytest.mark.parametrize("threshold", [0.3, 0.5, 0.7, float("nan")])
+@pytest.mark.parametrize("case", list(GATE_CASES))
+def test_each_gate_keeps_its_own_settings_bit_exact_on_device(case, threshold, noise, monkeypatch):
+    """Every gate is computed with its own temperature (fixed or learnable), eps and ``hard`` flag, as the reference's
+    GumbelSigmoid modules are, and one threshold serves both gates. A NaN threshold is no sentinel: a hard gate then
+    gives the reference's exact zeros. Checked through maskout, the fused projection in both point layouts and both
+    compaction kernels (each has its own gate code). At threshold 0.5 the hard mask does not depend on the
+    temperature; 0.3 and 0.7 are where a wrong temperature flips mask values."""
+    from dusty_gan_b200 import pipeline
+    from dusty_gan_b200.models.dusty import DUSty1, DUSty2, _head_call
+    kind, training, tau, setup = GATE_CASES[case]
+    B, H, W = 3, 40, 100                          # 4000 pixels: a partial last segment and a partial last image step
+    depth, conf, _, _ = head_inputs(B, kind, H, W, 60 + kind, "cuda")
+    head = (DUSty1 if kind == 1 else DUSty2)(torch.nn.Identity(), tau=tau).cuda().train(training)
+    setup(head)
+    if noise == "fixed":
+        g = torch.Generator().manual_seed(61)
+        for gate, shape in ([(head.gumbel, (1, 1, H, W))] if kind == 1 else
+                            [(head.gumbel_pixel, (1, 1, H, W)), (head.gumbel_image, (1, 1, 1, 1))]):
+            gate.fixed_noise = hp.logistic_noise(torch.rand(shape, generator=g).cuda(), torch.rand(shape, generator=g).cuda(),
+                                                 gate.eps)
+    seed = 62
+    mask, dout, _ = oracle_head_maskout(head, depth, conf, *oracle_head_noise(head, B, H, W, seed), threshold)
+    lidar = make_lidar(H, W)
+    pts = hp.project_2d_to_3d_dense(dout, lidar.angle, 0.9, 120.0, 0.0)
+    planar = hp.inv_to_xyz(hp.tanh_to_sigmoid_clamped(dout), lidar.angle, 0.9, 120.0, 0.0)
+    valid = hp.tanh_to_sigmoid_clamped(dout).flatten(1) != 0
+    pixel_gate = head.gumbel if kind == 1 else head.gumbel_pixel
+    if math.isnan(threshold) and pixel_gate.hard:
+        assert bool((mask[:, 0] == 0).all())      # soft > nan is false: every hard pixel mask is 0
+    for path in ("maskout", "points", "planar", "segment", "image"):
+        inputs = {"depth": depth.clone(), "confidence": conf.clone()}
+        torch.manual_seed(seed)                   # fresh noise: the draws the oracle replayed
+        if path == "maskout":
+            out = head.maskout(inputs, threshold=threshold)
+        elif path == "points":
+            out = pipeline.maskout_and_project(head, inputs, lidar, tol=0.0, threshold=threshold)
+            assert_bit_equal(out["points"], pts, f"{path}: points")
+        elif path == "planar":
+            out, points, _, _, _ = _head_call(head, inputs, threshold, lidar=lidar, tol=0.0, points_layout=0)
+            assert_bit_equal(points, planar, f"{path}: points")
+        else:
+            monkeypatch.setenv("DUSTY_HEAD_COMPACT", path)
+            out = pipeline.maskout_and_project(head, inputs, lidar, tol=0.0, threshold=threshold, compact=True)
+            assert_bit_equal(out["points"], pts, f"{path}: points")
+            assert torch.equal(out["valid_count"].long(), valid.sum(1)), path
+            for b in range(B):
+                k = int(valid[b].sum())
+                assert torch.equal(out["valid_index"][b, :k].long(), torch.nonzero(valid[b]).flatten()), path
+                assert_bit_equal(out["valid_points"][b, :k], pts[b][valid[b]], f"{path}: compacted points")
+        assert_bit_equal(out["mask"], mask, f"{path}: mask")
+        assert_bit_equal(out["depth"], dout, f"{path}: depth")
+
+
 def test_fresh_noise_uses_the_reference_rng_draws():
     from dusty_gan_b200.models.dusty import DUSty2
     depth, conf, _, _ = head_inputs(4, 2, 16, 64, 5, "cuda")
@@ -86,9 +161,10 @@ def test_gumbel_sigmoid_module_thresholds_and_grad():
     logits = torch.randn(3, 1, 16, 64, device="cuda", requires_grad=True)
     noise = g.logistic_noise(logits)[[0]]
     g.fixed_noise = noise
-    for thr in (0.5, 0.3, 0.9):
+    for thr in (0.5, 0.3, 0.9, float("nan")):        # NaN: soft > nan is false, so the hard gate gives exact zeros
         out = g(logits, thr)
         assert_bit_equal(out.detach(), hp.gumbel_sigmoid(logits.detach(), noise, 0.7, thr), f"thr={thr}")
+    assert bool((out == 0).all())
     out = g(logits)
     out.sum().backward()
     ref_logits = logits.detach().clone().requires_grad_(True)

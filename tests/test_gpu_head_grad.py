@@ -1,24 +1,27 @@
 """Backward of the fused head (dusty_head_project_backward) against autograd through the reference's op chain
-(oracle.head_projection) on the same GPU: DUSty-I / DUSty-II, fixed and fresh noise, the soft gate, the learnable
-temperature, the fused projection in both point layouts, exact zeros, the inversion loss end to end, determinism
-and the refused cases."""
-import math
-
+(oracle.head_projection) on the same GPU: DUSty-I / DUSty-II, fixed and fresh noise, soft gates, each gate's own
+learnable temperature, the fused projection in both point layouts, exact zeros, the inversion loss end to end, a
+DUSty-II generator step on its two temperatures, determinism and the refused cases."""
 import pytest
 import torch
 
-from helpers import head_inputs, sampled_clouds
+from helpers import head_inputs, oracle_head_maskout, oracle_head_noise, sampled_clouds
 from oracle import head_projection as hp
 
 pytestmark = pytest.mark.gpu
 
 MIN_DEPTH, MAX_DEPTH = 0.9, 120.0
 SHAPES = [(5, 64, 512), (3, 16, 64), (2, 8, 20), (130, 64, 512)]
-# (channels, training, noise, variant): variant "soft" is GumbelSigmoid(hard=False) (a NaN threshold), "learnable"
-# is tau=None with the temperature weight at 0.37
+# (channels, training, noise, variant): variant "soft" makes the pixel gate (DUSty-I's only gate) GumbelSigmoid(hard=False)
+# and "soft_image" DUSty-II's image gate; "learnable" is tau=None with the pixel gate's weight at 0.37, "diverged" is
+# tau=None with the pixel gate's weight at 0.37 and the image gate's at -1.2 (what training makes of them), run at
+# threshold 0.3, where the temperatures also decide mask values
 CASES = [(1, False, "fixed", None), (1, False, "fresh", None), (2, False, "fixed", None), (2, False, "fresh", None),
          (2, True, "fixed", None), (2, True, "fresh", None), (1, False, "fixed", "soft"),
-         (1, False, "fixed", "learnable"), (1, True, "fresh", "learnable"), (2, False, "fixed", "learnable")]
+         (1, False, "fixed", "learnable"), (1, True, "fresh", "learnable"), (2, False, "fixed", "learnable"),
+         (2, True, "fixed", "diverged"), (2, True, "fresh", "diverged"), (2, True, "fixed", "soft"),
+         (2, True, "fresh", "soft_image")]
+PROJ_CASES = [CASES[0], CASES[3], CASES[5], CASES[6], CASES[7], CASES[10], CASES[11], CASES[13]]
 
 
 def make_lidar(H, W):
@@ -47,12 +50,19 @@ def assert_close(a, b, rtol, atol, what):
 def make_head(kind, training, noise, variant, H, W, seed):
     """The head under test and, for fixed noise, its noise maps."""
     from dusty_gan_b200.models.dusty import DUSty1, DUSty2
-    head = (DUSty1 if kind == 1 else DUSty2)(torch.nn.Identity(), tau=None if variant == "learnable" else 1.0).cuda()
+    learnable = variant in ("learnable", "diverged")
+    head = (DUSty1 if kind == 1 else DUSty2)(torch.nn.Identity(), tau=None if learnable else 1.0).cuda()
     head.train(training)
     gate = head.gumbel if kind == 1 else head.gumbel_pixel
-    if variant == "learnable":
-        with torch.no_grad():
+    with torch.no_grad():
+        if learnable:
             gate.weight.fill_(0.37)
+        if variant == "diverged":
+            head.gumbel_image.weight.fill_(-1.2)
+    if variant == "soft":
+        gate.hard = False
+    if variant == "soft_image":
+        head.gumbel_image.hard = False
     if noise == "fixed":
         g = torch.Generator().manual_seed(seed)
         u = [torch.rand(1, 1, H, W, generator=g).cuda() for _ in range(2)]
@@ -63,70 +73,37 @@ def make_head(kind, training, noise, variant, H, W, seed):
     return head, gate
 
 
-def oracle_noise(head, kind, training, noise, B, H, W, rng_seed):
-    """The logistic noise the head read: its fixed maps, or the reference's RNG draws replayed."""
-    if noise == "fixed":
-        gate = head.gumbel if kind == 1 else head.gumbel_pixel
-        return gate.fixed_noise, (head.gumbel_image.fixed_noise if kind == 2 and training else None)
-    torch.manual_seed(rng_seed)
-    u1 = torch.rand(B, 1, H, W, device="cuda"); u2 = torch.rand_like(u1)
-    noise_image = None
-    if kind == 2 and training:
-        v1 = torch.rand(B, 1, 1, 1, device="cuda"); v2 = torch.rand_like(v1)
-        noise_image = hp.logistic_noise(v1, v2)
-    return hp.logistic_noise(u1, u2), noise_image
-
-
-def oracle_gate(logits, noise, threshold, it):
-    """hp.gumbel_sigmoid, with the learnable temperature multiplied in as the reference does (models/dusty.py:39-41)
-    and the soft output of hard=False (:58-59)."""
-    if it is None and not math.isnan(threshold):
-        return hp.gumbel_sigmoid(logits, noise, 1.0, threshold)
-    x = logits + (noise.expand(logits.shape[0], -1, -1, -1) if noise.shape[0] == 1 else noise)
-    soft = torch.sigmoid(x * it) if it is not None else torch.sigmoid(x / 1.0)
-    if math.isnan(threshold):
-        return soft
-    return (soft > threshold).float() - soft.detach() + soft
-
-
-def oracle_maskout(kind, depth, conf, noise_pixel, noise_image, threshold, it):
-    if it is None and not math.isnan(threshold):
-        if kind == 1:
-            return hp.maskout_dusty1(depth, conf, noise_pixel, threshold=threshold)
-        return hp.maskout_dusty2(depth, conf, noise_pixel, threshold=threshold, noise_image=noise_image)
-    dc = torch.tensor(-1.0).float().to(depth.device)
-    if kind == 1:
-        mask = oracle_gate(conf, noise_pixel, threshold, it)
-        return mask, mask * depth + (1 - mask) * dc
-    mask_pixel = oracle_gate(conf[:, [0]], noise_pixel, threshold, it)
-    mask_image = (conf[:, [1]] > 0.0).float() if noise_image is None else oracle_gate(conf[:, [1]], noise_image, threshold, it)
-    mask = mask_pixel * mask_image
-    return torch.cat([mask_pixel, mask_image], dim=1), mask * depth + (1 - mask) * dc
-
-
 def run_both(kind, training, noise, variant, shape, seed, lib_fn, oracle_fn, loss_fn):
     """Run the library arm (``lib_fn(head, depth, conf) -> outputs``) and the oracle arm (``oracle_fn(mask, dout)``
-    on the oracle's maskout), back-propagate ``loss_fn(outputs)`` through both and return the pairs of results."""
+    on the oracle's maskout), back-propagate ``loss_fn(outputs)`` through both and return the pairs of results: the
+    outputs, then (depth, confidence, (pixel weight grad, image weight grad)) of each arm, a weight grad being None
+    where the oracle has no learnable temperature for that gate."""
     B, H, W = shape
     depth, conf, _, _ = head_inputs(B, kind, H, W, seed, "cuda")
     head, gate = make_head(kind, training, noise, variant, H, W, seed + 1)
-    threshold = float("nan") if variant == "soft" else 0.5
+    threshold = 0.3 if variant == "diverged" else 0.5
     d = depth.clone().requires_grad_(True)
     c = conf.clone().requires_grad_(True)
     torch.manual_seed(seed + 2)
     out = lib_fn(head, d, c, threshold)
     loss_fn(out).backward()
-    noise_pixel, noise_image = oracle_noise(head, kind, training, noise, B, H, W, seed + 2)
+    noise_pixel, noise_image = oracle_head_noise(head, B, H, W, None if noise == "fixed" else seed + 2)
     dr = depth.clone().requires_grad_(True)
     cr = conf.clone().requires_grad_(True)
-    wr = it = None
-    if variant == "learnable":
-        wr = gate.weight.detach().clone().requires_grad_(True)
-        it = torch.nn.functional.softplus(wr) + 1.0 / gate.tau_max
-    mask, dout = oracle_maskout(kind, dr, cr, noise_pixel, noise_image, threshold, it)
+    mask, dout, leaves = oracle_head_maskout(head, dr, cr, noise_pixel, noise_image, threshold)
     ref = oracle_fn(mask, dout)
     loss_fn(ref).backward()
-    return out, ref, (d, c, gate.weight.grad if variant == "learnable" else None), (dr, cr, wr.grad if wr is not None else None)
+    gates = (gate, head.gumbel_image if kind == 2 else None)
+    lib_w = tuple(None if w is None else g.weight.grad for g, w in zip(gates, leaves))
+    return out, ref, (d, c, lib_w), (dr, cr, tuple(None if w is None else w.grad for w in leaves))
+
+
+def assert_weight_grads(gw, gwr):
+    """Each learnable temperature's weight.grad, pixel gate and image gate separately."""
+    for what, a, b in zip(("pixel", "image"), gw, gwr):
+        if b is not None:
+            assert a is not None, what
+            assert_close(a, b, 1e-4, 1e-6, f"{what} gate temperature weight.grad")
 
 
 @pytest.mark.parametrize("shape", SHAPES)
@@ -150,13 +127,15 @@ def test_maskout_gradients_match_autograd_through_the_reference(kind, training, 
     assert_close(c.grad, cr.grad, 1e-5, 1e-7, "confidence.grad")
     if kind == 2 and not training:
         assert bool((c.grad[:, 1] == 0).all())                  # the eval-mode image gate is (logit > 0)
-    if variant == "learnable":
-        assert gw is not None and gwr is not None
-        assert_close(gw, gwr, 1e-4, 1e-6, "temperature weight.grad")
+    if variant in ("learnable", "diverged"):
+        assert gw[0] is not None and gwr[0] is not None
+    if variant == "diverged":
+        assert gw[1] is not None and gwr[1] is not None
+    assert_weight_grads(gw, gwr)
 
 
 @pytest.mark.parametrize("shape", SHAPES[:3])
-@pytest.mark.parametrize("kind,training,noise,variant", [CASES[0], CASES[3], CASES[5], CASES[6], CASES[7]])
+@pytest.mark.parametrize("kind,training,noise,variant", PROJ_CASES)
 @pytest.mark.parametrize("with_depth", [False, True])
 def test_fused_projection_gradients_match_autograd_through_the_reference(kind, training, noise, variant, shape,
                                                                          with_depth):
@@ -182,8 +161,7 @@ def test_fused_projection_gradients_match_autograd_through_the_reference(kind, t
     assert_bit_equal(out[1].detach(), ref[1].detach(), "points")
     assert_close(d.grad, dr.grad, 1e-4, 1e-6, "depth.grad")
     assert_close(c.grad, cr.grad, 1e-4, 1e-6, "confidence.grad")
-    if variant == "learnable":
-        assert_close(gw, gwr, 1e-4, 1e-6, "temperature weight.grad")
+    assert_weight_grads(gw, gwr)
 
 
 @pytest.mark.parametrize("kind", [1, 2])
@@ -295,24 +273,67 @@ def test_inversion_loss_end_to_end():
 
 
 def test_backward_is_deterministic():
-    """The temperature's gradient is a fixed-order reduction (per-CTA partials, one final pass): two backward passes
-    on the same inputs give bit-identical gradients."""
+    """Each temperature's gradient is a fixed-order reduction (per-CTA partials per gate, one final pass): two
+    backward passes on the same inputs give bit-identical gradients, DUSty-I and DUSty-II in training with both
+    temperatures learnable."""
     from dusty_gan_b200 import pipeline
     B, H, W = 8, 64, 512
     lidar = make_lidar(H, W)
-    head, gate = make_head(1, False, "fixed", "learnable", H, W, 5)
-    depth, conf, _, _ = head_inputs(B, 1, H, W, 6, "cuda")
-    w1, w3 = [torch.randn(s, generator=torch.Generator().manual_seed(8 + i)).cuda()
-              for i, s in enumerate([(B, 1, H, W), (B, H * W, 3)])]
-    grads = []
-    for _ in range(2):
-        gate.weight.grad = None
-        d, c = depth.clone().requires_grad_(True), conf.clone().requires_grad_(True)
-        out = pipeline.maskout_and_project(head, {"depth": d, "confidence": c}, lidar, differentiable=True)
-        ((w3 * out["points"]).sum() + (w1 * out["depth"]).sum()).backward()
-        grads.append((d.grad, c.grad, gate.weight.grad.clone()))
-    for a, b, what in zip(*grads, ("depth", "confidence", "weight")):
-        assert_bit_equal(a, b, what)
+    for kind, training, variant in ((1, False, "learnable"), (2, True, "diverged")):
+        head, _ = make_head(kind, training, "fixed", variant, H, W, 5)
+        weights = [p for p in head.parameters()]
+        assert len(weights) == kind
+        depth, conf, _, _ = head_inputs(B, kind, H, W, 6, "cuda")
+        w1, w3 = [torch.randn(s, generator=torch.Generator().manual_seed(8 + i)).cuda()
+                  for i, s in enumerate([(B, 1, H, W), (B, H * W, 3)])]
+        grads = []
+        for _ in range(2):
+            for w in weights:
+                w.grad = None
+            d, c = depth.clone().requires_grad_(True), conf.clone().requires_grad_(True)
+            out = pipeline.maskout_and_project(head, {"depth": d, "confidence": c}, lidar, threshold=0.3,
+                                               differentiable=True)
+            ((w3 * out["points"]).sum() + (w1 * out["depth"]).sum()).backward()
+            grads.append((d.grad, c.grad, *(w.grad.clone() for w in weights)))
+        for a, b, what in zip(*grads, ("depth", "confidence", "weight", "image weight")):
+            assert_bit_equal(a, b, f"DUSty-{'I' * kind}: {what}")
+
+
+def test_dusty2_generator_step_trains_each_temperature():
+    """A generator step of DUSty-II in training mode with tau=None: three SGD steps on the two gates' temperature
+    weights, with the same seeded noise in the library arm and in the oracle arm. Both start at 0; their gradients
+    differ, so they part after the first step, and the two arms move them alike."""
+    from dusty_gan_b200.models.dusty import DUSty2
+    B, H, W = 4, 32, 256
+    depth, conf, _, _ = head_inputs(B, 2, H, W, 71, "cuda")
+    w1, w2 = [torch.randn(s, generator=torch.Generator().manual_seed(72 + i)).cuda()
+              for i, s in enumerate([(B, 1, H, W), (B, 2, H, W)])]
+
+    def loss(mask, dout):
+        return (w1 * dout).mean() + (w2 * mask).mean()
+
+    head = DUSty2(torch.nn.Identity(), tau=None).cuda().train()
+    weights = [head.gumbel_pixel.weight, head.gumbel_image.weight]
+    ref = [w.detach().clone().requires_grad_(True) for w in weights]
+    opt, opt_ref = torch.optim.SGD(weights, lr=1.0), torch.optim.SGD(ref, lr=1.0)
+    for step in range(3):
+        seed = 73 + step
+        torch.manual_seed(seed)
+        out = head.maskout({"depth": depth.clone().requires_grad_(True), "confidence": conf.clone().requires_grad_(True)})
+        opt.zero_grad()
+        loss(out["mask"], out["depth"]).backward()
+        opt.step()
+        noise_pixel, noise_image = oracle_head_noise(head, B, H, W, seed)
+        it = [torch.nn.functional.softplus(w) + 1.0 / head.gumbel_pixel.tau_max for w in ref]
+        mask, dout = hp.maskout_dusty2(depth.clone().requires_grad_(True), conf.clone().requires_grad_(True), noise_pixel,
+                                       it[0], noise_image=noise_image, tau_image=it[1])
+        opt_ref.zero_grad()
+        loss(mask, dout).backward()
+        opt_ref.step()
+        for what, w, r in zip(("pixel", "image"), weights, ref):
+            assert_close(w.detach(), r.detach(), 1e-5, 1e-7, f"step {step}: {what} gate temperature weight")
+        if step == 0:
+            assert weights[0].item() != weights[1].item()
 
 
 @pytest.mark.parametrize("kind", [1, 2])
@@ -339,7 +360,7 @@ def test_forward_under_grad_is_the_no_grad_forward(kind):
 
 def test_refused_cases():
     from dusty_gan_b200 import pipeline
-    from dusty_gan_b200.models.dusty import DUSty1, DUSty2
+    from dusty_gan_b200.models.dusty import DUSty1
     B, H, W = 2, 8, 20
     lidar = make_lidar(H, W)
     depth, conf, _, _ = head_inputs(B, 2, H, W, 12, "cuda")
@@ -347,12 +368,6 @@ def test_refused_cases():
     d, c = depth.clone().requires_grad_(True), conf[:, :1].clone().requires_grad_(True)
     with pytest.raises(ValueError, match="compact"):
         pipeline.maskout_and_project(head1, {"depth": d, "confidence": c}, lidar, compact=True, differentiable=True)
-    head2 = DUSty2(torch.nn.Identity(), tau=None).cuda().train()
-    c2 = conf.clone().requires_grad_(True)
-    with pytest.raises(NotImplementedError, match="tau=None"):
-        head2.maskout({"depth": d, "confidence": c2})
-    with torch.no_grad():                                          # the forward alone still runs
-        head2.maskout({"depth": d, "confidence": c2})
     cpu = DUSty1(torch.nn.Identity(), tau=1.0)
     with pytest.raises(RuntimeError, match="CUDA tensor"):
         cpu.maskout({"depth": torch.zeros(1, 1, 8, 8, requires_grad=True),

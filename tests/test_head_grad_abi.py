@@ -35,7 +35,7 @@ def error():
 def test_workspace_query_without_a_gpu():
     from dusty_gan_b200 import _lib
     lib = _lib.load()
-    assert lib.dusty_head_project_backward_workspace_bytes(256, 64, 512) == 256 * 32 * 4      # one float per CTA
+    assert lib.dusty_head_project_backward_workspace_bytes(256, 64, 512) == 2 * 256 * 32 * 4  # one float per gate and CTA
     assert lib.dusty_head_project_backward_workspace_bytes(3, 8, 20) == 256                    # rounded up to 256 B
     assert lib.dusty_head_project_backward_workspace_bytes(0, 64, 512) == 0
     assert lib.dusty_head_project_backward_workspace_bytes(2, 0, 512) == 0
@@ -53,6 +53,7 @@ def test_workspace_query_without_a_gpu():
     ("misaligned grad_mask", DUSTY_EALIGN, "16-byte aligned"),
     ("misaligned grad_points", DUSTY_EALIGN, "16-byte aligned"),
     ("gate without noise pointer", DUSTY_EINVAL, "needs noise_a"),
+    ("gate hard flag not 0 or 1", DUSTY_EINVAL, "hard must be 0 or 1"),
     ("grad_inv_tau without workspace", DUSTY_ENOSPACE, "workspace bytes"),
 ])
 def test_argument_errors_are_reported_without_a_gpu(case, code, message):
@@ -80,6 +81,8 @@ def test_argument_errors_are_reported_without_a_gpu(case, code, message):
         kw.update(grad_points=0x7000c, trig=0x90000)
     elif case == "gate without noise pointer":
         p.gate_pixel.noise_a = None
+    elif case == "gate hard flag not 0 or 1":
+        p.gate_pixel.hard = 2
     elif case == "grad_inv_tau without workspace":
         kw["grad_tau"] = 0xa0000
     assert backward(p, **kw) == code, case
