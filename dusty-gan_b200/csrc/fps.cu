@@ -572,7 +572,7 @@ static_assert(MT_SMEM_BYTES >= CELLS * 4, "the cell counters alias the box/recor
 
 struct MtRec { float maxT; int e; float x, y, z; float pad0, pad1, pad2; };   // 32 B
 struct MtWin { unsigned val; int e; float x, y, z; };
-// CHIP variant: the running distances of the first MT_DCAP eligible points live in shared memory (64 KB), three
+// CHIP variant: the running distances of the first MT_DCAP eligible points live in shared memory (56 KB), three
 // clouds per SM. Only the read-only coordinates of a touched bucket then travel from L2, and the clouds in flight
 // (444 x 15.6 k points x 12 B = 83 MB) fit the 126 MB L2: the six-clouds-per-SM layout keeps 277 MB of coordinates,
 // distances and indices in flight and pays 13 GB of DRAM traffic per 888 clouds for it (profiles/SUMMARY_r1.md).
