@@ -82,6 +82,12 @@ SIGNATURES = {
     "dusty_jsd_vote":(C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_int, c_float_p, c_int_p, c_float_p, C.c_float,
                                  C.c_void_p, C.c_void_p, C.c_void_p]),
     "dusty_jsd_from_counts": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, c_float_p, C.c_void_p]),
+    "dusty_swd_descriptors_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "dusty_swd_descriptors": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_int_p, C.c_int,
+                                        c_float_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dusty_swd_sliced_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "dusty_swd_sliced": (C.c_int, [c_float_p, c_float_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, c_float_p, C.c_int,
+                                   C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "dusty_fps_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "dusty_fps": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, c_int_p, c_float_p, C.c_void_p, C.c_size_t,
                             C.c_void_p]),

@@ -1,6 +1,6 @@
 """The flow of the reference's evaluate_synthesis.py (:20-195) on the B200 kernels, with synthetic stand-ins
 for what this container lacks (KITTI scans, a trained checkpoint): raw scans -> real cache -> generated
-range images -> clouds -> JSD + MMD / COV / 1-NNA, printed as the reference's score dict.
+range images -> clouds -> SWD + JSD + MMD / COV / 1-NNA, printed as the reference's score dict.
 
     python examples/evaluate_synthesis.py --num-test 200 --num-points 2048 [--dusty 2] [--tol 0.0]
 
@@ -9,9 +9,9 @@ Every stage is one call of this package where the reference script calls its own
     [skip:limit:skip] subsampling (:102-110)         pipeline.subsample_time_series
     G(latent) -> maskout (:157-158)                  a stand-in backbone + DUSty1/DUSty2.maskout fused with
     project_2d_to_3d (:59-64)                        pipeline.generate_points
+    compute_swd (:169-173)                           utils.metrics.swd.compute_swd
     compute_jsd (:174-177)                           utils.metrics.jsd.compute_jsd
     compute_cov_mmd_1nna (:178-183)                  utils.metrics.cov_mmd_1nna.compute_cov_mmd_1nna
-(SWD, :169-173, is a 2-D image metric outside the path.)
 """
 import argparse
 import json
@@ -28,6 +28,7 @@ from dusty_gan_b200.models.dusty import DUSty1, DUSty2  # noqa: E402
 from dusty_gan_b200.utils.lidar import LiDAR, synthetic_hdl64e_angles  # noqa: E402
 from dusty_gan_b200.utils.metrics.cov_mmd_1nna import compute_cov_mmd_1nna  # noqa: E402
 from dusty_gan_b200.utils.metrics.jsd import compute_jsd  # noqa: E402
+from dusty_gan_b200.utils.metrics.swd import compute_swd  # noqa: E402
 
 H, W = 64, 512
 
@@ -103,7 +104,8 @@ def main():
     fakes = {k: torch.cat(v, dim=0)[:N_test] for k, v in fakes.items()}
     torch.cuda.synchronize(); t2 = time.perf_counter()
 
-    scores = {"jsd": compute_jsd(pcs_gen=fakes["3d"] / 2.0, pcs_ref=reals["3d"] / 2.0)}
+    scores = {"swd": float(compute_swd(fakes["2d"], reals["2d"]))}
+    scores["jsd"] = compute_jsd(pcs_gen=fakes["3d"] / 2.0, pcs_ref=reals["3d"] / 2.0)
     scores.update(compute_cov_mmd_1nna(pcs_gen=fakes["3d"], pcs_ref=reals["3d"], batch_size=512, metrics=metrics))
     torch.cuda.synchronize(); t3 = time.perf_counter()
     scores["#test"] = args.num_test

@@ -30,6 +30,9 @@
  *                                compute_cov_mmd_1nna, with the fused minima of dusty_chamfer_matrix_fused
  *   dusty_jsd_vote, dusty_jsd_from_counts   utils/metrics/jsd.py:23-92, 110-121 (entropy_of_occupancy_grid,
  *                                _jensen_shannon_divergence)
+ *   dusty_swd_descriptors, dusty_swd_sliced   utils/metrics/swd.py (compute_swd, called evaluate_synthesis.py:169-173):
+ *                                Laplacian pyramid, 7x7 patches, random projections, sort (SURVEY.md S2; the contract
+ *                                is the swd-pytorch algorithm, DESIGN.md S2.7)
  *   dusty_fps                    utils/sampling/fps/furthest_point_sampling.cpp:79-100
  *                                -> furthest_point_sampling_kernel_wrapper, furthest_point_sampling.cu:209-260
  *   dusty_gather_points          utils/sampling/fps/furthest_point_sampling.cpp:27-50
@@ -255,6 +258,44 @@ DUSTY_API int dusty_jsd_vote(const float* pcs, int b, int npts, int resolution, 
 /* _jensen_shannon_divergence of two count vectors (jsd.py:110-121), base-2 entropies; out[0] f32. */
 DUSTY_API int dusty_jsd_from_counts(const uint32_t* counts_p, const uint32_t* counts_q, int ng, float* out,
                                     void* stream);
+
+/* --------------------------------------------------------------------------------------------
+ * Sliced Wasserstein distance between range-image sets (reference utils/metrics/swd.py)
+ * -------------------------------------------------------------------------------------------- */
+
+/* Scratch for dusty_swd_descriptors: the Gaussian levels 1..levels-1 and per-image statistics. */
+DUSTY_API size_t dusty_swd_descriptors_workspace_bytes(int n, int c, int h, int w, int levels, int n_desc);
+
+/* Patch descriptors of one image set at every level of its Laplacian pyramid, and their per-channel statistics.
+ *   images (n,c,h,w) f32 contiguous, 1 <= c <= 4; h and w divisible by 2^(levels-1), every level at least 7x7.
+ *   Level l is (h_l, w_l) = (h >> l, w >> l); G(0) = images, G(l+1) = conv2d(G(l), k, padding 2, stride 2) with k the
+ *   5x5 binomial [1,4,6,4,1]^T [1,4,6,4,1] / 256 per channel; Lap(l) = G(l) - conv2d(nearest_up2(G(l+1)), k, padding
+ *   2) for l < levels-1 and Lap(levels-1) = G(levels-1).
+ *   positions (levels, n_desc) i32, device: position p of level l is the 7x7 patch with top-left corner
+ *   (p / (w_l-6), p % (w_l-6)), 0 <= p < (h_l-6)(w_l-6); the same positions serve every image. They are read back
+ *   and checked on the host before any kernel runs (the call synchronises the stream once).
+ *   desc: level l at desc + l*n*n_desc*c*49, (n*n_desc, c*49) f32, rows (image, descriptor), components
+ *   (channel, ky, kx).
+ *   stats (levels, c, 2) f64: mean and unbiased standard deviation of each channel's components over all rows of the
+ *   level, combined over the images in a fixed order (bit-identical from call to call). */
+DUSTY_API int dusty_swd_descriptors(const float* images, int n, int c, int h, int w, int levels,
+                                    const int32_t* positions, int n_desc, float* desc, double* stats,
+                                    void* workspace, size_t workspace_bytes, void* stream);
+
+/* Scratch for dusty_swd_sliced: the sort keys of a batch of directions (at most 4 GiB). */
+DUSTY_API size_t dusty_swd_sliced_workspace_bytes(int rows, int c, int n_dirs);
+
+/* Sliced W1 sums of one level between two descriptor sets of `rows` rows each (1 <= rows <= 2^30):
+ *   every row is normalised as x = (x - mean) / (std + 1e-8) per channel in f32 (stats1 / stats2: (c, 2) f64 of
+ *   dusty_swd_descriptors), projected onto direction d (column d of dirs (c*49, n_dirs) f32, one fixed FMA order), both
+ *   projections are sorted ascending and
+ *     sums[d] = sum_i |a_(i) - b_(i)|       (f64; a NaN key gives NaN)
+ *   for d = dir_begin, dir_begin + dir_stride, ... < dir_end (the multi-GPU deal); other entries of sums (n_dirs) are
+ *   not touched. Each sum is reduced in a fixed order: it is bit-identical from call to call and does not depend on
+ *   the direction range of the call. */
+DUSTY_API int dusty_swd_sliced(const float* desc1, const float* desc2, const double* stats1, const double* stats2,
+                               int rows, int c, const float* dirs, int n_dirs, int dir_begin, int dir_end,
+                               int dir_stride, double* sums, void* workspace, size_t workspace_bytes, void* stream);
 
 /* --------------------------------------------------------------------------------------------
  * Farthest-point sampling
