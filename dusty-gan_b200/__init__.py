@@ -9,9 +9,11 @@ The package mirrors the reference's module paths for that path and nothing else:
     utils.metrics.distance       chamfer_distance, ChamferDistance, earth_mover_distance
     utils.metrics.cov_mmd_1nna   compute_cd, compute_emd, emd_matrix, _pairwise_distance, compute_cov_mmd_1nna
     utils.metrics.jsd            compute_jsd                              (reference utils/metrics/jsd.py)
+    utils.metrics.depth          compute_depth_metrics                    (reference utils/metrics/depth.py)
     datasets                     define_dataset, KITTIOdometry, preprocess_scans (reference datasets/kitti.py)
     pipeline                     fused generate->points entry (project_2d_to_3d of evaluate_synthesis.py:59-64),
-                                 preprocess_reals / build_real_cache (evaluate_synthesis.py:49-57, 69-110)
+                                 preprocess_reals / build_real_cache (evaluate_synthesis.py:49-57, 69-110),
+                                 reconstruction_scores (evaluate_reconstruction.py:124-131)
     sharding                     row-sharded Chamfer matrix over torch.distributed
 
 All compute goes through ``libdustyb200.so`` (C ABI in include/dusty_b200.h); there is no CPU or

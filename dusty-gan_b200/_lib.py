@@ -88,6 +88,9 @@ SIGNATURES = {
     "dusty_swd_sliced_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "dusty_swd_sliced": (C.c_int, [c_float_p, c_float_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, c_float_p, C.c_int,
                                    C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dusty_depth_metrics_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "dusty_depth_metrics": (C.c_int, [C.POINTER(HeadParams), c_float_p, c_float_p, C.c_void_p, c_float_p, c_float_p,
+                                      C.c_void_p, C.c_size_t, C.c_void_p]),
     "dusty_fps_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "dusty_fps": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, c_int_p, c_float_p, C.c_void_p, C.c_size_t,
                             C.c_void_p]),

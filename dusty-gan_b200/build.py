@@ -16,7 +16,8 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libdustyb200.so")
-SOURCES = ["api.cu", "chamfer.cu", "fps.cu", "head_project.cu", "metrics.cu", "jsd.cu", "scan_preprocess.cu", "emd.cu", "swd.cu"]
+SOURCES = ["api.cu", "chamfer.cu", "fps.cu", "head_project.cu", "metrics.cu", "jsd.cu", "scan_preprocess.cu", "emd.cu", "swd.cu",
+           "depth_metrics.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden",

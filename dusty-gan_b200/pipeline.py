@@ -70,6 +70,21 @@ def build_real_cache(scan_batches, lidar, num_points, drop_const=-1, device="cud
     return {"2d": torch.cat(two_d, dim=0), "3d": torch.cat(three_d, dim=0)}
 
 
+@torch.no_grad()
+def reconstruction_scores(head, output, real_inv, real_points, lidar, tol=0.0):
+    """The per-batch scores of evaluate_reconstruction.py:124-131 for a generator's reconstructions of real scans:
+    ``output`` is the backbone's dict for the inverted latents, ``real_inv`` (B,1,H,W) the scans' tanh-space inverse
+    depth and ``real_points`` (B,H*W,3) their un-sampled clouds (``preprocess_reals``). Returns the depth metrics of
+    ``maskout``'s depth against ``real_inv`` (``compute_depth_metrics``, reduction "mean") plus ``"cd"``, the mean
+    ``compute_cd(real_points, generated points)`` over the batch on the un-sampled generated clouds."""
+    from .utils.metrics.cov_mmd_1nna import compute_cd
+    from .utils.metrics.depth import compute_depth_metrics
+    out = maskout_and_project(head, output, lidar, tol=tol)
+    scores = compute_depth_metrics(out["depth"], real_inv, lidar, tol=tol)
+    scores["cd"] = float(compute_cd(real_points, out["points"]).mean())
+    return scores
+
+
 def subsample_time_series(t, num_test):
     """Every ``len(t)//num_test``-th sample (evaluate_synthesis.py:102-110); -1 keeps everything."""
     if num_test == -1:

@@ -33,6 +33,9 @@
  *   dusty_swd_descriptors, dusty_swd_sliced   utils/metrics/swd.py (compute_swd, called evaluate_synthesis.py:169-173):
  *                                Laplacian pyramid, 7x7 patches, random projections, sort (SURVEY.md S2; the contract
  *                                is the swd-pytorch algorithm, DESIGN.md S2.7)
+ *   dusty_depth_metrics          utils/metrics/depth.py (RMSE / abs-rel / delta accuracy of evaluate_reconstruction.py,
+ *                                SURVEY.md S2; the contract is Eigen et al.'s set as monodepth2 computes it, DESIGN.md
+ *                                S2.8) with utils.postprocess's revert_depth on both images
  *   dusty_fps                    utils/sampling/fps/furthest_point_sampling.cpp:79-100
  *                                -> furthest_point_sampling_kernel_wrapper, furthest_point_sampling.cu:209-260
  *   dusty_gather_points          utils/sampling/fps/furthest_point_sampling.cpp:27-50
@@ -407,6 +410,26 @@ DUSTY_API int dusty_head_project_backward(const dusty_head_params* p, const floa
 /* Projection only: inv (b,1,h,w) in [0,1] (already tanh_to_sigmoid'ed and clamped) -> xyz. */
 DUSTY_API int dusty_inv_to_xyz(const dusty_head_params* p, const float* inv, const float* trig,
                      float* out_points, void* stream);
+
+/* --------------------------------------------------------------------------------------------
+ * Reconstruction metrics of range images (reference utils/metrics/depth.py)
+ * -------------------------------------------------------------------------------------------- */
+
+/* Per-scan sums of the reconstruction metrics (reference utils/metrics/depth.py, restated: DESIGN.md 2.8).
+ *   pred, target (b,1,h,w) f32 tanh space, 16-byte aligned, w a multiple of 4; p supplies b, h, w, tol and the
+ *   projection constants (other fields ignored). Each pixel becomes inv = clamp((x + 1) / 2, 0, 1), valid =
+ *   |inv| > tol (a NaN pixel is not valid) and the depth in metres 1 / (inv * disp_scale + disp_shift), rounded as
+ *   dusty_head_project rounds it.
+ *   sums (b, 10) f64, 8-byte aligned, overwritten: |S|, |pred valid|, |target valid|, sum |d|/t, sum d^2/t, sum d^2,
+ *   sum (log p - log t)^2, #a1, #a2, #a3  (S = pixels valid in both images; d = p - t; counts exact). Each sum is
+ *   reduced in a fixed order: a scan's sums are bit-identical from call to call and whatever batch it is part of.
+ *   out_pred_m, out_target_m (b,1,h,w) f32 depth in metres, 0 where invalid (NaN where the input is NaN, as the
+ *   reference's valid multiply leaves it), or NULL.
+ *   workspace: dusty_depth_metrics_workspace_bytes(b, h, w), 8-byte aligned. */
+DUSTY_API size_t dusty_depth_metrics_workspace_bytes(int b, int h, int w);
+DUSTY_API int dusty_depth_metrics(const dusty_head_params* p, const float* pred, const float* target,
+                                  double* sums, float* out_pred_m, float* out_target_m,
+                                  void* workspace, size_t workspace_bytes, void* stream);
 
 /* --------------------------------------------------------------------------------------------
  * Real-data side: organised LiDAR scans -> range images + clouds (the reference set of the evaluation)
