@@ -9,14 +9,16 @@ import numpy as np
 import torch
 
 
-def grid_points(resolution, clip_sphere=True):
+def grid_points(resolution, clip_sphere=True, device="cpu"):
+    """The reference builds its grid on the points' device; on a GPU, torch.norm may round a point that lies exactly
+    on the sphere (odd resolutions only) to the other side of 0.5 than on the CPU."""
     spacing = 1.0 / float(resolution - 1)
-    steps = torch.arange(resolution)
+    steps = torch.arange(resolution, device=device)
     grid = torch.stack(torch.meshgrid(steps, steps, steps, indexing="ij"), dim=-1) * spacing - 0.5
     grid = grid.reshape(-1, 3)
     if clip_sphere:
         grid = grid[torch.norm(grid, dim=1) <= 0.5]
-    return grid.numpy().astype(np.float32), spacing
+    return grid.cpu().numpy().astype(np.float32), spacing
 
 
 def vote(pcs, resolution=28, in_sphere=True):
@@ -38,6 +40,41 @@ def vote(pcs, resolution=28, in_sphere=True):
     return counters, touching
 
 
+def nearest_torch(points, grid, max_bytes=1 << 30):
+    """(dist, idx) of the nearest grid point to each of ``points`` (n,3) on their device: vote()'s arithmetic as
+    separate element-wise f32 ops (no ``.sum(-1)`` or matmul form, which may reorder the sum), first minimum on
+    ties, in chunks of points so that no intermediate exceeds about ``max_bytes``."""
+    points = points.reshape(-1, 3)
+    grid = grid.to(points.device)
+    dist = torch.empty(len(points), dtype=torch.float32, device=points.device)
+    idx = torch.empty(len(points), dtype=torch.int64, device=points.device)
+    chunk = max(1, max_bytes // (12 * max(len(grid), 1)))
+    for j in range(0, len(points), chunk):
+        d = points[j:j + chunk, None, :] - grid[None, :, :]
+        d = d * d
+        dj = (d[..., 0] + d[..., 1]) + d[..., 2]
+        dist[j:j + chunk], idx[j:j + chunk] = dj.amin(dim=1), dj.argmin(dim=1)
+    return dist, idx
+
+
+def vote_torch(pcs, resolution=28, in_sphere=True, grid_device=None):
+    """vote() in torch on ``pcs``'s device (a CUDA tensor for the evaluation's sizes) -> (counters, touching) as
+    int64 tensors there. The grid is built on ``grid_device``, by default the points' device as in the reference.
+    Pinned to vote() by tests/test_gpu_jsd_edges.py."""
+    pcs = torch.as_tensor(pcs, dtype=torch.float32)
+    B, Np, _ = pcs.shape
+    grid = torch.from_numpy(grid_points(resolution, in_sphere, grid_device or pcs.device)[0])
+    ng = len(grid)
+    if B * Np == 0:
+        zero = torch.zeros(ng, dtype=torch.int64, device=pcs.device)
+        return zero, zero.clone()
+    _, idx = nearest_torch(pcs, grid)
+    counters = torch.bincount(idx, minlength=ng)
+    touched = torch.zeros(B, ng, dtype=torch.bool, device=pcs.device)
+    touched.scatter_(1, idx.view(B, Np), True)
+    return counters, touched.sum(0)
+
+
 def _entropy(p, base2=True, eps=np.float32(1e-8)):
     p += eps                                                           # in place, like the reference
     log_p = np.log2(p) if base2 else np.log(p)
@@ -50,6 +87,32 @@ def jsd_from_counts(P, Q):
     e1 = _entropy(P_); e2 = _entropy(Q_)
     e_sum = _entropy((P_ + Q_) / np.float32(2.0))
     return float(e_sum - ((e1 + e2) / np.float32(2.0)))
+
+
+_EPS64 = float(np.float32(1e-8))       # the reference adds 1e-8 to f32 tensors: the f32 value of 1e-8
+
+
+def _entropy64(p, log):
+    return -(p * log(p)).sum()
+
+
+def jsd_from_counts_f64(P, Q):
+    """_jensen_shannon_divergence in float64 from exact counts, with the reference's eps placement: _entropy adds eps
+    to P_ and Q_ in place, so e_sum sees it twice. -> (jsd, e_sum, e1, e2)."""
+    P = np.asarray(P, np.float64); Q = np.asarray(Q, np.float64)
+    p = P / P.sum() + _EPS64
+    q = Q / Q.sum() + _EPS64
+    e1, e2 = _entropy64(p, np.log2), _entropy64(q, np.log2)
+    e_sum = _entropy64((p + q) / 2.0 + _EPS64, np.log2)
+    return e_sum - (e1 + e2) / 2.0, e_sum, e1, e2
+
+
+def acc_entropy_f64(touching, n_clouds, ng):
+    """entropy_of_occupancy_grid's acc_entropy (reference jsd.py:23-92: natural log, eps added once) in float64
+    from exact touching counts."""
+    t = np.asarray(touching, np.float64)
+    p = t[t > 0] / n_clouds
+    return _entropy64(np.concatenate([p, 1.0 - p]) + _EPS64, np.log) / ng
 
 
 def compute_jsd(pcs_gen, pcs_ref, resolution=28):
